@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- one AM() forward step of the Eagle genome-scan hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic data set of the BASELINE.json shape:
     decode (ASCII -> int8)  ->  transpose (Mt)  ->  M.Mt (int8 tcgen05)  [-> all-reduce(int32) when N>1]
@@ -12,6 +12,8 @@ Markers are sharded over the N ranks (strong scaling: the data set is fixed, L/N
 `forward_search` (N=1, after the timed region): BASELINE config 3 as it is worded -- the full multi-locus AM() forward
 search (<= 10 QTL, 5 planted) through eagleeverything_b200/am.py; --no-search skips it, --search-host adds the route with
 every n x n matrix crossing the host-level ABI.
+--dump-outputs DIR writes what the last timed step computed (a, var(a), the pick, rows of K) as float64 .npy files: the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 --impl reference times the CPU restatement of the reference path (numpy/OpenBLAS, all host threads)
 on a bounded sample of the same workload; it is the only leg that imports oracle/.
@@ -155,18 +157,15 @@ def run_reference(args):
     n, L = w["n"], w["L"]
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     t0 = time.perf_counter()
-    # every step costs the same whatever --steps is; cap the repetitions so that the arm ends within a few minutes
-    steps = max(1, min(args.steps, 8))
-    last = cpu_reference_sample(n, L, steps=steps, warmup=min(args.warmup, 1))
+    last = cpu_reference_sample(n, L, steps=args.steps, warmup=min(args.warmup, 1))
     wall = time.perf_counter() - t0
     v = last["value"]
     jprint({"impl": "reference", "metric": METRIC, "value": v, "unit": METRIC, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * L / v, "higher_is_better": True, "scaling": "strong",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": bench_config(w, n, L, world),
-            "note": "CPU restatement of the reference path; the reference itself (R + RcppEigen) cannot be built in this "
-                    f"image.  {steps} timed passes over the same fixed {REF_SAMPLE_MARKERS}-marker sample (of the --steps "
-                    f"{args.steps} asked for: a pass takes seconds and every pass times the same work)",
+            "note": "CPU restatement of the reference path (the reference itself runs inside R with RcppEigen); "
+                    f"{args.steps} timed passes over the same fixed {REF_SAMPLE_MARKERS}-marker sample",
             "cpu_baseline": last,
             "e2e": {"value": v, "unit": METRIC, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "wall_s": wall})
@@ -423,7 +422,11 @@ def run_gpu(args):
     _lib.check(lib.eg_last_prep_kernels(C.byref(p_ms), C.byref(p_ops)))
     # ---------------- results of the last step, hashed (the same hashes must come out at every N) and, at N > 1, compared
     # bit for bit with a single-GPU run of the same data set computed here (rank 0) -- a mismatch fails the run
-    checks = result_checks(args, torch, dist, device, egd, lib, n, L, Lg, c0, world, rank, K, oa, ov, S, V, ah, res)
+    a_all, v_all = egd.gather_sharded(oa, L, world), egd.gather_sharded(ov, L, world)   # a, var(a) over ALL markers
+    checks = result_checks(args, torch, dist, device, egd, lib, n, L, Lg, c0, world, rank, K, a_all, v_all, S, V, ah, res)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, K, a_all, v_all, res)
+    del a_all, v_all
     if checks.get("failed"):
         if rank == 0:
             jprint({"metric": METRIC, "value": None, "n_gpus": world, "error": "multi-rank parity failed", "checks": checks})
@@ -841,19 +844,37 @@ def run_dropin(args, torch, lib, device, n, L, img_h, S_h, V_h, a_h, time_host):
         shutil.rmtree(d, ignore_errors=True)
 
 
+DUMP_K_BYTES = 24 << 20   # rows of K kept by --dump-outputs; with a and var(a) of the largest workload under 64 MB
+DUMP_SEED = 7
+
+
+def dump_outputs(d, torch, K, a, vara, res):
+    """--dump-outputs: what the timed step hands its caller, as one float64 .npy per array under `d`: a and var(a) of
+    every marker, the picked marker and its t^2 statistic, and the rows of K -- every row when K fits DUMP_K_BYTES,
+    otherwise a fixed seeded sample of rows, listed in K_rows_index.npy.  The inputs are seeded as well, so two builds
+    run with the same arguments can be compared file by file."""
+    import numpy as np
+    n = K.shape[0]
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(n, DUMP_K_BYTES // (8 * n)), replace=False))
+    arrays = {"a": a, "vara": vara, "K_rows": K[torch.from_numpy(rows).to(K.device)], "K_rows_index": rows,
+              "picked_marker": [int(res[1])], "picked_tsq": [float(res[0])]}
+    os.makedirs(d, exist_ok=True)
+    for name, v in arrays.items():
+        v = v.cpu().numpy() if torch.is_tensor(v) else v
+        np.save(os.path.join(d, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def _sha(t):
     import hashlib
     return hashlib.sha256(t.contiguous().cpu().numpy().tobytes()).hexdigest()
 
 
-def result_checks(args, torch, dist, device, egd, lib, n, L, Lg, c0, world, rank, K, oa, ov, S, V, ah, res):
+def result_checks(args, torch, dist, device, egd, lib, n, L, Lg, c0, world, rank, K, a_all, v_all, S, V, ah, res):
     """sha256 of the results of the last timed step -- K (after the all-reduce), a, var(a) over ALL markers, the pick -- so
     that the lines of a scaling run can be compared with each other; and at N > 1 (when the whole data set fits one GPU)
     the same step recomputed on rank 0 alone and compared bit for bit: the all-reduced K, every shard of a / var(a), the
     pick.  `failed` is set on any mismatch (the run then exits non-zero)."""
     out = {}
-    a_all = egd.gather_sharded(oa, L, world) if world > 1 else oa
-    v_all = egd.gather_sharded(ov, L, world) if world > 1 else ov
     picked = int(res[1]) if not hasattr(res[1], "item") else int(res[1].item())
     if world > 1:   # every rank holds the same K after the all-reduce: compare 128-bit fingerprints across ranks
         kv = K.view(torch.int64).reshape(-1)
@@ -1136,7 +1157,12 @@ def main():
     ap.add_argument("--no-dropin", action="store_true", help="skip the file-based drop-in legs of the end-to-end measurement")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the in-run comparison with a single-GPU evaluation")
     ap.add_argument("--no-extras", action="store_true", help="N = 8: skip the one-step config 5 / config 4 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; --impl reference has none to write")
     if args.impl == "reference":
         run_reference(args)
     else:

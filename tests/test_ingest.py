@@ -2,8 +2,9 @@
 src/createM_ASCII_rcpp.cpp:19-106 + src/CreateASCIInospace.cpp:17-164) and createMt_ASCII_rcpp (M.ascii -> Mt.ascii,
 src/createMt_ASCII_rcpp.cpp:15-245).
 
-CPU tests: oracle/eagle_oracle.c against the reference's own sources compiled through oracle/refshim (file bytes, return
-value and every message).  GPU tests: the device tokeniser / encoder through the C ABI against the oracle, byte for byte."""
+CPU tests: oracle/eagle_oracle.c against the reference's own sources (file bytes, return value and every message), as
+recorded in tests/golden/reference_calls.json and, where they are compiled through oracle/refshim, live.  GPU tests:
+the device tokeniser / encoder through the C ABI against the oracle, byte for byte."""
 import hashlib
 import os
 
@@ -13,6 +14,7 @@ import pytest
 from eagleeverything_b200 import synth
 from oracle import eagle_oracle as eo
 from oracle import np_oracle as npo
+from reference_record import error_message, fingerprint, reference  # noqa: F401  (fixture)
 
 
 def write_text(path, G, codes=("0", "1", "2"), missing=None, miss_at=(), style=0, final_newline=True, seed=0):
@@ -120,27 +122,26 @@ def test_oracle_tokeniser_known_answers(ingest_cases, tmp_path):
     assert not ok and msgs == ["ERROR: Text file could not be opened with filename  " + str(tmp_path / "absent.txt") + "\n"]
 
 
-@pytest.mark.skipif(not eo.reference_available(), reason="oracle/_ref/libeagle_ref.so not built")
-def test_oracle_ingest_matches_reference_code(ingest_cases, tmp_path, demo):
+def test_oracle_ingest_matches_reference_code(ingest_cases, tmp_path, demo, reference):
+    tmp = reference.tmp
     for case in ingest_cases:
         for quiet in (False, True):
-            mine = run_oracle(case, str(tmp_path / "mine.ascii"), quiet)
-            with eo.use_reference():
-                ref = run_oracle(case, str(tmp_path / "ref.ascii"), quiet)
+            mine = fingerprint(run_oracle(case, str(tmp_path / "mine.ascii"), quiet), tmp)
             if case[0] == "long_row":      # the reference writes beyond its row buffer here (CreateASCIInospace.cpp:85): same
-                assert mine[0] == ref[0] and mine[1] == ref[1]  # verdict and messages, file content undefined
+                ref = reference(lambda: run_oracle(case, str(tmp_path / "ref.ascii"), quiet)[:2])
+                assert mine[:2] == ref     # verdict and messages, file content undefined
                 continue
-            assert mine == ref, (case[0], quiet)
+            assert mine == reference(lambda: run_oracle(case, str(tmp_path / "ref.ascii"), quiet)), (case[0], quiet)
     # createMt: both situations of the reference write the same bytes; messages but for the two formatted doubles
     for d, mems in ((demo, (8.0, 0.002)), ):
         dims = (d["n"], d["L"])
         for mem in mems:
             for quiet in (False, True):
                 m1 = eo.createMt_ASCII_rcpp(d["M"], str(tmp_path / "mine.Mt"), "text", mem, dims, quiet)
-                with eo.use_reference():
-                    m2 = eo.createMt_ASCII_rcpp(d["M"], str(tmp_path / "ref.Mt"), "text", mem, dims, quiet)
-                assert open(tmp_path / "mine.Mt", "rb").read() == open(tmp_path / "ref.Mt", "rb").read() == open(d["Mt"], "rb").read()
-                assert m1 == m2, (mem, quiet)
+                m2, ref_bytes = reference(lambda: (eo.createMt_ASCII_rcpp(d["M"], str(tmp_path / "ref.Mt"), "text", mem, dims, quiet),
+                                                   open(tmp_path / "ref.Mt", "rb").read()))
+                assert fingerprint(open(tmp_path / "mine.Mt", "rb").read(), tmp) == ref_bytes == fingerprint(open(d["Mt"], "rb").read(), tmp)
+                assert fingerprint(m1, tmp) == m2, (mem, quiet)
                 assert (len(m1) > 10) == (mem < 1 and not quiet)   # the block situation announces itself
 
 
@@ -253,25 +254,20 @@ def test_oracle_plink_known_answers(plink_cases, tmp_path):
     assert any("unequal number of columns" in m for m in msgs) and not any("more than two alleles" in m for m in msgs)
 
 
-@pytest.mark.skipif(not eo.reference_available(), reason="oracle/_ref/libeagle_ref.so not built")
-def test_oracle_plink_matches_reference_code(plink_cases, tmp_path):
+def test_oracle_plink_matches_reference_code(plink_cases, tmp_path, reference):
+    tmp = reference.tmp
     for case in plink_cases:
         mine = run_oracle_ped(case, str(tmp_path / "mine.ascii"))
-        with eo.use_reference():
-            ref = run_oracle_ped(case, str(tmp_path / "ref.ascii"))
-        assert mine == ref, case[0]
+        assert fingerprint(mine, tmp) == reference(lambda: run_oracle_ped(case, str(tmp_path / "ref.ascii"))), case[0]
     # multi-character allele tokens: the reference reads them character by character; so does the restatement
     p = str(tmp_path / "multi.ped")
     open(p, "w").write("f i1 0 0 1 0 AC G T T\nf i2 0 0 1 0 A C GT T\n")
     case = ("multi", p, (2, 10), True)
     mine = run_oracle_ped(case, str(tmp_path / "mine.ascii"))
-    with eo.use_reference():
-        ref = run_oracle_ped(case, str(tmp_path / "ref.ascii"))
-    assert mine == ref
+    assert fingerprint(mine, tmp) == reference(lambda: run_oracle_ped(case, str(tmp_path / "ref.ascii")))
     mine = eo.createM_ASCII_rcpp(str(tmp_path / "absent.ped"), str(tmp_path / "o"), "PLINK", "", "", "", 8, (2, 10), True, "")
-    with eo.use_reference():
-        ref = eo.createM_ASCII_rcpp(str(tmp_path / "absent.ped"), str(tmp_path / "o"), "PLINK", "", "", "", 8, (2, 10), True, "")
-    assert mine == ref and not mine[0] and len(mine[1]) == 2
+    ref = reference(lambda: eo.createM_ASCII_rcpp(str(tmp_path / "absent.ped"), str(tmp_path / "o"), "PLINK", "", "", "", 8, (2, 10), True, ""))
+    assert fingerprint(mine, tmp) == ref and not mine[0] and len(mine[1]) == 2
 
 
 # ---------------------------------------------------------------------------------------------------- ReshapeM, getRowColumn
@@ -299,25 +295,22 @@ def test_oracle_reshape_and_rowcolumn_known_answers(synth_small, tmp_path, inges
     assert eo.getRowColumn(s["M"]) == [s["n"], 1]
 
 
-@pytest.mark.skipif(not eo.reference_available(), reason="oracle/_ref/libeagle_ref.so not built")
-def test_oracle_reshape_and_rowcolumn_match_reference_code(synth_small, tmp_path, ingest_cases, plink_cases):
+def test_oracle_reshape_and_rowcolumn_match_reference_code(synth_small, tmp_path, ingest_cases, plink_cases, reference):
     s = synth_small
     for k, idx in enumerate(RESHAPE_CASES):
         m1, mt1 = _reshape_files(tmp_path, s, f"a{k}")
         m2, mt2 = _reshape_files(tmp_path, s, f"b{k}")
-        mine = eo.ReshapeM_rcpp(m1, mt1, idx, (s["n"], s["L"]))
-        with eo.use_reference():
-            ref = eo.ReshapeM_rcpp(m2, mt2, idx, (s["n"], s["L"]))
-        assert mine == ref, idx
-        assert open(m1 + "tmp", "rb").read() == open(m2 + "tmp", "rb").read(), idx
-        assert open(mt1 + "tmp", "rb").read() == open(mt2 + "tmp", "rb").read(), idx
+        mine = reshape_and_read(m1, mt1, idx, (s["n"], s["L"]))
+        assert fingerprint(mine, "") == reference(lambda: reshape_and_read(m2, mt2, idx, (s["n"], s["L"]))), idx
     for case in list(ingest_cases) + list(plink_cases):
-        mine = eo.getRowColumn(case[1])
-        with eo.use_reference():
-            assert eo.getRowColumn(case[1]) == mine, case[0]
-    with eo.use_reference():
-        with pytest.raises(eo.OracleError, match="ERROR: Could not open"):
-            eo.getRowColumn(str(tmp_path / "absent"))
+        assert eo.getRowColumn(case[1]) == reference(lambda: eo.getRowColumn(case[1])), case[0]
+    msg = reference(lambda: error_message(eo.getRowColumn, str(tmp_path / "absent")))
+    assert msg is not None and "ERROR: Could not open" in msg
+
+
+def reshape_and_read(m, mt, idx, dims):
+    """ReshapeM_rcpp's return value and the two files it writes."""
+    return eo.ReshapeM_rcpp(m, mt, idx, dims), open(m + "tmp", "rb").read(), open(mt + "tmp", "rb").read()
 
 
 @pytest.mark.gpu
@@ -414,35 +407,28 @@ def fuzz_ped_case(rng, path):
     return (rows, 6 + 2 * nsnp)
 
 
-@pytest.mark.skipif(not eo.reference_available(), reason="oracle/_ref/libeagle_ref.so not built")
-def test_oracle_ingest_fuzz_against_reference_code(tmp_path):
+def test_oracle_ingest_fuzz_against_reference_code(tmp_path, reference):
     rng = np.random.default_rng(2026)
     p = str(tmp_path / "f.txt")
     n_bad = 0
+    read = lambda name: open(tmp_path / name, "rb").read()
     for k in range(300):
         dims, AA, AB, BB, missing = fuzz_text_case(rng, p)
         mine = eo.createM_ASCII_rcpp(p, str(tmp_path / "a"), "text", AA, AB, BB, 8.0, dims, True, missing)
-        with eo.use_reference():
-            ref = eo.createM_ASCII_rcpp(p, str(tmp_path / "b"), "text", AA, AB, BB, 8.0, dims, True, missing)
-        assert mine == ref, (k, open(p, "rb").read())
         too_long = not mine[0] and any("which contains" in m and int(m.split("contains")[1].split()[0]) > dims[1] for m in mine[1])
-        if not too_long:   # beyond dims[1] tokens the reference writes outside its row buffer
-            assert open(tmp_path / "a", "rb").read() == open(tmp_path / "b", "rb").read(), k
+        # beyond dims[1] tokens the reference writes outside its row buffer: file content undefined
+        ref = reference(lambda: (eo.createM_ASCII_rcpp(p, str(tmp_path / "b"), "text", AA, AB, BB, 8.0, dims, True, missing),
+                                 None if too_long else read("b")), digest=True)
+        assert reference.fp((mine, None if too_long else read("a")), digest=True) == ref, (k, open(p, "rb").read())
         n_bad += not mine[0]
-        assert eo.getRowColumn(p) == _ref(eo.getRowColumn, p)
+        assert eo.getRowColumn(p) == reference(lambda: eo.getRowColumn(p))
     assert 60 < n_bad < 240
     for k in range(200):
         dims = fuzz_ped_case(rng, p)
         mine = eo.createM_ASCII_rcpp(p, str(tmp_path / "a"), "PLINK", "", "", "", 8.0, dims, True, "")
-        with eo.use_reference():
-            ref = eo.createM_ASCII_rcpp(p, str(tmp_path / "b"), "PLINK", "", "", "", 8.0, dims, True, "")
-        assert mine == ref, (k, open(p, "rb").read())
-        assert open(tmp_path / "a", "rb").read() == open(tmp_path / "b", "rb").read(), k
-
-
-def _ref(fn, *a):
-    with eo.use_reference():
-        return fn(*a)
+        ref = reference(lambda: (eo.createM_ASCII_rcpp(p, str(tmp_path / "b"), "PLINK", "", "", "", 8.0, dims, True, ""), read("b")),
+                        digest=True)
+        assert reference.fp((mine, read("a")), digest=True) == ref, (k, open(p, "rb").read())
 
 
 def test_second_restatement_agrees_with_the_c_oracle_on_the_fuzz_corpus(tmp_path):
@@ -498,8 +484,7 @@ def fuzz_reshape_case(rng, tmp_path, tag):
     return (m, mt, [int(i) for i in idx], (n, L)) if ok and size > 0 and len(set(idx)) < n else None
 
 
-@pytest.mark.skipif(not eo.reference_available(), reason="oracle/_ref/libeagle_ref.so not built")
-def test_oracle_reshape_fuzz_against_reference_code(tmp_path):
+def test_oracle_reshape_fuzz_against_reference_code(tmp_path, reference):
     rng = np.random.default_rng(77)
     done = 0
     for k in range(150):
@@ -510,9 +495,8 @@ def test_oracle_reshape_fuzz_against_reference_code(tmp_path):
         import shutil
         m2, mt2 = str(tmp_path / "Mb.ascii"), str(tmp_path / "Mtb.ascii")
         shutil.copy(m, m2); shutil.copy(mt, mt2)
-        assert eo.ReshapeM_rcpp(m, mt, idx, dims) == _ref(eo.ReshapeM_rcpp, m2, mt2, idx, dims), idx
-        assert open(m + "tmp", "rb").read() == open(m2 + "tmp", "rb").read(), idx
-        assert open(mt + "tmp", "rb").read() == open(mt2 + "tmp", "rb").read(), idx
+        mine = reshape_and_read(m, mt, idx, dims)
+        assert reference.fp(mine, digest=True) == reference(lambda: reshape_and_read(m2, mt2, idx, dims), digest=True), idx
         done += 1
     assert done > 100
 

@@ -146,7 +146,23 @@ def test_am_forward_search_golden(demo):
     np.testing.assert_allclose(r["extBIC"], [925.742, 887.799, 886.762, 885.097, 889.442], atol=2e-3)
     t0 = r["trace"][0]
     np.testing.assert_allclose(t0["a"], z["it1_a"], rtol=1e-9, atol=1e-9)
-    np.testing.assert_allclose(t0["vara"], z["it1_vara"], rtol=1e-9, atol=1e-9)
+    # The n x n algebra before the scan runs through numpy's multi-threaded LAPACK / BLAS, so S and V carry rounding that
+    # depends on the host's thread count.  The scan itself is reproducible: at the stored first-iteration inputs it
+    # must give the stored a / var(a); the search's own var(a) may differ from them by what its S, V differences
+    # propagate (|m|' |W - W_stored| |m|) plus the contraction's rounding -- var(a) of monomorphic markers is 0 up to
+    # exactly that noise.
+    n, L = demo["n"], demo["L"]
+    S0, V0, h0 = z["it1_S"], z["it1_V"], z["it1_hat_a"]
+    scan0 = eo.calculate_a_and_vara_rcpp(demo["Mt"], [NA], S0, V0, 8, (L, n), h0)
+    np.testing.assert_allclose(scan0["a"][:, 0], z["it1_a"], rtol=1e-9, atol=1e-9)
+    np.testing.assert_allclose(scan0["vara"][:, 0], z["it1_vara"], rtol=1e-9, atol=1e-9)
+    for k in ("S", "V", "hat_a"):
+        np.testing.assert_allclose(t0[k], z["it1_" + k], rtol=0, atol=1e-9 * np.abs(z["it1_" + k]).max())
+    Mabs = np.abs(demo["G"].astype(np.float64) - 1)
+    W, W0 = t0["S"] @ t0["V"] @ t0["S"], S0 @ V0 @ S0
+    drift = np.einsum("ij,ij->j", Mabs, np.abs(W - W0) @ Mabs)
+    rounding = 4 * (n + 10) * np.finfo(np.float64).eps * np.einsum("ij,ij->j", Mabs, np.abs(W) @ Mabs)
+    assert (np.abs(t0["vara"] - z["it1_vara"]) <= 1e-9 * np.abs(z["it1_vara"]) + 1e-9 + drift + rounding).all()
     np.testing.assert_allclose(t0["a"][:3], [28.8059, -12.3227, -40.3413], atol=1e-3)
     # the tie hazard: demo columns 2207 and 2209 are identical, their tsq tie and the first wins
     assert np.array_equal(demo["G"][:, 2206], demo["G"][:, 2208])
