@@ -212,6 +212,36 @@ void pool_give_back() {
     if (cudaDeviceGetDefaultMemPool(&pool, g_ctx.device) == cudaSuccess) cudaMemPoolTrimTo(pool, 0);
 }
 
+// Scratch for work queued on `st` by another translation unit (syrk_i8.cu: the E2M1 copy of a store).  The pool orders
+// everything on g_ctx.stream, so `st` waits for the allocation and g_ctx.stream for the work on `st` before the block
+// can be handed out again.
+static void stream_after(cudaStream_t waiter, cudaStream_t st) {
+    if (waiter == st) return;
+    cudaEvent_t ev;
+    if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+        cudaGetLastError();
+        cudaStreamSynchronize(st);
+        return;
+    }
+    cudaEventRecord(ev, st);
+    cudaStreamWaitEvent(waiter, ev, 0);
+    cudaEventDestroy(ev);
+}
+cudaError_t scratch_alloc(void** p, size_t bytes, cudaStream_t st) {
+    cudaError_t e = pool_alloc(p, bytes);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        *p = nullptr;
+        return e;
+    }
+    stream_after(st, g_ctx.stream);
+    return cudaSuccess;
+}
+void scratch_free(void* p, cudaStream_t st) {
+    stream_after(g_ctx.stream, st);
+    pool_free(p);
+}
+
 // RAII device buffer (valid on g_ctx.stream)
 struct DevBuf {
     void* p = nullptr;

@@ -13,6 +13,8 @@ int check_cuda(cudaError_t e, const char* what); // EG_OK or EG_ERR_CUDA (+messa
 int check_launch(const char* kernel);            // cudaGetLastError() after a launch
 int num_sms();                                   // SM count of the current device (148 on B200)
 void pool_give_back();                           // release the library's cached device memory to the driver (retry after an OOM)
+cudaError_t scratch_alloc(void** p, size_t bytes, cudaStream_t st);  // pool block usable on st (capi.cu)
+void scratch_free(void* p, cudaStream_t st);                         // back to the pool after the work queued on st
 // cudaMalloc with one retry after pool_give_back()
 static inline cudaError_t malloc_retry(void** p, size_t bytes) {
     cudaError_t e = cudaMalloc(p, bytes);

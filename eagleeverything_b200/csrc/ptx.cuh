@@ -135,6 +135,19 @@ __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t desc_a, uint64
         "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// D[tmem] (+)= (A[smem] * scale_A[tmem]) * (B[smem] * scale_B[tmem]), packed E2M1 x E2M1 -> f32, K = 64 per
+// instruction, one ue8m0 scale per 32 elements along K (block32 = scale_vec::2X).
+__device__ __forceinline__ void umma_mxf4(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t tmem_sfa, uint32_t tmem_sfb, uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.block32 [%0], %1, %2, %3, [%5], [%6], p;\n"
+        "}\n" ::"r"(tmem_d),
+        "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(tmem_sfa), "r"(tmem_sfb)
+        : "memory");
+}
 // mbarrier arrive when all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -180,6 +193,12 @@ __device__ __forceinline__ void tmem_ld_32x24(uint32_t taddr, uint32_t (&v)[32])
                  : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// 32 lanes x 8 columns of 32-bit, every cell set to `x` (thread i of the warp writes lane base_lane + i)
+__device__ __forceinline__ void tmem_fill_32x8(uint32_t taddr, uint32_t x) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %1, %1, %1, %1, %1, %1, %1};" ::"r"(taddr), "r"(x)
+                 : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ---------------------------------------------------------------- CTA pairs (cluster of 2, tcgen05 cta_group::2)
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -268,6 +287,11 @@ __device__ __forceinline__ uint64_t make_desc_k_sw128(uint32_t smem_addr) {
 // Instruction descriptor for kind::i8: D = s32, A = B = signed 8-bit, both K-major.
 __host__ __device__ constexpr uint32_t make_idesc_i8(int M, int N) {
     return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+// Instruction descriptor for kind::mxf4 (block-scaled layout): A = B = E2M1 (format 1), both K-major, D = f32,
+// scale format ue8m0 (bit 23), scale-factor ids 0 (bits [4,6) and [29,31)).
+__host__ __device__ constexpr uint32_t make_idesc_mxf4(int M, int N) {
+    return (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | (1u << 23) | ((uint32_t)(M >> 4) << 24);
 }
 
 // ---------------------------------------------------------------- FP64 tensor core (DMMA.8x8x4)

@@ -1,23 +1,31 @@
-// K2 -- genomic relationship product  C = M * M^T  on the int8 tcgen05 tensor cores.
+// K2 -- genomic relationship product  C = M * M^T  on the tcgen05 tensor cores, exact in int32.
 //
 // Replaces the FP64 Eigen product `MMt.noalias() = genoMat * genoMat.transpose()`
 // (reference: src/calculateMMt_rcpp.cpp:95, blocked variants :138, :161).  Genotypes are
-// {-1,0,1}, so s8 x s8 -> s32 accumulation is EXACT (|entry| <= L < 2^31) and any summation
-// order gives the same integers as the reference's double arithmetic.
+// {-1,0,1}, so every product is an exact integer with |entry| <= L, and any summation order gives
+// the same integers as the reference's double arithmetic.  Two kernels compute it:
 //
-// Layout: M is the resident int8 store, n rows x K columns, row-major (markers contiguous =
-// K-major for both operands of M*M^T), row pitch a multiple of 128 B, zero padded.
-// One TMA tensor map over it (128 B x 128 row boxes, SWIZZLE_128B) feeds both operands.
+//   syrk_fp4_kernel (default)  the store is first packed to E2M1 (+1 -> 0x2, -1 -> 0xA, 0 -> 0x0, two
+//       markers per byte, pack_e2m1_kernel), then tcgen05.mma.kind::mxf4.block_scale with every ue8m0
+//       block scale 2^0 and FP32 accumulation: half the operand bytes of int8 at twice its nominal rate.
+//       The FP32 sums are integers; they stay exact while one accumulator chain holds at most
+//       MMT_FP4_CHAIN markers (DESIGN.md section 4b: the probe), and the epilogue rounds them to int32.
+//   syrk_i8_kernel (EAGLE_MMT_MODE=i8)  s8 x s8 -> s32 on the store itself.
+//
+// Layout: the operand is K-major for both sides of M*M^T (markers contiguous), either M row-major with a
+// row pitch (multiple of 128 B, zero padded) or K-blocked [K/128][rows][128] (eg_dev_decode_kb); the E2M1
+// copy is always K-blocked [ceil(K/256)][rows][128 B].  TMA boxes of 128 B x rows, SWIZZLE_128B.
 //
 // Kernel: persistent, warp specialised, 192 threads:
-//   warp 0   TMA producer  (3 box loads / stage: A 128 rows, B 2 x 128 rows), 4-stage smem ring
-//   warp 1   UMMA issuer   tcgen05.mma.cta_group::1.kind::i8, M=128 N=256 K=32, 4 per stage,
-//                          accumulators in TMEM, double buffered (2 x 256 columns)
+//   warp 0   TMA producer  (A 128 rows, B BN rows per stage), 4-stage smem ring
+//   warp 1   UMMA issuer   M=128, 4 MMAs per 128-B atom (int8: N=256 K=32; E2M1: N=224 K=64),
+//                          accumulators in TMEM, double buffered (int8 2 x 256 columns; E2M1 2 x 224
+//                          columns + 64 columns of scale factors, written once per CTA)
 //   warps 2-5 epilogue     tcgen05.ld 32x32b -> registers -> red.global.add.s32 into C
-// Work unit = (output tile 128 x 256 that touches the upper triangle, K chunk).  K is split only
-// when there are too few tiles to fill the SMs; integer atomics keep the result exact and
-// order independent.  Tiles are ordered in compact super-rows so that one wave of CTAs shares
-// operand rows in L2 while all of them stream along K together.
+// Work unit = (output tile 128 x BN that touches the upper triangle, K chunk).  K is split when there
+// are too few tiles to fill the SMs and, for E2M1, wherever a chain would pass MMT_FP4_CHAIN; integer
+// atomics keep the result exact and order independent.  Tiles are ordered in compact super-rows so
+// that one wave of CTAs shares operand rows in L2 while all of them stream along K together.
 //
 // K-phase flow control.  The L2 reuse above only happens if the CTAs of a wave stay within the L2
 // window along K (126 MB / (rows of the wave x 128 B) ~ 200 k-blocks); measured without it at
@@ -35,17 +43,25 @@
 namespace eg {
 
 constexpr int SY_BM = 128;
-constexpr int SY_BN = 256;
-constexpr int SY_BK = 128;  // bytes == int8 elements per stage along K (one 128-B swizzle atom)
+constexpr int SY_BK = 128;  // bytes per stage along K (one 128-B swizzle atom): 128 int8 or 256 E2M1 markers
 constexpr int SY_STAGES = 4;
 constexpr int SY_A_BYTES = SY_BM * SY_BK;
-constexpr int SY_B_BYTES = SY_BN * SY_BK;
-constexpr int SY_STAGE_BYTES = SY_A_BYTES + SY_B_BYTES;
 constexpr int SY_THREADS = 192;
 constexpr int SY_TMEM_COLS = 512;
-constexpr int SY_PHASE = 16;  // k-blocks per flow-control phase (2 KB of K)
+constexpr int SY_PHASE = 16;  // k-blocks per flow-control phase (16 x 128 B of K)
 constexpr int SY_LAG = 4;     // a producer may run at most this many phases ahead of the slowest CTA
-constexpr int SY_SMEM_BYTES = SY_STAGES * SY_STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
+// Longest exact FP32 accumulator chain of the E2M1 kernel, in markers (DESIGN.md section 4b).
+constexpr int64_t MMT_FP4_CHAIN = (int64_t)1 << 20;
+
+template <bool FP4>
+struct SyrkShape {
+    static constexpr int BN = FP4 ? 224 : 256;
+    static constexpr int B_BYTES = BN * SY_BK;
+    static constexpr int STAGE_BYTES = SY_A_BYTES + B_BYTES;
+    static constexpr int SMEM_BYTES = SY_STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
+    static constexpr uint32_t SF_COL = 2 * BN;  // E2M1: 64 columns of ue8m0 scales after the two accumulators
+};
+static_assert(2 * SyrkShape<true>::BN + 64 <= SY_TMEM_COLS, "E2M1 accumulators + scale factors exceed TMEM");
 
 struct SyrkParams {
     int64_t n;
@@ -70,14 +86,16 @@ __device__ __forceinline__ uint32_t ld_relaxed(const uint32_t* p) {
     return v;
 }
 
-// KB == false: M row-major, 2-D tensor map {K, rows};  KB == true: M K-blocked [K/128][rows][128],
-// 3-D tensor map {128, rows, K/128} -- one K-block of all rows is a contiguous range of memory.
-template <bool KB>
-__global__ void __launch_bounds__(SY_THREADS, 1)
-syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
+// KB == false: M row-major, 2-D tensor maps {K, rows};  KB == true: M K-blocked [K/128 B][rows][128 B],
+// 3-D tensor maps {128, rows, K-blocks} -- one K-block of all rows is a contiguous range of memory.
+// tmA has 128-row boxes; int8 loads B as two of them, E2M1 as one box of tmB (224 rows).
+template <bool KB, bool FP4>
+__device__ __forceinline__ void syrk_body(const CUtensorMap* tmA, const CUtensorMap* tmB, const SyrkParams& p) {
+    using S = SyrkShape<FP4>;
+    constexpr int BN = S::BN;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SY_STAGES * SY_STAGE_BYTES);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SY_STAGES * S::STAGE_BYTES);
     uint64_t* full = bars;                       // [SY_STAGES]
     uint64_t* empty = bars + SY_STAGES;          // [SY_STAGES]
     uint64_t* tmem_full = bars + 2 * SY_STAGES;  // [2]
@@ -87,7 +105,8 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
     if (warp == 0 && lane == 0) {
-        ptx::prefetch_tmap(&tmap);
+        ptx::prefetch_tmap(tmA);
+        if (FP4) ptx::prefetch_tmap(tmB);
         for (int s = 0; s < SY_STAGES; s++) {
             ptx::mbar_init(&full[s], 1);
             ptx::mbar_init(&empty[s], 1);
@@ -103,6 +122,19 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
     __syncthreads();
     ptx::tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
+    if (FP4) {
+        // every ue8m0 scale factor is 0x7F = 2^0: fill 64 columns of all 128 lanes, whatever part of them the
+        // scale-factor layout reads
+        if (warp >= 2) {
+            const uint32_t base = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + S::SF_COL;
+#pragma unroll
+            for (int c = 0; c < 64; c += 8) ptx::tmem_fill_32x8(base + c, 0x7F7F7F7Fu);
+            ptx::tmem_st_wait();
+        }
+        ptx::tc_fence_before();
+        __syncthreads();
+        ptx::tc_fence_after();
+    }
 
     if (warp == 0) {
         // ------------------------------------------------------------ TMA producer
@@ -143,17 +175,20 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
                         }
                     }
                     ptx::mbar_wait(&empty[stage], phase ^ 1);
-                    uint8_t* sA = smem + stage * SY_STAGE_BYTES;
+                    uint8_t* sA = smem + stage * S::STAGE_BYTES;
                     uint8_t* sB = sA + SY_A_BYTES;
-                    ptx::mbar_expect_tx(&full[stage], SY_STAGE_BYTES);
-                    if (KB) {
-                        ptx::tma_load_3d(sA, &tmap, 0, t.x * SY_BM, kb, &full[stage]);
-                        ptx::tma_load_3d(sB, &tmap, 0, t.y * SY_BN, kb, &full[stage]);
-                        ptx::tma_load_3d(sB + SY_B_BYTES / 2, &tmap, 0, t.y * SY_BN + 128, kb, &full[stage]);
+                    ptx::mbar_expect_tx(&full[stage], S::STAGE_BYTES);
+                    if (FP4) {
+                        ptx::tma_load_3d(sA, tmA, 0, t.x * SY_BM, kb, &full[stage]);
+                        ptx::tma_load_3d(sB, tmB, 0, t.y * BN, kb, &full[stage]);
+                    } else if (KB) {
+                        ptx::tma_load_3d(sA, tmA, 0, t.x * SY_BM, kb, &full[stage]);
+                        ptx::tma_load_3d(sB, tmA, 0, t.y * BN, kb, &full[stage]);
+                        ptx::tma_load_3d(sB + S::B_BYTES / 2, tmA, 0, t.y * BN + 128, kb, &full[stage]);
                     } else {
-                        ptx::tma_load_2d(sA, &tmap, kb * SY_BK, t.x * SY_BM, &full[stage]);
-                        ptx::tma_load_2d(sB, &tmap, kb * SY_BK, t.y * SY_BN, &full[stage]);
-                        ptx::tma_load_2d(sB + SY_B_BYTES / 2, &tmap, kb * SY_BK, t.y * SY_BN + 128, &full[stage]);
+                        ptx::tma_load_2d(sA, tmA, kb * SY_BK, t.x * SY_BM, &full[stage]);
+                        ptx::tma_load_2d(sB, tmA, kb * SY_BK, t.y * BN, &full[stage]);
+                        ptx::tma_load_2d(sB + S::B_BYTES / 2, tmA, kb * SY_BK, t.y * BN + 128, &full[stage]);
                     }
                     if (++stage == SY_STAGES) { stage = 0; phase ^= 1; }
                 }
@@ -162,7 +197,8 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
     } else if (warp == 1) {
         // ------------------------------------------------------------ UMMA issuer
         if (lane == 0) {
-            constexpr uint32_t idesc = ptx::make_idesc_i8(SY_BM, SY_BN);
+            constexpr uint32_t idesc = FP4 ? ptx::make_idesc_mxf4(SY_BM, BN) : ptx::make_idesc_i8(SY_BM, BN);
+            const uint32_t sf_tmem = tmem_base + S::SF_COL;
             int stage = 0;
             uint32_t phase = 0;
             int acc = 0;
@@ -174,7 +210,7 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
                 const int kb1 = min(kb0 + p.kblocks_per_chunk, p.kblocks_total);
                 ptx::mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
                 ptx::tc_fence_after();
-                const uint32_t d_tmem = tmem_base + (uint32_t)(acc * SY_BN);
+                const uint32_t d_tmem = tmem_base + (uint32_t)(acc * BN);
                 for (int kb = kb0; kb < kb1; kb++) {
                     ptx::mbar_wait(&full[stage], phase);
                     if (p.phase_ctr) {
@@ -189,14 +225,18 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
                         }
                     }
                     ptx::tc_fence_after();
-                    const uint32_t a_addr = ptx::smem_u32(smem + stage * SY_STAGE_BYTES);
+                    const uint32_t a_addr = ptx::smem_u32(smem + stage * S::STAGE_BYTES);
                     const uint64_t a_desc = ptx::make_desc_k_sw128(a_addr);
                     const uint64_t b_desc = ptx::make_desc_k_sw128(a_addr + SY_A_BYTES);
 #pragma unroll
-                    for (int k = 0; k < SY_BK / 32; k++) {
-                        // advance 32 bytes along K inside the swizzle atom: +2 in 16-byte units
-                        ptx::umma_i8(d_tmem, a_desc + (uint64_t)(2 * k), b_desc + (uint64_t)(2 * k), idesc,
-                                     (kb > kb0 || k > 0) ? 1u : 0u);
+                    for (int k = 0; k < 4; k++) {
+                        // advance 32 bytes along K inside the swizzle atom (32 int8 / 64 E2M1): +2 in 16-byte units
+                        const uint32_t accum = (kb > kb0 || k > 0) ? 1u : 0u;
+                        if (FP4)
+                            ptx::umma_mxf4(d_tmem, a_desc + (uint64_t)(2 * k), b_desc + (uint64_t)(2 * k), idesc, sf_tmem,
+                                           sf_tmem + 32, accum);
+                        else
+                            ptx::umma_i8(d_tmem, a_desc + (uint64_t)(2 * k), b_desc + (uint64_t)(2 * k), idesc, accum);
                     }
                     ptx::umma_commit(&empty[stage]);  // frees the smem stage once these MMAs retire
                     if (++stage == SY_STAGES) { stage = 0; phase ^= 1; }
@@ -219,16 +259,18 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
             const int64_t row = row0 + lane;
             int32_t* crow = p.C + row * p.ldc;
 #pragma unroll 1
-            for (int c = 0; c < SY_BN / 32; c++) {
-                const int64_t col0 = (int64_t)t.y * SY_BN + c * 32;
+            for (int c = 0; c < BN / 32; c++) {
+                const int64_t col0 = (int64_t)t.y * BN + c * 32;
                 if (col0 + 31 < row0 || col0 >= p.n) continue;  // strictly lower triangle / out of range
                 uint32_t v[32];
-                ptx::tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * SY_BN + c * 32), v);
+                ptx::tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN + c * 32), v);
                 ptx::tmem_ld_wait();
                 if (row < p.n) {
 #pragma unroll
                     for (int j = 0; j < 32; j++) {
-                        if (col0 + j < p.n) atomicAdd(crow + col0 + j, (int32_t)v[j]);
+                        // E2M1: an FP32 integer (exact, see MMT_FP4_CHAIN) -> int32 by cvt.rni
+                        const int32_t x = FP4 ? __float2int_rn(__uint_as_float(v[j])) : (int32_t)v[j];
+                        if (col0 + j < p.n) atomicAdd(crow + col0 + j, x);
                     }
                 }
             }
@@ -244,6 +286,60 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const SyrkParams p) {
     if (warp == 1) {
         ptx::tc_fence_after();
         ptx::tmem_dealloc<SY_TMEM_COLS>(tmem_base);
+    }
+}
+
+template <bool KB>
+__global__ void __launch_bounds__(SY_THREADS, 1)
+syrk_i8_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap unused, const SyrkParams p) {
+    syrk_body<KB, false>(&tmap, &unused, p);
+}
+
+__global__ void __launch_bounds__(SY_THREADS, 1)
+syrk_fp4_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const SyrkParams p) {
+    syrk_body<true, true>(&tmA, &tmB, p);
+}
+
+// 4 genotype bytes (0x01, 0x00, 0xFF) -> 4 E2M1 nibbles (0x2, 0x0, 0xA), packed in pairs: the first of two markers in
+// the low nibble.  Returns 16 bits.
+__device__ __forceinline__ uint32_t e2m1_pairs(uint32_t w) {
+    const uint32_t t = ((w & 0x01010101u) << 1) | ((w >> 4) & 0x08080808u);  // one nibble in the low half of each byte
+    const uint32_t u = t | (t >> 4);                                         // bytes 0 and 2 hold the pairs
+    return (u & 0xFFu) | ((u >> 8) & 0xFF00u);
+}
+
+// Genotype store -> E2M1 operand [ceil(kcols/256)][n][128 B]: byte j of (block b, row r) holds markers 256 b + 2 j (low
+// nibble) and 256 b + 2 j + 1 (high nibble); markers >= kcols are 0.  pitch > 0: M row-major with that pitch; pitch == 0:
+// M K-blocked [ceil(kcols/128)][n][128].  One thread makes 16 output bytes from 32 input bytes.
+__global__ void __launch_bounds__(256) pack_e2m1_kernel(const int8_t* __restrict__ M, int64_t n, int64_t kcols, int64_t pitch,
+                                                        uint8_t* __restrict__ out, int64_t nblocks) {
+    const int64_t pieces = n * 8;
+    for (int64_t b = blockIdx.y; b < nblocks; b += gridDim.y) {
+        for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < pieces; j += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t r = j >> 3;
+            const int64_t m0 = b * 256 + (j & 7) * 32;  // first marker of this piece
+            uint4 lo = make_uint4(0, 0, 0, 0), hi = lo;
+            if (m0 < kcols) {
+                const int8_t* src = pitch ? M + r * pitch + m0 : M + ((m0 >> 7) * n + r) * 128 + (m0 & 127);
+                lo = __ldg(reinterpret_cast<const uint4*>(src));
+                hi = __ldg(reinterpret_cast<const uint4*>(src + 16));
+                if (m0 + 32 > kcols) {  // the store's padding is not relied upon
+                    const int valid = (int)(kcols - m0);
+                    auto keep = [valid](uint32_t w, int word) -> uint32_t {
+                        const int k = valid - 4 * word;
+                        return k >= 4 ? w : (k <= 0 ? 0u : w & ((1u << (8 * k)) - 1u));
+                    };
+                    lo = make_uint4(keep(lo.x, 0), keep(lo.y, 1), keep(lo.z, 2), keep(lo.w, 3));
+                    hi = make_uint4(keep(hi.x, 4), keep(hi.y, 5), keep(hi.z, 6), keep(hi.w, 7));
+                }
+            }
+            uint4 o;
+            o.x = e2m1_pairs(lo.x) | (e2m1_pairs(lo.y) << 16);
+            o.y = e2m1_pairs(lo.z) | (e2m1_pairs(lo.w) << 16);
+            o.z = e2m1_pairs(hi.x) | (e2m1_pairs(hi.y) << 16);
+            o.w = e2m1_pairs(hi.z) | (e2m1_pairs(hi.w) << 16);
+            *reinterpret_cast<uint4*>(out + (b * n + r) * 128 + (j & 7) * 16) = o;
+        }
     }
 }
 
@@ -269,103 +365,86 @@ struct TileTable {
     int device = -1;
     int2* d_tiles = nullptr;
     int ntiles = 0;
-    uint32_t* d_phase = nullptr;  // flow-control counters
-    size_t phase_cap = 0;
 };
-static thread_local TileTable g_tiles;
+static thread_local TileTable g_tiles[2];  // [FP4]: 128 x 256 (int8) and 128 x 224 (E2M1) tiles
+static thread_local uint32_t* g_phase = nullptr;  // flow-control counters
+static thread_local size_t g_phase_cap = 0;
+static thread_local int g_phase_device = -1;
 
-// tiles (ti, tj) with tj >= ti/2 (128-row x 256-column tiles touching the upper triangle), ordered
-// by super-rows of 16 tile rows, then tile column, then tile row.
-static int build_tiles(int64_t n, cudaStream_t st) {
+// tiles (ti, tj) of 128 x bn that touch the upper triangle ((tj + 1) bn > ti 128), ordered by super-rows of 16 tile
+// rows, then tile column, then tile row.
+static int build_tiles(TileTable& T, int64_t n, int bn, cudaStream_t st) {
     int dev = 0;
     EG_CUDA(cudaGetDevice(&dev));
-    if (g_tiles.n == n && g_tiles.device == dev && g_tiles.d_tiles) return EG_OK;
-    if (g_tiles.device != dev && g_tiles.d_phase) {
-        cudaFree(g_tiles.d_phase);
-        g_tiles.d_phase = nullptr;
-        g_tiles.phase_cap = 0;
-    }
-    const int TM = (int)((n + SY_BM - 1) / SY_BM), TN = (int)((n + SY_BN - 1) / SY_BN);
+    if (T.n == n && T.device == dev && T.d_tiles) return EG_OK;
+    const int TM = (int)((n + SY_BM - 1) / SY_BM), TN = (int)((n + bn - 1) / bn);
     std::vector<int2> h;
     for (int sr = 0; sr < TM; sr += 16)
-        for (int tj = sr >> 1; tj < TN; tj++)
+        for (int tj = (int)((int64_t)sr * SY_BM / bn); tj < TN; tj++)
             for (int ti = sr; ti < TM && ti < sr + 16; ti++)
-                if (tj >= (ti >> 1)) h.push_back(make_int2(ti, tj));
-    if (g_tiles.d_tiles) cudaFree(g_tiles.d_tiles);
-    g_tiles.d_tiles = nullptr;
-    EG_CUDA(cudaMalloc(&g_tiles.d_tiles, h.size() * sizeof(int2)));
-    EG_CUDA(cudaMemcpyAsync(g_tiles.d_tiles, h.data(), h.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
+                if ((int64_t)(tj + 1) * bn > (int64_t)ti * SY_BM) h.push_back(make_int2(ti, tj));
+    if (T.d_tiles) cudaFree(T.d_tiles);
+    T.d_tiles = nullptr;
+    EG_CUDA(cudaMalloc(&T.d_tiles, h.size() * sizeof(int2)));
+    EG_CUDA(cudaMemcpyAsync(T.d_tiles, h.data(), h.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
     EG_CUDA(cudaStreamSynchronize(st));
-    g_tiles.n = n;
-    g_tiles.device = dev;
-    g_tiles.ntiles = (int)h.size();
+    T.n = n;
+    T.device = dev;
+    T.ntiles = (int)h.size();
     return EG_OK;
 }
 
 void syrk_release_cache() {
-    if (g_tiles.d_tiles) cudaFree(g_tiles.d_tiles);
-    if (g_tiles.d_phase) cudaFree(g_tiles.d_phase);
-    g_tiles = TileTable();
+    for (TileTable& T : g_tiles) {
+        if (T.d_tiles) cudaFree(T.d_tiles);
+        T = TileTable();
+    }
+    if (g_phase) cudaFree(g_phase);
+    g_phase = nullptr;
+    g_phase_cap = 0;
+    g_phase_device = -1;
 }
 
-}  // namespace eg
+static int encode_kb(PFN_encodeTiled enc, CUtensorMap* tm, const void* base, int64_t rows, int64_t kblocks, uint32_t box_rows) {
+    const cuuint64_t gdim[3] = {128, (cuuint64_t)rows, (cuuint64_t)kblocks};
+    const cuuint64_t gstride[2] = {128, (cuuint64_t)rows * 128};
+    const cuuint32_t box[3] = {128, box_rows, 1};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    const CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(base), gdim, gstride, box, estr,
+                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS ? EG_OK : set_error(EG_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
+}
 
-static int syrk_launch(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitch, bool kblocked, int32_t* d_C,
-                       int64_t ldc, void* stream) {
-    using namespace eg;
-    if (!d_M || !d_C || n <= 0 || kcols < 0 || ldc < n || ((uintptr_t)d_M & 127) ||
-        (!kblocked && ((pitch & 127) || pitch < round_up(kcols, 128))))
-        return set_error(EG_ERR_ARG, "eg_dev_syrk_i8: bad argument");
-    if (kcols == 0) return EG_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    PFN_encodeTiled enc = get_encode_fn();
-    if (!enc) return set_error(EG_ERR_CUDA, "cuTensorMapEncodeTiled is not available (no CUDA driver?)");
-    EG_TRY(build_tiles(n, st));
-
-    CUtensorMap tmap;
-    const int64_t kblocks = (kcols + SY_BK - 1) / SY_BK;
-    CUresult r;
-    if (kblocked) {
-        const cuuint64_t gdim[3] = {128, (cuuint64_t)n, (cuuint64_t)kblocks};
-        const cuuint64_t gstride[2] = {128, (cuuint64_t)n * 128};
-        const cuuint32_t box[3] = {128, 128, 1};
-        const cuuint32_t estr[3] = {1, 1, 1};
-        r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<int8_t*>(d_M), gdim, gstride, box, estr,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else {
-        const cuuint64_t gdim[2] = {(cuuint64_t)round_up(kcols, 128), (cuuint64_t)n};
-        const cuuint64_t gstride[1] = {(cuuint64_t)pitch};
-        const cuuint32_t box[2] = {128, 128};
-        const cuuint32_t estr[2] = {1, 1};
-        r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<int8_t*>(d_M), gdim, gstride, box, estr,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    }
-    if (r != CUDA_SUCCESS) return set_error(EG_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-
+// Units, flow-control counters and the cooperative launch of either kernel.  kblocks: 128-B blocks along K;
+// min_blocks: the least a K split may leave per chunk; max_blocks: the most one chain may take.
+static int launch_units(void (*kern)(CUtensorMap, CUtensorMap, SyrkParams), const CUtensorMap& tmA, const CUtensorMap& tmB,
+                        const TileTable& T, int64_t n, int64_t kblocks, int min_blocks, int64_t max_blocks, int smem,
+                        int32_t* d_C, int64_t ldc, cudaStream_t st, const char* name) {
     SyrkParams p;
     p.n = n;
     p.ldc = ldc;
     p.C = d_C;
-    p.tiles = g_tiles.d_tiles;
-    p.ntiles = g_tiles.ntiles;
+    p.tiles = T.d_tiles;
+    p.ntiles = T.ntiles;
     p.kblocks_total = (int32_t)kblocks;
     const int sms = num_sms();
-    int kchunks = 1;
+    int64_t kchunks = 1;
     const int target = 4 * sms;
     if (p.ntiles < target) {
         kchunks = (target + p.ntiles - 1) / p.ntiles;
-        int maxc = p.kblocks_total / 32;  // at least 4096 markers per chunk
+        int64_t maxc = kblocks / min_blocks;
         if (maxc < 1) maxc = 1;
         if (kchunks > maxc) kchunks = maxc;
     }
-    p.kblocks_per_chunk = (p.kblocks_total + kchunks - 1) / kchunks;
-    kchunks = (p.kblocks_total + p.kblocks_per_chunk - 1) / p.kblocks_per_chunk;
-    p.nunits = p.ntiles * kchunks;
+    int64_t per = (kblocks + kchunks - 1) / kchunks;
+    if (per > max_blocks) per = max_blocks;
+    p.kblocks_per_chunk = (int32_t)per;
+    kchunks = (kblocks + per - 1) / per;
+    if ((int64_t)p.ntiles * kchunks > INT32_MAX) return set_error(EG_ERR_ARG, "%s: too many work units", name);
+    p.nunits = (int32_t)(p.ntiles * kchunks);
 
-    auto kern = kblocked ? syrk_i8_kernel<true> : syrk_i8_kernel<false>;
-    EG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SY_SMEM_BYTES));
+    EG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const int grid = p.nunits < sms ? p.nunits : sms;
 
     // flow-control counters: one per (round, phase); zeroed on the launch stream
@@ -376,27 +455,108 @@ static int syrk_launch(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitc
     const bool flow = !(env_fc && env_fc[0] == '0') && grid > 1;
     p.phase_ctr = nullptr;
     if (flow) {
-        if (nctr > g_tiles.phase_cap) {
-            if (g_tiles.d_phase) cudaFree(g_tiles.d_phase);
-            g_tiles.d_phase = nullptr;
-            EG_CUDA(cudaMalloc(&g_tiles.d_phase, nctr * sizeof(uint32_t)));
-            g_tiles.phase_cap = nctr;
+        if (nctr > g_phase_cap || g_phase_device != T.device) {
+            if (g_phase) cudaFree(g_phase);
+            g_phase = nullptr;
+            g_phase_cap = 0;
+            EG_CUDA(cudaMalloc(&g_phase, nctr * sizeof(uint32_t)));
+            g_phase_cap = nctr;
+            g_phase_device = T.device;
         }
-        EG_CUDA(cudaMemsetAsync(g_tiles.d_phase, 0, nctr * sizeof(uint32_t), st));
-        p.phase_ctr = g_tiles.d_phase;
+        EG_CUDA(cudaMemsetAsync(g_phase, 0, nctr * sizeof(uint32_t), st));
+        p.phase_ctr = g_phase;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(SY_THREADS);
-    cfg.dynamicSmemBytes = SY_SMEM_BYTES;
+    cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeCooperative;  // all CTAs co-resident: the soft barrier cannot deadlock
     attr[0].val.cooperative = flow ? 1 : 0;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    EG_CUDA(cudaLaunchKernelEx(&cfg, kern, tmap, p));
-    return check_launch("syrk_i8_kernel");
+    EG_CUDA(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, p));
+    return check_launch(name);
+}
+
+// markers per E2M1 accumulator chain: MMT_FP4_CHAIN, or EAGLE_MMT_FP4_CHUNK (the exactness probe of the tests: it also
+// turns the occupancy split off, so that every chain is exactly that long)
+static int64_t fp4_chunk_override() {
+    const char* e = getenv("EAGLE_MMT_FP4_CHUNK");
+    const long long v = e ? atoll(e) : 0;
+    return v > 0 ? (int64_t)v : 0;
+}
+
+}  // namespace eg
+
+static int syrk_i8_launch(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitch, bool kblocked, int32_t* d_C,
+                          int64_t ldc, cudaStream_t st) {
+    using namespace eg;
+    PFN_encodeTiled enc = get_encode_fn();
+    if (!enc) return set_error(EG_ERR_CUDA, "cuTensorMapEncodeTiled is not available (no CUDA driver?)");
+    EG_TRY(build_tiles(g_tiles[0], n, SyrkShape<false>::BN, st));
+    CUtensorMap tmap;
+    const int64_t kblocks = (kcols + SY_BK - 1) / SY_BK;
+    if (kblocked) {
+        EG_TRY(encode_kb(enc, &tmap, d_M, n, kblocks, 128));
+    } else {
+        const cuuint64_t gdim[2] = {(cuuint64_t)round_up(kcols, 128), (cuuint64_t)n};
+        const cuuint64_t gstride[1] = {(cuuint64_t)pitch};
+        const cuuint32_t box[2] = {128, 128};
+        const cuuint32_t estr[2] = {1, 1};
+        const CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<int8_t*>(d_M), gdim, gstride, box, estr,
+                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return set_error(EG_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
+    }
+    return launch_units(kblocked ? syrk_i8_kernel<true> : syrk_i8_kernel<false>, tmap, tmap, g_tiles[0], n, kblocks,
+                        32 /* >= 4096 markers per chunk */, INT32_MAX, SyrkShape<false>::SMEM_BYTES, d_C, ldc, st,
+                        "syrk_i8_kernel");
+}
+
+// pack to E2M1 into a pool block, then the E2M1 kernel; without room for the copy (half the store's bytes), the int8
+// kernel on the store itself gives the same integers
+static int syrk_fp4_launch(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitch, bool kblocked, int32_t* d_C,
+                           int64_t ldc, cudaStream_t st) {
+    using namespace eg;
+    PFN_encodeTiled enc = get_encode_fn();
+    if (!enc) return set_error(EG_ERR_CUDA, "cuTensorMapEncodeTiled is not available (no CUDA driver?)");
+    const int64_t kblocks = (kcols + 255) / 256;
+    void* ws = nullptr;
+    if (scratch_alloc(&ws, (size_t)kblocks * n * 128, st) != cudaSuccess)
+        return syrk_i8_launch(d_M, n, kcols, pitch, kblocked, d_C, ldc, st);
+    int rc = build_tiles(g_tiles[1], n, SyrkShape<true>::BN, st);
+    CUtensorMap tmA, tmB;
+    if (rc == EG_OK) rc = encode_kb(enc, &tmA, ws, n, kblocks, SY_BM);
+    if (rc == EG_OK) rc = encode_kb(enc, &tmB, ws, n, kblocks, SyrkShape<true>::BN);
+    if (rc == EG_OK) {
+        const int64_t xs = (n * 8 + 255) / 256;
+        const int64_t ys = kblocks < 65535 ? kblocks : 65535;
+        pack_e2m1_kernel<<<dim3((unsigned)(xs < 1024 ? xs : 1024), (unsigned)ys), 256, 0, st>>>(
+            d_M, n, kcols, kblocked ? 0 : pitch, reinterpret_cast<uint8_t*>(ws), kblocks);
+        rc = check_launch("pack_e2m1_kernel");
+    }
+    if (rc == EG_OK) {
+        const int64_t forced = fp4_chunk_override();
+        const int64_t chain = forced ? forced : MMT_FP4_CHAIN;
+        rc = launch_units(syrk_fp4_kernel, tmA, tmB, g_tiles[1], n, kblocks, forced ? INT32_MAX : 16 /* >= 4096 markers */,
+                          chain / 256 > 0 ? chain / 256 : 1, SyrkShape<true>::SMEM_BYTES, d_C, ldc, st, "syrk_fp4_kernel");
+    }
+    scratch_free(ws, st);
+    return rc;
+}
+
+static int syrk_launch(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitch, bool kblocked, int32_t* d_C,
+                       int64_t ldc, void* stream) {
+    using namespace eg;
+    if (!d_M || !d_C || n <= 0 || kcols < 0 || ldc < n || ((uintptr_t)d_M & 127) ||
+        (!kblocked && ((pitch & 127) || pitch < round_up(kcols, 128))))
+        return set_error(EG_ERR_ARG, "eg_dev_syrk_i8: bad argument");
+    if (kcols == 0) return EG_OK;
+    const char* mode = getenv("EAGLE_MMT_MODE");  // "i8": the int8 kernel; default: E2M1
+    if (mode && mode[0] == 'i') return syrk_i8_launch(d_M, n, kcols, pitch, kblocked, d_C, ldc, (cudaStream_t)stream);
+    return syrk_fp4_launch(d_M, n, kcols, pitch, kblocked, d_C, ldc, (cudaStream_t)stream);
 }
 
 extern "C" int eg_dev_syrk_i8(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitch, int32_t* d_C, int64_t ldc,

@@ -202,7 +202,9 @@ int eg_dev_transpose_kb_i8(const int8_t* d_in_kb, int64_t rows, int64_t cols, in
 int eg_dev_syrk_i8_kb(const int8_t* d_Mkb, int64_t n, int64_t kcols, int32_t* d_C, int64_t ldc, void* stream);
 /* K2: C (int32, n x n row-major, ld = ldc, must be zeroed by the caller) += M * M^T over columns
  * [0, kcols) of M (int8 n x kcols, row pitch multiple of 128 and padded with zeros).  Only entries
- * with col >= row are complete. */
+ * with col >= row are complete.  M holds genotypes in {-1, 0, +1}: by default both entry points copy
+ * it to E2M1 (a pool block of half its bytes) for the block-scaled FP4 kernel; EAGLE_MMT_MODE=i8
+ * contracts the int8 bytes themselves. */
 int eg_dev_syrk_i8(const int8_t* d_M, int64_t n, int64_t kcols, int64_t pitch, int32_t* d_C, int64_t ldc,
                    void* stream);
 /* C[r][c] -= sum_s M[r][zero_cols[s]] * M[c][zero_cols[s]]  (calculateMMt_rcpp.cpp:88-92 as a rank-k fix) */
