@@ -1,6 +1,6 @@
-// Host side of libeaglegpu.so: context, resident genotype stores + path cache, and the five
-// reference-facing entry points declared in include/eagle_gpu.h.  No CPU compute path exists
-// here: every entry point either runs the CUDA kernels or fails with an error code.
+// Host side of libeaglegpu.so: per-GPU contexts, resident genotype stores + path cache, the multi-GPU set, and the C
+// entry points of include/eagle_gpu.h (the reference-facing exports, the store API, device-level pieces and ingest).
+// No CPU compute path exists here: every entry point either runs the CUDA kernels or fails with an error code.
 #include <cublas_v2.h>
 #include <dlfcn.h>
 #include <fcntl.h>
@@ -152,58 +152,52 @@ int launch_scan(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const d
 // the driver pool from splitting a 10 GB block for an 800 MB request and then having to map 10 GB of fresh memory for
 // the next store -- measured as random 0.2 - 0.9 s stalls inside eg_store_from_host_ascii / eg_store_a_and_vara
 // (scripts/e2e_probe.py: steps of 540 ms turning into 1,200 - 1,400 ms).  Everything here is ordered on g_ctx.stream.
-#define g_pool_mu g_ctx.pool_mu
-#define g_free_blocks g_ctx.free_blocks
-#define g_live_blocks g_ctx.live_blocks
-#define g_free_bytes g_ctx.free_bytes
-#define g_recycle_limit g_ctx.recycle_limit
-
 static void pool_flush_locked() {
-    for (auto& b : g_free_blocks) cudaFreeAsync(b.p, g_ctx.stream);
-    g_free_blocks.clear();
-    g_free_bytes = 0;
+    for (auto& b : g_ctx.free_blocks) cudaFreeAsync(b.p, g_ctx.stream);
+    g_ctx.free_blocks.clear();
+    g_ctx.free_bytes = 0;
 }
 static cudaError_t pool_alloc(void** p, size_t bytes) {
     if (!bytes) bytes = 16;
-    std::lock_guard<std::mutex> lk(g_pool_mu);
-    for (size_t i = 0; i < g_free_blocks.size(); i++)
-        if (g_free_blocks[i].bytes == bytes) {
-            *p = g_free_blocks[i].p;
-            g_free_bytes -= bytes;
-            g_free_blocks.erase(g_free_blocks.begin() + i);
-            g_live_blocks[*p] = bytes;
+    std::lock_guard<std::mutex> lk(g_ctx.pool_mu);
+    for (size_t i = 0; i < g_ctx.free_blocks.size(); i++)
+        if (g_ctx.free_blocks[i].bytes == bytes) {
+            *p = g_ctx.free_blocks[i].p;
+            g_ctx.free_bytes -= bytes;
+            g_ctx.free_blocks.erase(g_ctx.free_blocks.begin() + i);
+            g_ctx.live_blocks[*p] = bytes;
             return cudaSuccess;
         }
     cudaError_t e = cudaMallocAsync(p, bytes, g_ctx.stream);
-    if (e != cudaSuccess && !g_free_blocks.empty()) {  // make room: give the recycled blocks back and try once more
+    if (e != cudaSuccess && !g_ctx.free_blocks.empty()) {  // make room: give the recycled blocks back and try once more
         cudaGetLastError();
         pool_flush_locked();
         cudaStreamSynchronize(g_ctx.stream);
         e = cudaMallocAsync(p, bytes, g_ctx.stream);
     }
-    if (e == cudaSuccess) g_live_blocks[*p] = bytes;
+    if (e == cudaSuccess) g_ctx.live_blocks[*p] = bytes;
     return e;
 }
 static void pool_free(void* p) {
     if (!p) return;
-    std::lock_guard<std::mutex> lk(g_pool_mu);
-    auto it = g_live_blocks.find(p);
-    const size_t bytes = it == g_live_blocks.end() ? 0 : it->second;
-    if (it != g_live_blocks.end()) g_live_blocks.erase(it);
-    if (bytes >= ((size_t)1 << 20) && g_free_bytes + bytes <= g_recycle_limit) {
-        g_free_blocks.push_back({p, bytes});
-        g_free_bytes += bytes;
+    std::lock_guard<std::mutex> lk(g_ctx.pool_mu);
+    auto it = g_ctx.live_blocks.find(p);
+    const size_t bytes = it == g_ctx.live_blocks.end() ? 0 : it->second;
+    if (it != g_ctx.live_blocks.end()) g_ctx.live_blocks.erase(it);
+    if (bytes >= ((size_t)1 << 20) && g_ctx.free_bytes + bytes <= g_ctx.recycle_limit) {
+        g_ctx.free_blocks.push_back({p, bytes});
+        g_ctx.free_bytes += bytes;
     } else {
         cudaFreeAsync(p, g_ctx.stream);
     }
 }
 static void pool_flush() {
-    std::lock_guard<std::mutex> lk(g_pool_mu);
+    std::lock_guard<std::mutex> lk(g_ctx.pool_mu);
     pool_flush_locked();
 }
 // For the plain cudaMalloc users of the library (LAPACK workspace, digit slices, host-level algebra buffers): when the
 // device is out of memory, hand the recycled blocks and the cached part of the stream-ordered pool back to the driver --
-// those bytes are invisible to cudaMalloc -- so that the caller can retry once.
+// those bytes are invisible to cudaMalloc -- so that the caller can retry once.  eg_cache_clear() uses it, too.
 void pool_give_back() {
     if (!g_ctx.ready) return;
     pool_flush();
@@ -344,6 +338,25 @@ static int store_alloc(int64_t rows, int64_t cols, bool kblocked, eg_store** out
     *out = s;
     return EG_OK;
 }
+// The end of every store built in this file: hand s out when rc is EG_OK, otherwise free it and pass rc on.
+static int finish_store(int rc, eg_store* s, eg_store** out) {
+    if (rc != EG_OK) {
+        free_store_tree(s);
+        return rc;
+    }
+    *out = s;
+    return EG_OK;
+}
+// The ASCII decoders' 4-int status (flag, row bits 0-30, column, row bits 31-) -> EG_ERR_FORMAT; row0 / col0: where the
+// decoded range starts in the image.
+static int decode_status(const int32_t* h_err, int64_t row0, int64_t col0) {
+    if (!h_err[0]) return EG_OK;
+    const int64_t brow = ((int64_t)h_err[3] << 31) | (int64_t)h_err[1];
+    return set_error(EG_ERR_FORMAT,
+                     "genotype file is not in no-space ASCII format: byte outside {'0','1','2'} near row %lld, column %lld "
+                     "(wrong dims / line pitch?)",
+                     (long long)(row0 + brow), (long long)(col0 + h_err[2]));
+}
 
 // K-blocked (M orientation) stores: the image is uploaded in COLUMN chunks (2-D copies, ~256 MB each, two staging
 // buffers); every chunk is decoded into its 128-marker blocks and its contribution to M * M^T is accumulated right
@@ -366,10 +379,7 @@ static int store_from_image_kb(const uint8_t* image, int64_t src_pitch_host, int
         s->C32 = nullptr;   // no room for the product: upload only
         eager = false;
     }
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
+    if (rc != EG_OK) return finish_store(rc, s, out);
     for (int i = 0; i < 2; i++) {
         cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
@@ -406,20 +416,8 @@ static int store_from_image_kb(const uint8_t* image, int64_t src_pitch_host, int
         cudaEventDestroy(copied[i]);
         cudaEventDestroy(decoded[i]);
     }
-    for (int64_t k = 0; k < nchunks && rc == EG_OK; k++)
-        if (h_err[4 * k]) {
-            const int64_t brow = ((int64_t)h_err[4 * k + 3] << 31) | (int64_t)h_err[4 * k + 1];
-            rc = set_error(EG_ERR_FORMAT,
-                           "genotype file is not in no-space ASCII format: byte outside {'0','1','2'} near row %lld, column %lld "
-                           "(wrong dims / line pitch?)",
-                           (long long)(row0 + brow), (long long)(col0 + k * cw + h_err[4 * k + 2]));
-        }
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
-    *out = s;
-    return EG_OK;
+    for (int64_t k = 0; k < nchunks && rc == EG_OK; k++) rc = decode_status(&h_err[4 * k], row0, col0 + k * cw);
+    return finish_store(rc, s, out);
 }
 
 // Host ASCII image -> store.  Rows [row0,row1), columns [col0,col1) of an image with `cols_total`
@@ -451,10 +449,7 @@ static int store_from_image(const uint8_t* image, int64_t cols_total, int64_t ro
     cudaEvent_t copied[2], decoded[2];
     int rc = EG_OK;
     for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc((size_t)block_rows * dev_pitch + 64, "ASCII staging");
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
+    if (rc != EG_OK) return finish_store(rc, s, out);
     for (int i = 0; i < 2; i++) {
         cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
@@ -505,19 +500,8 @@ static int store_from_image(const uint8_t* image, int64_t cols_total, int64_t ro
         cudaEventDestroy(copied[i]);
         cudaEventDestroy(decoded[i]);
     }
-    if (rc == EG_OK && h_err[0]) {
-        const int64_t brow = ((int64_t)h_err[3] << 31) | (int64_t)h_err[1];
-        rc = set_error(EG_ERR_FORMAT,
-                       "genotype file is not in no-space ASCII format: byte outside {'0','1','2'} near row %lld, column %lld "
-                       "(wrong dims / line pitch?)",
-                       (long long)(row0 + brow), (long long)(col0 + h_err[2]));
-    }
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
-    *out = s;
-    return EG_OK;
+    if (rc == EG_OK) rc = decode_status(h_err, row0, col0);
+    return finish_store(rc, s, out);
 }
 
 struct MappedFile {
@@ -724,80 +708,6 @@ __global__ void __launch_bounds__(256) symmetry_kernel(const double* __restrict_
     }
 }
 
-// ------------------------------------------------------------------ compute helpers on stores
-// keep_product: cache the int32 product with the store (stores of the path cache: calculateMMt_rcpp is called again by
-// SummaryAM with other selected loci, R/summary_am.R:142 -- the repeat then costs a copy, the rank-k correction and the
-// finalize pass instead of a second contraction)
-static int partial_product(const eg_store* M, const std::vector<int64_t>& zero_cols, DevBuf& C, bool keep_product);
-static int mmt_of_composite(const eg_store* M, const std::vector<int64_t>& zero_cols, double* out_host, bool keep_product);
-static int scan_of_composite(const eg_store* Mt, const std::vector<int64_t>& zero_rows, const double* S, const double* V,
-                             const double* a, double* out_a, double* out_vara);
-static int mmt_of_store(const eg_store* M, const std::vector<int64_t>& zero_cols, double* out_host, bool keep_product = false) {
-    Pin pin(M);
-    if (M->nparts > 1) return mmt_of_composite(M, zero_cols, out_host, keep_product);
-    const int64_t n = M->rows;
-    DevBuf C, D;
-    EG_TRY(partial_product(M, zero_cols, C, keep_product));
-    EG_TRY(D.alloc((size_t)n * n * sizeof(double), "MMt output"));
-    cudaStream_t st = g_ctx.stream;
-    {
-        Timer t(st);
-        EG_TRY(eg_dev_mmt_finalize(C.as<int32_t>(), n, n, D.as<double>(), st));
-        g_ctx.timing[2] = t.stop();
-    }
-    {
-        Timer t(st);
-        EG_TRY(d2h_staged(out_host, D.p, (size_t)n * n * sizeof(double), st));
-        g_ctx.timing[3] = t.stop();
-    }
-    return EG_OK;
-}
-
-static int scan_of_store(const eg_store* Mt, const std::vector<int64_t>& zero_rows, const double* S, const double* V,
-                         const double* a, double* out_a, double* out_vara) {
-    const int64_t L = Mt->rows, n = Mt->cols;
-    if (!Mt->pitch)
-        return set_error(EG_ERR_ARG, "the scan needs an Mt store (markers as rows); transpose the M store first");
-    Pin pin(Mt);
-    if (Mt->nparts > 1) return scan_of_composite(Mt, zero_rows, S, V, a, out_a, out_vara);
-    cudaStream_t st = g_ctx.stream;
-    DevBuf dS, dV, da, dT, dW, oa, ov;
-    EG_TRY(dS.alloc((size_t)n * n * 8, "inv_MMt_sqrt"));
-    EG_TRY(dV.alloc((size_t)n * n * 8, "dim_reduced_vara"));
-    EG_TRY(dT.alloc((size_t)n * n * 8, "scan scratch"));
-    EG_TRY(da.alloc((size_t)n * 8, "a"));
-    EG_TRY(dW.alloc((size_t)eg_scan_wp_elems(n) * 8, "packed W"));
-    EG_TRY(oa.alloc((size_t)L * 8, "a out"));
-    EG_TRY(ov.alloc((size_t)L * 8, "vara out"));
-    {
-        Timer t(st);
-        EG_TRY(h2d_staged(dS.p, S, (size_t)n * n * 8, st));   // R-owned (pageable) matrices: page-locked ring, parallel copiers
-        EG_TRY(h2d_staged(dV.p, V, (size_t)n * n * 8, st));
-        EG_CUDA(cudaMemcpyAsync(da.p, a, (size_t)n * 8, cudaMemcpyHostToDevice, st));
-        g_ctx.timing[4] = t.stop();
-    }
-    {
-        Timer t(st);
-        EG_TRY(eg_dev_scan_prepare(dS.as<double>(), dV.as<double>(), da.as<double>(), n, dT.as<double>(),
-                                   dW.as<double>(), st));
-        g_ctx.timing[5] = t.stop();
-    }
-    {
-        Timer t(st);
-        EG_TRY(eg_dev_scan(Mt->d, L, n, Mt->pitch, dW.as<double>(), zero_rows.empty() ? nullptr : zero_rows.data(),
-                           (int64_t)zero_rows.size(), oa.as<double>(), ov.as<double>(), st));
-        g_ctx.timing[6] = t.stop();
-    }
-    {
-        Timer t(st);
-        EG_CUDA(cudaMemcpyAsync(out_a, oa.p, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
-        EG_CUDA(cudaMemcpyAsync(out_vara, ov.p, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
-        EG_CUDA(cudaStreamSynchronize(st));
-        g_ctx.timing[7] = t.stop();
-    }
-    return EG_OK;
-}
-
 static void say(eg_message_fn message, void* ctx, const char* fmt, ...) {
     if (!message) return;
     char buf[512];
@@ -913,10 +823,12 @@ static bool multi_trace() {
     if (on < 0) { const char* e = getenv("EAGLE_MULTI_TRACE"); on = e && e[0] == '1'; }
     return on == 1;
 }
-#define MTRACE(...) do { if (multi_trace()) { fprintf(stderr, "[eagle gpu %d] ", g_ctx.device); fprintf(stderr, __VA_ARGS__); fputc('\n', stderr); fflush(stderr); } } while (0)
+#define MTRACE(...) do { if (t_is_worker && multi_trace()) { fprintf(stderr, "[eagle gpu %d] ", g_ctx.device); fprintf(stderr, __VA_ARGS__); fputc('\n', stderr); fflush(stderr); } } while (0)
 // Every GPU thread calls agree(my status so far); all return the same value: EG_OK, or the first failure's code.  The
-// thread that failed keeps its own message; the others get a short note.
+// thread that failed keeps its own message; the others get a short note.  Off the worker threads (a plain store worked on
+// by the calling thread as slot 0 of 1, also while a multi-GPU set exists) there is nobody to agree with: rc comes back.
 static int agree(int rc) {
+    if (!t_is_worker) return rc;
     WorkerPool& P = *g_multi.pool;
     std::unique_lock<std::mutex> lk(P.mu);
     if (rc != EG_OK && P.bar_rc == EG_OK) P.bar_rc = rc;
@@ -977,18 +889,22 @@ static int init_slot(Context& c, int device) {
     c.ready = true;
     return EG_OK;
 }
-// runs on the thread that owns the slot (its thread-local workspaces are released with it)
-static void shutdown_slot() {
-    if (!g_ctx.ready) return;
-    cudaSetDevice(g_ctx.device);
-    cudaDeviceSynchronize();
-    eg_cache_clear();
+// the calling thread's workspaces of the other translation units (thread-local: each thread releases its own)
+static void release_workspaces() {
     syrk_release_cache();
     scan_i8_release();
     prep_i8_release();
     algebra_release();
     eigbasis_release();
     hostio_release();
+}
+// runs on the thread that owns the slot (its thread-local workspaces are released with it)
+static void shutdown_slot() {
+    if (!g_ctx.ready) return;
+    cudaSetDevice(g_ctx.device);
+    cudaDeviceSynchronize();
+    eg_cache_clear();
+    release_workspaces();
     if (g_ctx.scan_ev[0]) { cudaEventDestroy(g_ctx.scan_ev[0]); cudaEventDestroy(g_ctx.scan_ev[1]); }
     if (g_ctx.cublas) cublasDestroy(g_ctx.cublas);
     if (g_ctx.stream) cudaStreamDestroy(g_ctx.stream);
@@ -1009,19 +925,19 @@ static int check_devices(int* ndev_out) {
 }
 
 // ------------------------------------------------------------------ marker-sharded (composite) stores
+// part r of a composite store; runs on the thread of GPU slot r (the part's memory belongs to that slot's pool)
+static void free_part(eg_store* S, int r) {
+    eg_store* p = S->part[r];
+    if (!p) return;
+    pool_free(p->C32);
+    pool_free(p->d);
+    delete p;
+    S->part[r] = nullptr;
+}
 static void free_store_tree(eg_store* s) {
     if (!s) return;
     if (s->nparts > 1) {
-        auto drop = [s](int r) {
-            eg_store* p = r < s->nparts ? s->part[r] : nullptr;
-            if (p) {
-                pool_free(p->C32);
-                pool_free(p->d);
-                delete p;
-            }
-            return EG_OK;
-        };
-        if (g_multi.n > 1 && g_multi.pool && !t_is_worker) run_all(drop);
+        if (g_multi.n > 1 && g_multi.pool && !t_is_worker) run_all([s](int r) { free_part(s, r); return EG_OK; });
         delete s;
         return;
     }
@@ -1064,12 +980,7 @@ static int store_from_image_any(const uint8_t* image, int64_t cols_total, int64_
     if (!image || row1 <= row0 || col1 <= col0 || col0 < 0 || col1 > cols_total || row0 < 0)
         return set_error(EG_ERR_ARG, "genotype store: bad image range");
     eg_store* S = new_composite(row1 - row0, col1 - col0, kblocked);
-    auto undo = [S]() {
-        run_all([S](int r) {
-            if (S->part[r]) { pool_free(S->part[r]->C32); pool_free(S->part[r]->d); delete S->part[r]; S->part[r] = nullptr; }
-            return EG_OK;
-        });
-    };
+    auto undo = [S]() { run_all([S](int r) { free_part(S, r); return EG_OK; }); };
     const int rc = run_all_evicting([&](int r) -> int {
         const int64_t a = S->off[r], b = S->off[r + 1];
         if (a == b) return EG_OK;
@@ -1088,7 +999,23 @@ static int store_from_image_any(const uint8_t* image, int64_t cols_total, int64_
     return EG_OK;
 }
 
+// ------------------------------------------------------------------ compute helpers on stores
+// A plain store is worked on as slot 0 of 1 on the calling thread, a composite one by every GPU slot on its own thread.
+static const eg_store* slot_part(const eg_store* S, int r) { return S->nparts > 1 ? S->part[r] : S; }
+static int on_each_slot(const eg_store* S, const std::function<int(int)>& fn) { return S->nparts > 1 ? run_all(fn) : fn(0); }
+// the entries of `idx` (markers of the whole store) that slot r holds, relative to its first marker
+static std::vector<int64_t> slot_indices(const eg_store* S, int r, const std::vector<int64_t>& idx) {
+    if (S->nparts <= 1) return idx;
+    std::vector<int64_t> z;
+    for (int64_t c : idx)
+        if (c >= S->off[r] && c < S->off[r + 1]) z.push_back(c - S->off[r]);
+    return z;
+}
+
 // Partial product of one plain store into C (n x n int32, zeroed / overwritten here), zeroed columns corrected.
+// keep_product: cache the int32 product with the store (stores of the path cache: calculateMMt_rcpp is called again by
+// SummaryAM with other selected loci, R/summary_am.R:142 -- the repeat then costs a copy, the rank-k correction and the
+// finalize pass instead of a second contraction)
 static int partial_product(const eg_store* M, const std::vector<int64_t>& zero_cols, DevBuf& C, bool keep_product) {
     const int64_t n = M->rows;
     cudaStream_t st = g_ctx.stream;
@@ -1119,81 +1046,89 @@ static int partial_product(const eg_store* M, const std::vector<int64_t>& zero_c
     return EG_OK;
 }
 
-// M.Mt of a composite store: every GPU contracts its marker shard, ONE int32 all-reduce (exact, order-free) over NVLink,
-// every GPU finalizes and returns its own block of rows of K to the host (the n x n result crosses PCIe once, in parallel).
-static int mmt_of_composite(const eg_store* M, const std::vector<int64_t>& zero_cols, double* out_host, bool keep_product) {
+// M.Mt, slot r of N: the slot contracts its marker shard; with several GPUs ONE int32 all-reduce (exact, order-free) over
+// NVLink follows; every slot finalizes and returns its own block of rows of K to the host (the n x n result crosses PCIe
+// once, in parallel).
+static int mmt_slot(const eg_store* M, int r, const std::vector<int64_t>& zero_cols, double* out_host, bool keep_product) {
     const int64_t n = M->rows;
-    const int N = M->nparts;
-    EG_TRY(run_all([&](int r) -> int {
-        cudaStream_t st = g_ctx.stream;
-        DevBuf C, D;
-        const eg_store* part = M->part[r];
-        auto local = [&]() -> int {
-            if (part) {
-                std::vector<int64_t> z;
-                for (int64_t c : zero_cols)
-                    if (c >= M->off[r] && c < M->off[r + 1]) z.push_back(c - M->off[r]);
-                EG_TRY(partial_product(part, z, C, keep_product));
-            } else {
-                EG_TRY(C.alloc((size_t)n * n * sizeof(int32_t), "MMt int32 accumulator"));
-                EG_CUDA(cudaMemsetAsync(C.p, 0, (size_t)n * n * sizeof(int32_t), st));
-            }
-            return D.alloc((size_t)n * n * sizeof(double), "MMt output");
-        };
-        MTRACE("mmt: partial product of markers [%lld, %lld)", (long long)M->off[r], (long long)M->off[r + 1]);
-        EG_TRY(agree(local()));
-        {
-            Timer t(st);
+    const int N = M->nparts > 1 ? M->nparts : 1;
+    cudaStream_t st = g_ctx.stream;
+    DevBuf C, D;
+    const eg_store* part = slot_part(M, r);
+    auto local = [&]() -> int {
+        if (part) {
+            EG_TRY(partial_product(part, slot_indices(M, r, zero_cols), C, keep_product));
+        } else {   // no markers on this GPU: zeros into the all-reduce
+            EG_TRY(C.alloc((size_t)n * n * sizeof(int32_t), "MMt int32 accumulator"));
+            EG_CUDA(cudaMemsetAsync(C.p, 0, (size_t)n * n * sizeof(int32_t), st));
+        }
+        return D.alloc((size_t)n * n * sizeof(double), "MMt output");
+    };
+    MTRACE("mmt: partial product of markers [%lld, %lld)", (long long)M->off[r], (long long)M->off[r + 1]);
+    EG_TRY(agree(local()));
+    {   // timing slot 2: the all-reduce with several GPUs, the finalize with one
+        Timer t(st);
+        if (N > 1) {
             MTRACE("mmt: all-reduce of %lld x %lld int32", (long long)n, (long long)n);
             EG_NCCL(g_nccl.AllReduce(C.p, C.p, (size_t)n * n, NCCL_INT32, NCCL_SUM, g_multi.comm[r], st));
-            g_ctx.timing[2] = t.stop();
+        } else {
+            EG_TRY(eg_dev_mmt_finalize(C.as<int32_t>(), n, n, D.as<double>(), st));
         }
-        EG_TRY(eg_dev_mmt_finalize(C.as<int32_t>(), n, n, D.as<double>(), st));
-        int64_t i0, i1;
-        shard_range(n, N, r, 1, &i0, &i1);
-        Timer t(st);
-        if (i1 > i0) EG_TRY(d2h_staged(out_host + i0 * n, D.as<double>() + i0 * n, (size_t)(i1 - i0) * n * sizeof(double), st));
-        EG_CUDA(cudaStreamSynchronize(st));
-        g_ctx.timing[3] = t.stop();
-        MTRACE("mmt: done");
-        return EG_OK;
-    }));
+        g_ctx.timing[2] = t.stop();
+    }
+    if (N > 1) EG_TRY(eg_dev_mmt_finalize(C.as<int32_t>(), n, n, D.as<double>(), st));
+    int64_t i0, i1;
+    shard_range(n, N, r, 1, &i0, &i1);
+    Timer t(st);
+    if (i1 > i0) EG_TRY(d2h_staged(out_host + i0 * n, D.as<double>() + i0 * n, (size_t)(i1 - i0) * n * sizeof(double), st));
+    EG_CUDA(cudaStreamSynchronize(st));
+    g_ctx.timing[3] = t.stop();
+    MTRACE("mmt: done");
     return EG_OK;
 }
+static int mmt_of_store(const eg_store* M, const std::vector<int64_t>& zero_cols, double* out_host, bool keep_product = false) {
+    Pin pin(M);
+    return on_each_slot(M, [&](int r) { return mmt_slot(M, r, zero_cols, out_host, keep_product); });
+}
 
-// The scan on a composite Mt store.  S and V cross PCIe once: GPU r uploads columns [k0_r, k1_r) of each and the blocks are
-// exchanged over NVLink (one grouped broadcast); the columns of W = S (V S) are split over the GPUs at equal cost and
-// exchanged the same way; every GPU scans its own markers and writes its slice of a / var(a) straight into the caller's
-// vectors.
-static int scan_of_composite(const eg_store* Mt, const std::vector<int64_t>& zero_rows, const double* S, const double* V,
-                             const double* a, double* out_a, double* out_vara) {
+// The scan, slot r of N.  S and V cross PCIe once: slot r uploads columns [k0_r, k1_r) of each and, with several GPUs, the
+// blocks are exchanged over NVLink (one grouped broadcast); when the pre-products take the digit-slice path the columns of
+// W = S (V S) are split over the GPUs at equal cost and exchanged the same way; every slot scans its own markers and writes
+// its slice of a / var(a) straight into the caller's vectors.  With one slot the cuts are [0, n) and the steps are those of
+// eg_dev_scan_prepare: symmetry check, zeroed Wp, all columns of W, fold.
+static int scan_slot(const eg_store* Mt, int r, const std::vector<int64_t>& zero_rows, const double* S, const double* V,
+                     const double* a, double* out_a, double* out_vara) {
     const int64_t n = Mt->cols;
-    const int N = Mt->nparts;
+    const int N = Mt->nparts > 1 ? Mt->nparts : 1;
     const int64_t Kpad = round_up(n, 32);
-    return run_all([&](int r) -> int {
-        cudaStream_t st = g_ctx.stream;
-        const eg_store* part = Mt->part[r];
-        const int64_t L = part ? part->rows : 0;
-        DevBuf dS, dV, da, dT, dW, oa, ov;
-        Timer t_up(st);
-        auto upload = [&]() -> int {
-            EG_TRY(dS.alloc((size_t)n * n * 8, "inv_MMt_sqrt"));
-            EG_TRY(dV.alloc((size_t)n * n * 8, "dim_reduced_vara"));
-            EG_TRY(da.alloc((size_t)n * 8, "a"));
-            EG_TRY(dW.alloc((size_t)eg_scan_wp_elems(n) * 8, "packed W"));
-            EG_TRY(oa.alloc((size_t)(L ? L : 1) * 8, "a out"));
-            EG_TRY(ov.alloc((size_t)(L ? L : 1) * 8, "vara out"));
-            int64_t k0, k1;
-            shard_range(n, N, r, 1, &k0, &k1);
-            if (k1 > k0) {
-                EG_TRY(h2d_staged(dS.as<double>() + k0 * n, S + k0 * n, (size_t)(k1 - k0) * n * 8, st));
-                EG_TRY(h2d_staged(dV.as<double>() + k0 * n, V + k0 * n, (size_t)(k1 - k0) * n * 8, st));
-            }
-            EG_CUDA(cudaMemcpyAsync(da.p, a, (size_t)n * 8, cudaMemcpyHostToDevice, st));
-            return EG_OK;
-        };
-        MTRACE("scan: upload of 1/%d of S and V", N);
-        EG_TRY(agree(upload()));
+    cudaStream_t st = g_ctx.stream;
+    const eg_store* part = slot_part(Mt, r);
+    const int64_t L = part ? part->rows : 0;
+    DevBuf dS, dV, da, dT, dW, oa, ov;
+    auto alloc = [&]() -> int {
+        EG_TRY(dS.alloc((size_t)n * n * 8, "inv_MMt_sqrt"));
+        EG_TRY(dV.alloc((size_t)n * n * 8, "dim_reduced_vara"));
+        EG_TRY(da.alloc((size_t)n * 8, "a"));
+        EG_TRY(dW.alloc((size_t)eg_scan_wp_elems(n) * 8, "packed W"));
+        EG_TRY(oa.alloc((size_t)(L ? L : 1) * 8, "a out"));
+        return ov.alloc((size_t)(L ? L : 1) * 8, "vara out");
+    };
+    const int rc_alloc = alloc();
+    Timer t_up(st);
+    auto upload = [&]() -> int {
+        EG_TRY(rc_alloc);
+        int64_t k0, k1;
+        shard_range(n, N, r, 1, &k0, &k1);
+        if (k1 > k0) {   // R-owned (pageable) matrices: page-locked ring, parallel copiers
+            EG_TRY(h2d_staged(dS.as<double>() + k0 * n, S + k0 * n, (size_t)(k1 - k0) * n * 8, st));
+            EG_TRY(h2d_staged(dV.as<double>() + k0 * n, V + k0 * n, (size_t)(k1 - k0) * n * 8, st));
+        }
+        EG_CUDA(cudaMemcpyAsync(da.p, a, (size_t)n * 8, cudaMemcpyHostToDevice, st));
+        return EG_OK;
+    };
+    MTRACE("scan: upload of 1/%d of S and V", N);
+    EG_TRY(agree(upload()));
+    if (N > 1) {
         EG_NCCL(g_nccl.GroupStart());
         for (int q = 0; q < N; q++) {
             int64_t q0, q1;
@@ -1203,61 +1138,68 @@ static int scan_of_composite(const eg_store* Mt, const std::vector<int64_t>& zer
             EG_NCCL(g_nccl.Broadcast(dV.as<double>() + q0 * n, dV.as<double>() + q0 * n, (size_t)(q1 - q0) * n, NCCL_FLOAT64, q, g_multi.comm[r], st));
         }
         EG_NCCL(g_nccl.GroupEnd());
-        g_ctx.timing[4] = t_up.stop();
-        Timer t_prep(st);
-        int sym = 0;
-        bool split = false;
-        std::vector<int64_t> cuts(N + 1, n);
-        auto products = [&]() -> int {
-            EG_TRY(eg_dev_inputs_symmetric(dS.as<double>(), dV.as<double>(), n, &sym, st));
-            split = sym && eg_prep_uses_i8(n);   // otherwise every GPU computes all of W itself (bit-identical to one GPU)
-            for (int q = 0; q < N; q++) {
-                if (split) {   // cost of columns [0,c): n c (V S) + c^2 / 2 (upper part of S X)  ->  equal-cost cuts
-                    int64_t c = (int64_t)llround((double)n * (sqrt(1.0 + 3.0 * q / N) - 1.0) / 32.0) * 32;
-                    cuts[q] = c < n ? c : n;
-                } else {
-                    cuts[q] = q == 0 ? 0 : n;
-                }
+    }
+    g_ctx.timing[4] = t_up.stop();
+    Timer t_prep(st);
+    int sym = 0;
+    bool split = false;
+    std::vector<int64_t> cuts(N + 1, n);
+    auto products = [&]() -> int {
+        EG_TRY(eg_dev_inputs_symmetric(dS.as<double>(), dV.as<double>(), n, &sym, st));
+        split = sym && eg_prep_uses_i8(n);   // otherwise every GPU computes all of W itself (bit-identical to one GPU)
+        for (int q = 0; q < N; q++) {
+            if (split) {   // cost of columns [0,c): n c (V S) + c^2 / 2 (upper part of S X)  ->  equal-cost cuts
+                int64_t c = (int64_t)llround((double)n * (sqrt(1.0 + 3.0 * q / N) - 1.0) / 32.0) * 32;
+                cuts[q] = c < n ? c : n;
+            } else {
+                cuts[q] = q == 0 ? 0 : n;
             }
-            int64_t widest = 1;
-            for (int q = 0; q < N; q++) widest = std::max(widest, cuts[q + 1] - cuts[q]);
-            EG_TRY(dT.alloc((size_t)n * (split ? widest : n) * 8, "scan scratch"));
-            EG_CUDA(cudaMemsetAsync(dW.p, 0, (size_t)eg_scan_wp_elems(n) * 8, st));
-            if (!split) return eg_dev_scan_prepare_cols(dS.as<double>(), dV.as<double>(), n, 0, n, sym, dT.as<double>(), dW.as<double>(), st);
-            return eg_dev_scan_prepare_cols(dS.as<double>(), dV.as<double>(), n, cuts[r], cuts[r + 1], sym, dT.as<double>(), dW.as<double>(), st);
-        };
-        MTRACE("scan: pre-products of my columns of W");
-        EG_TRY(agree(products()));
+        }
+        int64_t widest = 1;
+        for (int q = 0; q < N; q++) widest = std::max(widest, cuts[q + 1] - cuts[q]);
+        EG_TRY(dT.alloc((size_t)n * (split ? widest : n) * 8, "scan scratch"));
+        EG_CUDA(cudaMemsetAsync(dW.p, 0, (size_t)eg_scan_wp_elems(n) * 8, st));
+        return eg_dev_scan_prepare_cols(dS.as<double>(), dV.as<double>(), n, split ? cuts[r] : 0, split ? cuts[r + 1] : n, sym,
+                                        dT.as<double>(), dW.as<double>(), st);
+    };
+    MTRACE("scan: pre-products of my columns of W");
+    EG_TRY(agree(products()));
+    if (N > 1) {
         EG_NCCL(g_nccl.GroupStart());
         for (int q = 0; q < N && split; q++)
             if (cuts[q + 1] > cuts[q])
                 EG_NCCL(g_nccl.Broadcast(dW.as<double>() + cuts[q] * Kpad, dW.as<double>() + cuts[q] * Kpad,
                                          (size_t)(cuts[q + 1] - cuts[q]) * Kpad, NCCL_FLOAT64, q, g_multi.comm[r], st));
         EG_NCCL(g_nccl.GroupEnd());
-        EG_TRY(eg_dev_scan_fold(dS.as<double>(), da.as<double>(), n, sym, dW.as<double>(), st));
-        g_ctx.timing[5] = t_prep.stop();
-        MTRACE("scan: %lld markers", (long long)L);
-        if (L > 0) {
-            std::vector<int64_t> z;
-            for (int64_t c : zero_rows)
-                if (c >= Mt->off[r] && c < Mt->off[r + 1]) z.push_back(c - Mt->off[r]);
-            {
-                Timer t(st);
-                EG_TRY(eg_dev_scan(part->d, L, n, part->pitch, dW.as<double>(), z.empty() ? nullptr : z.data(), (int64_t)z.size(),
-                                   oa.as<double>(), ov.as<double>(), st));
-                g_ctx.timing[6] = t.stop();
-            }
+    }
+    EG_TRY(eg_dev_scan_fold(dS.as<double>(), da.as<double>(), n, sym, dW.as<double>(), st));
+    g_ctx.timing[5] = t_prep.stop();
+    MTRACE("scan: %lld markers", (long long)L);
+    if (L > 0) {
+        const std::vector<int64_t> z = slot_indices(Mt, r, zero_rows);
+        {
             Timer t(st);
-            EG_CUDA(cudaMemcpyAsync(out_a + Mt->off[r], oa.p, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
-            EG_CUDA(cudaMemcpyAsync(out_vara + Mt->off[r], ov.p, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
-            EG_CUDA(cudaStreamSynchronize(st));
-            g_ctx.timing[7] = t.stop();
-        } else {
-            EG_CUDA(cudaStreamSynchronize(st));
+            EG_TRY(eg_dev_scan(part->d, L, n, part->pitch, dW.as<double>(), z.empty() ? nullptr : z.data(), (int64_t)z.size(),
+                               oa.as<double>(), ov.as<double>(), st));
+            g_ctx.timing[6] = t.stop();
         }
-        MTRACE("scan: done");
-        return EG_OK;
-    });
+        Timer t(st);   // off[0] is 0 for every store, so a plain store's results start at out_a[0]
+        EG_CUDA(cudaMemcpyAsync(out_a + Mt->off[r], oa.p, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
+        EG_CUDA(cudaMemcpyAsync(out_vara + Mt->off[r], ov.p, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
+        EG_CUDA(cudaStreamSynchronize(st));
+        g_ctx.timing[7] = t.stop();
+    } else {
+        EG_CUDA(cudaStreamSynchronize(st));
+    }
+    MTRACE("scan: done");
+    return EG_OK;
+}
+static int scan_of_store(const eg_store* Mt, const std::vector<int64_t>& zero_rows, const double* S, const double* V,
+                         const double* a, double* out_a, double* out_vara) {
+    if (!Mt->pitch)
+        return set_error(EG_ERR_ARG, "the scan needs an Mt store (markers as rows); transpose the M store first");
+    Pin pin(Mt);
+    return on_each_slot(Mt, [&](int r) { return scan_slot(Mt, r, zero_rows, S, V, a, out_a, out_vara); });
 }
 }  // namespace eg
 
@@ -1337,20 +1279,11 @@ extern "C" int eg_gpu_count(void) { return g_multi.n > 1 ? g_multi.n : (g_ctxs[0
 extern "C" void eg_cache_clear(void) {
     for (auto& e : g_ctx.cache) free_store_tree(e.store);
     g_ctx.cache.clear();
-    if (g_multi.n > 1 && !t_is_worker && g_multi.pool)   // called by the user: the parts' pools live on the workers
-        run_all([](int) {
-            pool_flush();
-            cudaStreamSynchronize(g_ctx.stream);
-            cudaMemPool_t pool;
-            if (cudaDeviceGetDefaultMemPool(&pool, g_ctx.device) == cudaSuccess) cudaMemPoolTrimTo(pool, 0);
-            return EG_OK;
-        });
-    else if (g_ctx.ready) {
-        pool_flush();
-        cudaStreamSynchronize(g_ctx.stream);  // hand the recycled memory back to the driver
-        cudaMemPool_t pool;
-        if (cudaDeviceGetDefaultMemPool(&pool, g_ctx.device) == cudaSuccess) cudaMemPoolTrimTo(pool, 0);
-    }
+    // hand the recycled memory back to the driver; called by the user with a multi-GPU set: the parts' pools live on the workers
+    if (g_multi.n > 1 && !t_is_worker && g_multi.pool)
+        run_all([](int) { pool_give_back(); return EG_OK; });
+    else
+        pool_give_back();
 }
 
 extern "C" int eg_shutdown(void) {
@@ -1359,7 +1292,7 @@ extern "C" int eg_shutdown(void) {
         eg_cache_clear();   // composite stores: parts are freed on their own threads
         // the calling thread's own workspaces on device 0 (single-GPU entry points it ran itself)
         cudaSetDevice(g_ctxs[0].device);
-        syrk_release_cache(); scan_i8_release(); prep_i8_release(); algebra_release(); eigbasis_release(); hostio_release();
+        release_workspaces();
         run_all([](int r) {
             if (g_multi.comm[r]) g_nccl.CommDestroy(g_multi.comm[r]);
             g_multi.comm[r] = nullptr;
@@ -1401,24 +1334,22 @@ extern "C" int eg_get_scan_digits(void) { return scan_i8_digits(); }
 
 namespace eg {
 // CUDA events around the dominant scan kernel of the last eg_dev_scan call (for roofline reporting)
-#define g_scan_ev g_ctx.scan_ev
-#define g_scan_ops g_ctx.scan_ops
 void scan_kernel_mark(int which, cudaStream_t st, double ops) {
-    if (!g_scan_ev[0]) {
-        cudaEventCreate(&g_scan_ev[0]);
-        cudaEventCreate(&g_scan_ev[1]);
+    if (!g_ctx.scan_ev[0]) {
+        cudaEventCreate(&g_ctx.scan_ev[0]);
+        cudaEventCreate(&g_ctx.scan_ev[1]);
     }
-    cudaEventRecord(g_scan_ev[which], st);
-    if (which == 0) g_scan_ops = ops;
+    cudaEventRecord(g_ctx.scan_ev[which], st);
+    if (which == 0) g_ctx.scan_ops = ops;
 }
 }  // namespace eg
 extern "C" int eg_last_scan_kernel(double* ms, double* ops) {
-    if (!g_scan_ev[0] || !ms || !ops) return set_error(EG_ERR_ARG, "eg_last_scan_kernel: no scan has run");
-    EG_CUDA(cudaEventSynchronize(g_scan_ev[1]));
+    if (!g_ctx.scan_ev[0] || !ms || !ops) return set_error(EG_ERR_ARG, "eg_last_scan_kernel: no scan has run");
+    EG_CUDA(cudaEventSynchronize(g_ctx.scan_ev[1]));
     float f = 0;
-    EG_CUDA(cudaEventElapsedTime(&f, g_scan_ev[0], g_scan_ev[1]));
+    EG_CUDA(cudaEventElapsedTime(&f, g_ctx.scan_ev[0], g_ctx.scan_ev[1]));
     *ms = f;
-    *ops = g_scan_ops;
+    *ops = g_ctx.scan_ops;
     return EG_OK;
 }
 
@@ -1451,44 +1382,20 @@ extern "C" int eg_store_from_host_ascii_rows(const uint8_t* image, int64_t rows,
     return store_from_image_any(image, cols, row0, row1, 0, cols, false, out, true);  // Mt orientation: row-major
 }
 // ------------------------------------------------------------------ packed 2-bit container (pack2.cu)
-// Host words in, K-blocked (M orientation) or row-major (Mt orientation) store out: H2D of rows*wpr*8 bytes in two
-// row blocks overlapped with the unpack kernel.
+// Host words in, K-blocked (M orientation) or row-major (Mt orientation) store out: one H2D copy of the whole (4x smaller
+// than the store) rows*wpr*8 bytes, then the unpack kernel writes the store in its layout.
 extern "C" int eg_store_from_host_packed(const uint64_t* words, int64_t rows, int64_t cols, int kblocked, eg_store_t** out) {
     if (!words || !out || rows <= 0 || cols <= 0) return set_error(EG_ERR_ARG, "eg_store_from_host_packed: bad argument");
     EG_TRY(ensure_init());
     const int64_t wpr = eg_packed_words_per_row(cols);
-    if (kblocked) {
-        // K-blocked stores interleave the rows: unpack after the whole (4x smaller) image has landed
-        eg_store* s = nullptr;
-        EG_TRY(store_alloc(rows, cols, true, &s));
-        DevBuf w;
-        int rc = w.alloc((size_t)rows * wpr * 8, "packed genotype words");
-        Timer total(g_ctx.stream);
-        if (rc == EG_OK) rc = check_cuda(cudaMemcpyAsync(w.p, words, (size_t)rows * wpr * 8, cudaMemcpyHostToDevice, g_ctx.stream), "H2D of the packed genotypes");
-        if (rc == EG_OK) rc = check_cuda(cudaMemsetAsync(g_ctx.d_err, 0, 4 * sizeof(int32_t), g_ctx.stream), "memset");
-        if (rc == EG_OK) rc = eg_dev_unpack_2bit(w.as<uint64_t>(), rows, cols, s->d, 0, g_ctx.d_err, g_ctx.stream);
-        int32_t h_err[4] = {0, 0, 0, 0};
-        if (rc == EG_OK) rc = check_cuda(cudaMemcpyAsync(h_err, g_ctx.d_err, sizeof(h_err), cudaMemcpyDeviceToHost, g_ctx.stream), "status D2H");
-        if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "unpack");
-        g_ctx.timing[0] = total.stop();
-        if (rc == EG_OK && h_err[0])
-            rc = set_error(EG_ERR_FORMAT, "packed genotype container: code 3 or stray bits near row %lld, column %lld",
-                           (long long)(((int64_t)h_err[3] << 31) | h_err[1]), (long long)h_err[2]);
-        if (rc != EG_OK) {
-            eg_store_free(s);
-            return rc;
-        }
-        *out = s;
-        return EG_OK;
-    }
     eg_store* s = nullptr;
-    EG_TRY(store_alloc(rows, cols, false, &s));
+    EG_TRY(store_alloc(rows, cols, kblocked != 0, &s));
     DevBuf w;
     int rc = w.alloc((size_t)rows * wpr * 8, "packed genotype words");
     Timer total(g_ctx.stream);
     if (rc == EG_OK) rc = check_cuda(cudaMemcpyAsync(w.p, words, (size_t)rows * wpr * 8, cudaMemcpyHostToDevice, g_ctx.stream), "H2D of the packed genotypes");
     if (rc == EG_OK) rc = check_cuda(cudaMemsetAsync(g_ctx.d_err, 0, 4 * sizeof(int32_t), g_ctx.stream), "memset");
-    if (rc == EG_OK) rc = eg_dev_unpack_2bit(w.as<uint64_t>(), rows, cols, s->d, s->pitch, g_ctx.d_err, g_ctx.stream);
+    if (rc == EG_OK) rc = eg_dev_unpack_2bit(w.as<uint64_t>(), rows, cols, s->d, s->pitch, g_ctx.d_err, g_ctx.stream);  // pitch 0: K-blocked
     int32_t h_err[4] = {0, 0, 0, 0};
     if (rc == EG_OK) rc = check_cuda(cudaMemcpyAsync(h_err, g_ctx.d_err, sizeof(h_err), cudaMemcpyDeviceToHost, g_ctx.stream), "status D2H");
     if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "unpack");
@@ -1496,12 +1403,7 @@ extern "C" int eg_store_from_host_packed(const uint64_t* words, int64_t rows, in
     if (rc == EG_OK && h_err[0])
         rc = set_error(EG_ERR_FORMAT, "packed genotype container: code 3 or stray bits near row %lld, column %lld",
                        (long long)(((int64_t)h_err[3] << 31) | h_err[1]), (long long)h_err[2]);
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
-    *out = s;
-    return EG_OK;
+    return finish_store(rc, s, out);
 }
 // store -> host words (rows * eg_packed_words_per_row(cols) uint64): what an ingest step writes to disk once
 extern "C" int eg_store_to_host_packed(const eg_store_t* s, uint64_t* out_words) {
@@ -1552,12 +1454,7 @@ extern "C" int eg_store_drop_individuals(const eg_store_t* in, const int64_t* id
         rc = eg_dev_gather_cols(in->d, in->rows, in->pitch, dm.as<int64_t>(), n_out, s->d, s->pitch, g_ctx.stream);
     }
     if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "ReshapeM gather");  // `map` goes out of scope
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
-    *out = s;
-    return EG_OK;
+    return finish_store(rc, s, out);
 }
 
 extern "C" int eg_store_from_file(const char* path, int64_t rows, int64_t cols, int64_t col0, int64_t col1,
@@ -1576,12 +1473,7 @@ extern "C" int eg_store_transpose(const eg_store_t* in, eg_store_t** out) {
         if (in->mt_orientation) return set_error(EG_ERR_ARG, "eg_store_transpose: sharded Mt stores are not transposed back");
         eg_store* S = new_composite(in->cols, in->rows, false);
         for (int r = 0; r <= in->nparts; r++) S->off[r] = in->off[r];
-        auto undo = [S]() {
-            run_all([S](int r) {
-                if (S->part[r]) { pool_free(S->part[r]->d); delete S->part[r]; S->part[r] = nullptr; }
-                return EG_OK;
-            });
-        };
+        auto undo = [S]() { run_all([S](int r) { free_part(S, r); return EG_OK; }); };
         const int rc = run_all_evicting([&](int r) -> int {
             const eg_store* p = in->part[r];
             if (!p) return EG_OK;
@@ -1603,12 +1495,7 @@ extern "C" int eg_store_transpose(const eg_store_t* in, eg_store_t** out) {
     int rc = in->pitch ? eg_dev_transpose_i8(in->d, in->rows, in->cols, in->pitch, s->d, s->pitch, g_ctx.stream)
                        : eg_dev_transpose_kb_i8(in->d, in->rows, in->cols, s->d, s->pitch, g_ctx.stream);
     if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "transpose");
-    if (rc != EG_OK) {
-        eg_store_free(s);
-        return rc;
-    }
-    *out = s;
-    return EG_OK;
+    return finish_store(rc, s, out);
 }
 extern "C" int eg_store_free(eg_store_t* s) {
     if (!s) return EG_OK;
@@ -1939,6 +1826,68 @@ struct TextFile {
     }
 };
 
+// bytes of text the tokeniser works on at a time (EAGLE_INGEST_PIECE_BYTES overrides the 256 MB; at least 64)
+static int64_t ingest_piece_bytes() {
+    const char* envp = getenv("EAGLE_INGEST_PIECE_BYTES");
+    const int64_t piece_max = envp ? atoll(envp) : (256LL << 20);
+    return piece_max < 64 ? 64 : piece_max;
+}
+// a piece = whole lines: the piece starting at `off` ends after the last '\n' inside the window, or extends to the end of
+// a longer line
+static size_t piece_end(const TextFile& in, size_t off, int64_t piece_max) {
+    size_t end = off + (size_t)piece_max < in.size ? off + (size_t)piece_max : in.size;
+    if (end < in.size) {
+        const void* nlp = memrchr(in.p + off, '\n', end - off);
+        if (nlp) end = (size_t)((const uint8_t*)nlp - in.p) + 1;
+        else {
+            const void* nx = memchr(in.p + end, '\n', in.size - end);
+            end = nx ? (size_t)((const uint8_t*)nx - in.p) + 1 : in.size;
+        }
+    }
+    return end;
+}
+// A piece of text on the device and the tokeniser's chunk prefix over it (tokens and '\n' before every chunk); the buffers
+// grow to the largest piece seen.
+struct TokenisedPiece {
+    DevBuf text, counts, prefix;
+    size_t text_cap = 0, chunk_cap = 0;
+    // uploads piece[0, nb) and runs the tokeniser's scan; *newlines: the '\n' in the piece
+    int scan(const uint8_t* piece, int64_t nb, const char* what, int64_t* newlines, cudaStream_t st) {
+        const int64_t nch = eg_tokenise_chunks(nb);
+        if ((size_t)nb + 64 > text_cap) {
+            text_cap = (size_t)nb + 64;
+            EG_TRY(text.alloc(text_cap, what));
+        }
+        if ((size_t)nch > chunk_cap) {
+            chunk_cap = (size_t)nch;
+            EG_TRY(counts.alloc(chunk_cap * 2 * sizeof(uint32_t), "tokeniser counts"));
+            EG_TRY(prefix.alloc((chunk_cap + 1) * 2 * sizeof(int64_t), "tokeniser prefix"));
+        }
+        EG_CUDA(cudaMemcpyAsync(text.p, piece, (size_t)nb, cudaMemcpyHostToDevice, st));
+        EG_TRY(eg_dev_tokenise_scan(text.as<uint8_t>(), nb, counts.as<uint32_t>(), prefix.as<int64_t>(), st));
+        int64_t totals[2] = {0, 0};
+        EG_CUDA(cudaMemcpyAsync(totals, prefix.as<int64_t>() + 2 * nch, sizeof(totals), cudaMemcpyDeviceToHost, st));
+        EG_CUDA(cudaStreamSynchronize(st));
+        *newlines = totals[1];
+        return EG_OK;
+    }
+    // row and token count of the scanned piece before byte `pos` (an error event): the prefix of pos's chunk, then a walk
+    int counts_before(const uint8_t* piece, int64_t nb, int64_t pos, int64_t* row, int64_t* toks, cudaStream_t st) {
+        const int64_t cb = eg_tokenise_chunk_bytes();
+        const int64_t ch = (pos >= nb ? nb - 1 : pos) / cb;
+        int64_t pre[2];
+        EG_CUDA(cudaMemcpyAsync(pre, prefix.as<int64_t>() + 2 * ch, sizeof(pre), cudaMemcpyDeviceToHost, st));
+        EG_CUDA(cudaStreamSynchronize(st));
+        *toks = pre[0];
+        *row = pre[1];
+        for (int64_t q = ch * cb; q < pos; q++) {
+            if (piece[q] == '\n') (*row)++;
+            else if (!host_ws(piece[q]) && (q == 0 || host_ws(piece[q - 1]))) (*toks)++;
+        }
+        return EG_OK;
+    }
+};
+
 static void echo_first_lines(const TextFile& in, int nrowsp, int ncolsp, eg_message_fn message, void* mctx);
 
 // CreateASCIInospace(fname, asciifname, dims, AA, AB, BB, quiet, message, missing)   src/CreateASCIInospace.cpp:17-164
@@ -1963,45 +1912,22 @@ static int create_ascii_nospace(const char* fname, const char* asciifname, const
         say(message, mctx, "%s", "");
         say(message, mctx, " Loading file ");
     }
-    const char* envp = getenv("EAGLE_INGEST_PIECE_BYTES");
-    int64_t piece_max = envp ? atoll(envp) : (256LL << 20);
-    if (piece_max < 64) piece_max = 64;
+    const int64_t piece_max = ingest_piece_bytes();
     cudaStream_t st = g_ctx.stream;
-    DevBuf dtext, dout, dcounts, dprefix, derr;
+    TokenisedPiece tok;
+    DevBuf dout, derr;
     PinnedBuf hout;
     EG_TRY(derr.alloc(sizeof(uint64_t), "tokeniser status"));
-    size_t text_cap = 0, out_cap = 0, chunk_cap = 0;
+    size_t out_cap = 0;
     int64_t rows_done = 0;
     size_t off = 0;
     while (off < in.size) {
-        // a piece = whole lines: cut after the last '\n' inside the window, or extend to the end of a longer line
-        size_t end = off + (size_t)piece_max < in.size ? off + (size_t)piece_max : in.size;
-        if (end < in.size) {
-            const void* nlp = memrchr(in.p + off, '\n', end - off);
-            if (nlp) end = (size_t)((const uint8_t*)nlp - in.p) + 1;
-            else {
-                const void* nx = memchr(in.p + end, '\n', in.size - end);
-                end = nx ? (size_t)((const uint8_t*)nx - in.p) + 1 : in.size;
-            }
-        }
+        const size_t end = piece_end(in, off, piece_max);
         const int64_t nb = (int64_t)(end - off);
         const uint8_t* piece = in.p + off;
-        const int64_t nch = eg_tokenise_chunks(nb);
-        if ((size_t)nb + 64 > text_cap) {
-            text_cap = (size_t)nb + 64;
-            EG_TRY(dtext.alloc(text_cap, "text piece"));
-        }
-        if ((size_t)nch > chunk_cap) {
-            chunk_cap = (size_t)nch;
-            EG_TRY(dcounts.alloc(chunk_cap * 2 * sizeof(uint32_t), "tokeniser counts"));
-            EG_TRY(dprefix.alloc((chunk_cap + 1) * 2 * sizeof(int64_t), "tokeniser prefix"));
-        }
-        EG_CUDA(cudaMemcpyAsync(dtext.p, piece, (size_t)nb, cudaMemcpyHostToDevice, st));
-        EG_TRY(eg_dev_tokenise_scan(dtext.as<uint8_t>(), nb, dcounts.as<uint32_t>(), dprefix.as<int64_t>(), st));
-        int64_t totals[2] = {0, 0};
-        EG_CUDA(cudaMemcpyAsync(totals, dprefix.as<int64_t>() + 2 * nch, sizeof(totals), cudaMemcpyDeviceToHost, st));
-        EG_CUDA(cudaStreamSynchronize(st));
-        const int64_t lines = totals[1] + (piece[nb - 1] != '\n' ? 1 : 0);
+        int64_t newlines = 0;
+        EG_TRY(tok.scan(piece, nb, "text piece", &newlines, st));
+        const int64_t lines = newlines + (piece[nb - 1] != '\n' ? 1 : 0);
         const size_t out_bytes = (size_t)lines * (size_t)(L + 1);
         if (out_bytes + 16 > out_cap) {
             out_cap = out_bytes + 16;
@@ -2010,23 +1936,16 @@ static int create_ascii_nospace(const char* fname, const char* asciifname, const
         EG_TRY(hout.ensure(out_bytes + 16, "no-space ASCII rows"));
         uint64_t h_err = UINT64_MAX;
         EG_CUDA(cudaMemcpyAsync(derr.p, &h_err, sizeof(h_err), cudaMemcpyHostToDevice, st));
-        EG_TRY(eg_dev_tokenise_emit(dtext.as<uint8_t>(), nb, dprefix.as<int64_t>(), L, AA, AB, BB, missing, dout.as<uint8_t>(), lines,
-                                    derr.as<uint64_t>(), st));
+        EG_TRY(eg_dev_tokenise_emit(tok.text.as<uint8_t>(), nb, tok.prefix.as<int64_t>(), L, AA, AB, BB, missing, dout.as<uint8_t>(),
+                                    lines, derr.as<uint64_t>(), st));
         EG_CUDA(cudaMemcpyAsync(&h_err, derr.p, sizeof(h_err), cudaMemcpyDeviceToHost, st));
         EG_CUDA(cudaStreamSynchronize(st));
         int64_t good_rows = lines;
         if (h_err != UINT64_MAX) {
             // first error event of the piece: recover its row and what the reference would have printed
-            const int64_t pos = (int64_t)h_err, cb = eg_tokenise_chunk_bytes();
-            const int64_t ch = (pos >= nb ? nb - 1 : pos) / cb;
-            int64_t pre[2];
-            EG_CUDA(cudaMemcpyAsync(pre, dprefix.as<int64_t>() + 2 * ch, sizeof(pre), cudaMemcpyDeviceToHost, st));
-            EG_CUDA(cudaStreamSynchronize(st));
-            int64_t toks = pre[0], row = pre[1];
-            for (int64_t q = ch * cb; q < pos; q++) {
-                if (piece[q] == '\n') row++;
-                else if (!host_ws(piece[q]) && (q == 0 || host_ws(piece[q - 1]))) toks++;
-            }
+            const int64_t pos = (int64_t)h_err;
+            int64_t row = 0, toks = 0;
+            EG_TRY(tok.counts_before(piece, nb, pos, &row, &toks, st));
             good_rows = row;
             const long long row1 = (long long)(rows_done + row + 1);
             if (pos >= nb || piece[pos] == '\n') {  // :108-116
@@ -2110,46 +2029,24 @@ static int create_ascii_nospace_plink(const char* fname, const char* asciifname,
     OutFile outf;
     outf.f = fopen(asciifname, "wb");
     if (!outf.f) return set_error(EG_ERR_OPEN, "ERROR: Could not open  %s for writing", asciifname);
-    const char* envp = getenv("EAGLE_INGEST_PIECE_BYTES");
-    int64_t piece_max = envp ? atoll(envp) : (256LL << 20);
-    if (piece_max < 64) piece_max = 64;
+    const int64_t piece_max = ingest_piece_bytes();
     cudaStream_t st = g_ctx.stream;
-    DevBuf dtext, dall, dout, dcounts, dprefix, dstat, dstate;
+    TokenisedPiece tok;
+    DevBuf dall, dout, dstat, dstate;
     PinnedBuf hout;
     EG_TRY(dstat.alloc(3 * sizeof(uint64_t), "ped status"));
     EG_TRY(dstate.alloc((size_t)nsnp * 2, "allele state"));
-    size_t text_cap = 0, rows_cap = 0, chunk_cap = 0;
+    size_t rows_cap = 0;
     int64_t rows_done = 0;
     bool warned = false;
     size_t off = 0;
     while (off < in.size) {
-        size_t end = off + (size_t)piece_max < in.size ? off + (size_t)piece_max : in.size;
-        if (end < in.size) {
-            const void* nlp = memrchr(in.p + off, '\n', end - off);
-            if (nlp) end = (size_t)((const uint8_t*)nlp - in.p) + 1;
-            else {
-                const void* nx = memchr(in.p + end, '\n', in.size - end);
-                end = nx ? (size_t)((const uint8_t*)nx - in.p) + 1 : in.size;
-            }
-        }
+        const size_t end = piece_end(in, off, piece_max);
         const int64_t nb = (int64_t)(end - off);
         const uint8_t* piece = in.p + off;
-        const int64_t nch = eg_tokenise_chunks(nb);
-        if ((size_t)nb + 64 > text_cap) {
-            text_cap = (size_t)nb + 64;
-            EG_TRY(dtext.alloc(text_cap, "ped piece"));
-        }
-        if ((size_t)nch > chunk_cap) {
-            chunk_cap = (size_t)nch;
-            EG_TRY(dcounts.alloc(chunk_cap * 2 * sizeof(uint32_t), "tokeniser counts"));
-            EG_TRY(dprefix.alloc((chunk_cap + 1) * 2 * sizeof(int64_t), "tokeniser prefix"));
-        }
-        EG_CUDA(cudaMemcpyAsync(dtext.p, piece, (size_t)nb, cudaMemcpyHostToDevice, st));
-        EG_TRY(eg_dev_tokenise_scan(dtext.as<uint8_t>(), nb, dcounts.as<uint32_t>(), dprefix.as<int64_t>(), st));
-        int64_t totals[2] = {0, 0};
-        EG_CUDA(cudaMemcpyAsync(totals, dprefix.as<int64_t>() + 2 * nch, sizeof(totals), cudaMemcpyDeviceToHost, st));
-        EG_CUDA(cudaStreamSynchronize(st));
-        const int64_t lines = totals[1] + (piece[nb - 1] != '\n' ? 1 : 0);
+        int64_t newlines = 0;
+        EG_TRY(tok.scan(piece, nb, "ped piece", &newlines, st));
+        const int64_t lines = newlines + (piece[nb - 1] != '\n' ? 1 : 0);
         if ((size_t)lines > rows_cap) {
             rows_cap = (size_t)lines;
             EG_TRY(dall.alloc(rows_cap * (size_t)nsnp * 2 + 16, "allele characters"));
@@ -2158,21 +2055,15 @@ static int create_ascii_nospace_plink(const char* fname, const char* asciifname,
         EG_TRY(hout.ensure((size_t)lines * (size_t)(nsnp + 1) + 16, "no-space ASCII rows"));
         uint64_t h_stat[3] = {UINT64_MAX, UINT64_MAX, UINT64_MAX};  // stage-1 error position, third-allele key, missing key
         EG_CUDA(cudaMemcpyAsync(dstat.p, h_stat, sizeof(h_stat), cudaMemcpyHostToDevice, st));
-        EG_TRY(eg_dev_ped_alleles(dtext.as<uint8_t>(), nb, dprefix.as<int64_t>(), ncols, dall.as<uint8_t>(), lines, dstat.as<uint64_t>(), st));
+        EG_TRY(eg_dev_ped_alleles(tok.text.as<uint8_t>(), nb, tok.prefix.as<int64_t>(), ncols, dall.as<uint8_t>(), lines,
+                                  dstat.as<uint64_t>(), st));
         EG_CUDA(cudaMemcpyAsync(h_stat, dstat.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         EG_CUDA(cudaStreamSynchronize(st));
         int64_t good_rows = lines, bad_cols = -1;
         if (h_stat[0] != UINT64_MAX) {  // rows before the offending line are still processed, as in the reference
-            const int64_t pos = (int64_t)h_stat[0], cb = eg_tokenise_chunk_bytes();
-            const int64_t ch = (pos >= nb ? nb - 1 : pos) / cb;
-            int64_t pre[2];
-            EG_CUDA(cudaMemcpyAsync(pre, dprefix.as<int64_t>() + 2 * ch, sizeof(pre), cudaMemcpyDeviceToHost, st));
-            EG_CUDA(cudaStreamSynchronize(st));
-            int64_t toks = pre[0], row = pre[1];
-            for (int64_t q = ch * cb; q < pos; q++) {
-                if (piece[q] == '\n') row++;
-                else if (!host_ws(piece[q]) && (q == 0 || host_ws(piece[q - 1]))) toks++;
-            }
+            const int64_t pos = (int64_t)h_stat[0];
+            int64_t row = 0, toks = 0;
+            EG_TRY(tok.counts_before(piece, nb, pos, &row, &toks, st));
             if (!(pos >= nb || piece[pos] == '\n')) {
                 int64_t e = pos;
                 while (e < nb && !host_ws(piece[e])) e++;
@@ -2439,25 +2330,14 @@ extern "C" int eg_getRowColumn(const char* fname, int64_t* dimen) {
     if (!in.open_ro(fname)) return set_error(EG_ERR_OPEN, "\n\n ERROR: Could not open  %s\n\n\n", fname);  // :36-39
     dimen[0] = dimen[1] = 0;
     if (in.size == 0) return EG_OK;
-    const char* envp = getenv("EAGLE_INGEST_PIECE_BYTES");
-    int64_t piece_max = envp ? atoll(envp) : (256LL << 20);
-    if (piece_max < 64) piece_max = 64;
-    cudaStream_t st = g_ctx.stream;
-    DevBuf dtext, dcounts, dprefix;
+    const int64_t piece_max = ingest_piece_bytes();
     const int64_t cap = (int64_t)in.size < piece_max ? (int64_t)in.size : piece_max;
-    const int64_t nch_max = eg_tokenise_chunks(cap);
-    EG_TRY(dtext.alloc((size_t)cap + 64, "text piece"));
-    EG_TRY(dcounts.alloc((size_t)nch_max * 2 * sizeof(uint32_t), "tokeniser counts"));
-    EG_TRY(dprefix.alloc((size_t)(nch_max + 1) * 2 * sizeof(int64_t), "tokeniser prefix"));
-    for (size_t off = 0; off < in.size; off += (size_t)cap) {
+    TokenisedPiece tok;   // sized by the first (largest) piece
+    for (size_t off = 0; off < in.size; off += (size_t)cap) {   // fixed-size cuts: only '\n' are counted
         const int64_t nb = (int64_t)(in.size - off < (size_t)cap ? in.size - off : (size_t)cap);
-        const int64_t nch = eg_tokenise_chunks(nb);
-        EG_CUDA(cudaMemcpyAsync(dtext.p, in.p + off, (size_t)nb, cudaMemcpyHostToDevice, st));
-        EG_TRY(eg_dev_tokenise_scan(dtext.as<uint8_t>(), nb, dcounts.as<uint32_t>(), dprefix.as<int64_t>(), st));
-        int64_t totals[2] = {0, 0};
-        EG_CUDA(cudaMemcpyAsync(totals, dprefix.as<int64_t>() + 2 * nch, sizeof(totals), cudaMemcpyDeviceToHost, st));
-        EG_CUDA(cudaStreamSynchronize(st));
-        dimen[0] += totals[1];
+        int64_t newlines = 0;
+        EG_TRY(tok.scan(in.p + off, nb, "text piece", &newlines, g_ctx.stream));
+        dimen[0] += newlines;
     }
     if (in.p[in.size - 1] != '\n') dimen[0]++;
     const void* nlp = memchr(in.p, '\n', in.size);
