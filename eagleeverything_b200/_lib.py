@@ -70,6 +70,9 @@ SIGNATURES = {
     "eg_store_to_host_packed": (C.c_int, [_vp, _vp]),
     "eg_dev_pack_2bit": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _vp]),
     "eg_dev_unpack_2bit": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp, _vp]),
+    "eg_store_from_bed": (C.c_int, [C.c_char_p, _i64, _i64, _i64, _i64, C.c_int, _lp, C.POINTER(_vp)]),
+    "eg_store_from_host_bed": (C.c_int, [_vp, _i64, _i64, _i64, _i64, C.c_int, _lp, C.POINTER(_vp)]),
+    "eg_bed_to_ascii": (C.c_int, [C.c_char_p, _i64, _i64, C.c_char_p, C.c_char_p]),
     "eg_store_transpose": (C.c_int, [_vp, C.POINTER(_vp)]),
     "eg_store_free": (C.c_int, [_vp]),
     "eg_store_info": (C.c_int, [_vp, _lp, _lp, _lp, C.POINTER(_vp)]),
@@ -78,6 +81,7 @@ SIGNATURES = {
     "eg_store_extract_col": (C.c_int, [_vp, _i64, _ip]),
     "eg_dev_decode": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
     "eg_dev_decode_kb": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _vp, _i64, _i64, _vp, _vp]),
+    "eg_dev_decode_bed": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp]),
     "eg_dev_transpose_kb_i8": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp]),
     "eg_dev_syrk_i8_kb": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp]),
     "eg_dev_transpose_i8": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp]),

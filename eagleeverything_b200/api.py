@@ -147,6 +147,26 @@ def getRowColumn(fname):
     return [int(out[0]), int(out[1])]
 
 
+def plink_dims(prefix):
+    """(n, L) of a PLINK 1 binary data set: the lines of <prefix>.fam (one per individual) and of <prefix>.bim (one per
+    SNP), counted by eg_getRowColumn.  `prefix` may also be the path of the .bed file."""
+    prefix = os.fspath(prefix)
+    if prefix.endswith(".bed"):
+        prefix = prefix[:-4]
+    return getRowColumn(prefix + ".fam")[0], getRowColumn(prefix + ".bim")[0]
+
+
+def bed_to_ascii(bed_path, n, L, M_ascii, Mt_ascii):
+    """A SNP-major .bed file -> M.ascii and Mt.ascii as the text readers write them (include/eagle_gpu.h, eg_bed_to_ascii);
+    both stores stay resident under the two names for the calculateMMt_rcpp / calculate_a_and_vara_rcpp calls that follow."""
+    lib = _lib.require_gpu()
+    _lib.check(lib.eg_bed_to_ascii(os.fsencode(bed_path), int(n), int(L), os.fsencode(M_ascii), os.fsencode(Mt_ascii)))
+
+
+def _bed_bytes(n, L):
+    return 3 + int(L) * ((int(n) + 3) // 4)
+
+
 # ------------------------------------------------------------------ resident stores (host buffers in, handles out)
 class GenotypeStore:
     """A decoded int8 genotype matrix resident in HBM (eg_store_t)."""
@@ -189,6 +209,41 @@ class GenotypeStore:
         _lib.check(lib.eg_store_from_file(os.fsencode(path), rows, cols, col0, cols if col1 is None else col1,
                                           C.byref(h)))
         return cls(h.value)
+
+    @classmethod
+    def from_bed(cls, path, n, L, snp0=0, snp1=None, kblocked=True):
+        """SNPs [snp0, snp1) of a SNP-major PLINK .bed file (n individuals, L SNPs) -> the K-blocked M store (kblocked) or
+        the row-major Mt store.  The store's `n_missing` counts the missing genotypes read (stored as heterozygotes)."""
+        lib = _lib.require_gpu()
+        h, miss = C.c_void_p(), C.c_int64()
+        _lib.check(lib.eg_store_from_bed(os.fsencode(path), int(n), int(L), int(snp0), int(L if snp1 is None else snp1),
+                                         int(bool(kblocked)), C.byref(miss), C.byref(h)))
+        s = cls(h.value)
+        s.n_missing = miss.value
+        return s
+
+    @classmethod
+    def from_host_bed(cls, image, n, L, snp0=0, snp1=None, kblocked=True):
+        """As from_bed, from the whole file image in host memory: a numpy uint8 array (or bytes), or a CPU torch tensor --
+        page-locked ones (pin_memory()) are copied without staging."""
+        lib = _lib.require_gpu()
+        if hasattr(image, "data_ptr"):
+            if image.device.type != "cpu" or not image.is_contiguous():
+                raise ValueError("from_host_bed: a contiguous CPU tensor is needed")
+            size, ptr, keep = image.numel() * image.element_size(), image.data_ptr(), image
+        else:
+            keep = np.ascontiguousarray(np.frombuffer(image, dtype=np.uint8) if isinstance(image, (bytes, bytearray))
+                                        else image, dtype=np.uint8).reshape(-1)
+            size, ptr = keep.size, keep.ctypes.data
+        if size != _bed_bytes(n, L):
+            raise ValueError(f"a .bed image of {L} SNPs x {n} individuals has {_bed_bytes(n, L)} bytes, not {size}")
+        h, miss = C.c_void_p(), C.c_int64()
+        _lib.check(lib.eg_store_from_host_bed(C.c_void_p(ptr), int(n), int(L), int(snp0), int(L if snp1 is None else snp1),
+                                              int(bool(kblocked)), C.byref(miss), C.byref(h)))
+        del keep
+        s = cls(h.value)
+        s.n_missing = miss.value
+        return s
 
     def info(self):
         r, c, p = C.c_int64(), C.c_int64(), C.c_int64()

@@ -2350,3 +2350,174 @@ extern "C" int eg_getRowColumn(const char* fname, int64_t* dimen) {
     }
     return EG_OK;
 }
+
+// ================================================================== PLINK .bed (bed.cu; format in include/eagle_gpu.h)
+namespace eg {
+static int bed_check_range(int64_t n, int64_t L, int64_t snp0, int64_t snp1, const char* who) {
+    if (n <= 0 || L <= 0) return set_error(EG_ERR_ARG, "%s: n and L must be positive", who);
+    if (snp0 < 0 || snp1 > L || snp0 >= snp1)
+        return set_error(EG_ERR_ARG, "%s: SNP range [%lld, %lld) is empty or outside [0, %lld)", who, (long long)snp0,
+                         (long long)snp1, (long long)L);
+    return EG_OK;
+}
+static int bed_check_header(const uint8_t* h, const char* what) {
+    if (h[0] != 0x6C || h[1] != 0x1B)
+        return set_error(EG_ERR_FORMAT, "%s is not a PLINK .bed file: magic bytes %02x %02x, expected 6c 1b", what, h[0], h[1]);
+    if (h[2] == 0x00)
+        return set_error(EG_ERR_FORMAT, "%s is an individual-major .bed file (mode byte 0x00); only SNP-major files (mode 0x01) "
+                         "are read", what);
+    if (h[2] != 0x01) return set_error(EG_ERR_FORMAT, "%s: unknown .bed mode byte 0x%02x (0x01 = SNP-major)", what, h[2]);
+    return EG_OK;
+}
+// opens a .bed file and checks its header and size against (n, L)
+static int bed_open(const char* path, int64_t n, int64_t L, MappedFile& f) {
+    EG_TRY(f.open_ro(path));
+    if (f.size < 3) return set_error(EG_ERR_FORMAT, "%s is not a PLINK .bed file: %zu bytes", path, f.size);
+    EG_TRY(bed_check_header(f.p, path));
+    const size_t want = 3 + (size_t)L * (size_t)((n + 3) / 4);
+    if (f.size != want)
+        return set_error(EG_ERR_FORMAT, "%s has %zu bytes; a SNP-major .bed of %lld SNPs x %lld individuals has 3 + L * ceil(n/4) "
+                         "= %zu (wrong n / L, or a truncated file?)", path, f.size, (long long)L, (long long)n, want);
+    return EG_OK;
+}
+// SNPs [snp0, snp1) of a .bed image -> one plain store.  Pieces of whole 128-SNP blocks (EAGLE_INGEST_PIECE_BYTES bytes at
+// most) go through two device buffers: the staging of piece k+1 overlaps the decode of piece k.
+static int store_from_bed(const HostSrc& src, int64_t n, int64_t snp0, int64_t snp1, bool kblocked, uint64_t* n_missing,
+                          eg_store** out) {
+    EG_TRY(ensure_init());
+    const int64_t bpr = (n + 3) / 4, nsnp = snp1 - snp0;
+    int64_t piece = ingest_piece_bytes() / bpr / 128 * 128;
+    if (piece < 128) piece = 128;
+    if (piece > round_up(nsnp, 128)) piece = round_up(nsnp, 128);
+    eg_store* s = nullptr;
+    EG_TRY(kblocked ? store_alloc(n, nsnp, true, &s) : store_alloc(nsnp, n, false, &s));
+    DevBuf stg[2], dmiss;
+    int rc = EG_OK;
+    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc((size_t)piece * bpr, ".bed staging");
+    if (rc == EG_OK) rc = dmiss.alloc(sizeof(uint64_t), "missing genotype count");
+    if (rc != EG_OK) return finish_store(rc, s, out);
+    cudaEvent_t copied[2], decoded[2];
+    for (int i = 0; i < 2; i++) {
+        cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
+        cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
+    }
+    cudaMemsetAsync(dmiss.p, 0, sizeof(uint64_t), g_ctx.stream);
+    cudaEventRecord(decoded[0], g_ctx.stream);
+    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);  // the staging buffers were allocated in g_ctx.stream order
+    Timer total(g_ctx.stream);
+    int k = 0;
+    for (int64_t m = 0; m < nsnp && rc == EG_OK; m += piece, k++) {
+        const int b = k & 1;
+        const int64_t ns = m + piece <= nsnp ? piece : nsnp - m;
+        const size_t bytes = (size_t)ns * (size_t)bpr;
+        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);
+        rc = h2d_staged_2d(stg[b].p, bytes, src, 3 + (size_t)(snp0 + m) * (size_t)bpr, bytes, bytes, 1, g_ctx.copy_stream);
+        if (rc != EG_OK) break;
+        cudaEventRecord(copied[b], g_ctx.copy_stream);
+        cudaStreamWaitEvent(g_ctx.stream, copied[b], 0);
+        rc = eg_dev_decode_bed(stg[b].as<uint8_t>(), n, ns, s->d, nsnp, s->pitch, m, dmiss.as<uint64_t>(), g_ctx.stream);
+        cudaEventRecord(decoded[b], g_ctx.stream);
+    }
+    uint64_t h_miss = 0;
+    if (rc == EG_OK)
+        rc = check_cuda(cudaMemcpyAsync(&h_miss, dmiss.p, sizeof(h_miss), cudaMemcpyDeviceToHost, g_ctx.stream), "missing count D2H");
+    if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), ".bed decode");
+    cudaStreamSynchronize(g_ctx.copy_stream);
+    g_ctx.timing[0] = total.stop();  // H2D + decode (overlapped)
+    for (int i = 0; i < 2; i++) {
+        cudaEventDestroy(copied[i]);
+        cudaEventDestroy(decoded[i]);
+    }
+    *n_missing = h_miss;
+    return finish_store(rc, s, out);
+}
+// with a multi-GPU set (and allow_multi) a composite store: GPU r pulls and decodes the SNPs of its marker shard, one
+// contiguous byte range of the file
+static int store_from_bed_any(const HostSrc& src, int64_t n, int64_t snp0, int64_t snp1, bool kblocked, bool allow_multi,
+                              uint64_t* n_missing, eg_store** out) {
+    if (g_multi.n <= 1 || !allow_multi || t_is_worker) return store_from_bed(src, n, snp0, snp1, kblocked, n_missing, out);
+    EG_TRY(ensure_init());
+    eg_store* S = kblocked ? new_composite(n, snp1 - snp0, true) : new_composite(snp1 - snp0, n, false);
+    std::vector<uint64_t> miss((size_t)g_multi.n, 0);
+    auto undo = [S]() { run_all([S](int r) { free_part(S, r); return EG_OK; }); };
+    const int rc = run_all_evicting([&](int r) -> int {
+        const int64_t a = S->off[r], b = S->off[r + 1];
+        if (a == b) return EG_OK;
+        return store_from_bed(src, n, snp0 + a, snp0 + b, kblocked, &miss[(size_t)r], &S->part[r]);
+    }, undo);
+    if (rc != EG_OK) {
+        const std::string msg = g_err;
+        undo();
+        delete S;
+        return set_error(rc, "%s", msg.c_str());
+    }
+    *n_missing = 0;
+    g_ctx.timing[0] = 0;
+    for (int r = 0; r < g_multi.n; r++) {
+        *n_missing += miss[(size_t)r];
+        g_ctx.timing[0] = std::max(g_ctx.timing[0], g_ctxs[r].timing[0]);
+    }
+    *out = S;
+    return EG_OK;
+}
+}  // namespace eg
+
+extern "C" int eg_store_from_bed(const char* path, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked, int64_t* n_missing,
+                                 eg_store_t** out) {
+    if (!path || !out) return set_error(EG_ERR_ARG, "eg_store_from_bed: null argument");
+    EG_TRY(bed_check_range(n, L, snp0, snp1, "eg_store_from_bed"));
+    MappedFile f;
+    EG_TRY(bed_open(path, n, L, f));
+    HostSrc src;
+    src.p = f.p;
+    src.fd = f.fd;
+    uint64_t miss = 0;
+    EG_TRY(store_from_bed_any(src, n, snp0, snp1, kblocked != 0, true, &miss, out));
+    if (n_missing) *n_missing = (int64_t)miss;
+    return EG_OK;
+}
+extern "C" int eg_store_from_host_bed(const uint8_t* image, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked,
+                                      int64_t* n_missing, eg_store_t** out) {
+    if (!image || !out) return set_error(EG_ERR_ARG, "eg_store_from_host_bed: null argument");
+    EG_TRY(bed_check_range(n, L, snp0, snp1, "eg_store_from_host_bed"));
+    EG_TRY(bed_check_header(image, "the image"));
+    HostSrc src;
+    src.p = image;
+    uint64_t miss = 0;
+    EG_TRY(store_from_bed_any(src, n, snp0, snp1, kblocked != 0, true, &miss, out));
+    if (n_missing) *n_missing = (int64_t)miss;
+    return EG_OK;
+}
+// One read of the .bed file into the K-blocked M store; its transpose is the Mt store, and the transpose of that the
+// row-major M the ASCII encoder needs for M.ascii.  M and Mt stay cached under the two file names (as createMt_ASCII_rcpp
+// leaves them).
+extern "C" int eg_bed_to_ascii(const char* bed_path, int64_t n, int64_t L, const char* M_ascii, const char* Mt_ascii) {
+    if (!bed_path || !M_ascii || !Mt_ascii) return set_error(EG_ERR_ARG, "eg_bed_to_ascii: null argument");
+    EG_TRY(bed_check_range(n, L, 0, L, "eg_bed_to_ascii"));
+    eg_store *M = nullptr, *Mt = nullptr, *Mrm = nullptr;
+    {
+        MappedFile f;
+        EG_TRY(bed_open(bed_path, n, L, f));
+        HostSrc src;
+        src.p = f.p;
+        src.fd = f.fd;
+        uint64_t miss = 0;
+        EG_TRY(store_from_bed_any(src, n, 0, L, true, false, &miss, &M));
+    }
+    int rc = eg_store_transpose(M, &Mt);
+    if (rc == EG_OK) rc = write_store_ascii(Mt, Mt_ascii);
+    if (rc == EG_OK) rc = eg_store_transpose(Mt, &Mrm);
+    if (rc == EG_OK) rc = write_store_ascii(Mrm, M_ascii);
+    eg_store_free(Mrm);
+    if (rc != EG_OK) {
+        eg_store_free(Mt);
+        eg_store_free(M);
+        return rc;
+    }
+    std::string key;
+    if (cache_key(M_ascii, n, L, true, key) == EG_OK) cache_insert(key, M);
+    else eg_store_free(M);
+    if (cache_key(Mt_ascii, L, n, false, key) == EG_OK) cache_insert(key, Mt);
+    else eg_store_free(Mt);
+    return EG_OK;
+}

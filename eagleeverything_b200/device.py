@@ -71,6 +71,25 @@ def decode_kb(img, src_pitch, rows, cols, out=None, err=None, src_offset=0):
     return out, err
 
 
+def decode_bed(bed, n, L, kblocked=True, out=None, missing=None):
+    """A SNP-major PLINK .bed file image in HBM (uint8 tensor, header included) -> the K-blocked M store
+    (ceil(L/128), n, 128) like decode_kb, or (kblocked=False) the row-major Mt store (L, pitch(n)) like transpose_kb.
+    missing: optional one-element int64 tensor that accumulates the number of missing genotypes."""
+    lib = _lib.load()
+    bpr = (n + 3) // 4
+    if bed.numel() != 3 + L * bpr:
+        raise ValueError(f"a .bed image of {L} SNPs x {n} individuals has {3 + L * bpr} bytes, not {bed.numel()}")
+    head = bytes(bed[:3].cpu().tolist())
+    if head != b"\x6c\x1b\x01":
+        raise ValueError(f"not a SNP-major PLINK .bed image (header {head.hex()}, expected 6c1b01)")
+    if out is None:
+        shape = ((L + 127) // 128, n, 128) if kblocked else (L, store_pitch(n))
+        out = torch.empty(shape, dtype=torch.int8, device=bed.device)
+    _lib.check(lib.eg_dev_decode_bed(C.c_void_p(bed.data_ptr() + 3), n, L, _ptr(out), L, 0 if kblocked else out.stride(0), 0,
+                                     None if missing is None else _ptr(missing), _stream()))
+    return out
+
+
 def transpose_kb(store_kb, rows, cols, out=None):
     """K-blocked M store (ceil(cols/128), rows, 128) -> row-major Mt store (cols, pitch(rows))."""
     lib = _lib.load()

@@ -170,6 +170,30 @@ int eg_store_to_host_packed(const eg_store_t* s, uint64_t* out_words);
 int eg_dev_pack_2bit(const int8_t* d_store, int64_t rows, int64_t cols, int64_t pitch, uint64_t* d_words, void* stream);
 int eg_dev_unpack_2bit(const uint64_t* d_words, int64_t rows, int64_t cols, int8_t* d_store, int64_t pitch, int32_t* d_err,
                        void* stream);
+/* PLINK 1 binary genotypes: a .bed file (with its .bim, one line per SNP, and .fam, one line per individual) straight into
+ * a store, 4 genotypes per byte over PCIe instead of 1 (csrc/bed.cu).  The format read:
+ *   header    0x6C 0x1B 0x01 (SNP-major).  Refused with EG_ERR_FORMAT: mode byte 0x00 (individual-major), any other magic,
+ *             and (files) a size that is not exactly 3 + L * ceil(n/4);
+ *   layout    SNP j in bytes 3 + j*bpr .. 3 + (j+1)*bpr - 1, bpr = ceil(n/4); individual i of it is
+ *             v = (byte[i/4] >> 2*(i%4)) & 3.  The bits past individual n-1 in a SNP's last byte are ignored;
+ *   values    v = 0 homozygous for the first .bim allele (A1) -> code 0 (AA, store +1); v = 2 heterozygous -> code 1 (AB,
+ *             store 0); v = 3 homozygous A2 -> code 2 (BB, store -1); v = 1 missing -> code 1, a heterozygote, as missing
+ *             text tokens and ped alleles are read.  Swapping A1 / A2 of a SNP negates its column: M.Mt, var(a) and the
+ *             picks do not change, a and extracted genotypes change sign.
+ * n and L come from the line counts of .fam and .bim (eg_getRowColumn); names and positions stay with the map file.
+ * SNPs [snp0, snp1) make the store (a marker shard; 0, L for everything); kblocked != 0: the K-blocked M store
+ * (n x (snp1 - snp0)), else the row-major Mt store ((snp1 - snp0) x n).  *n_missing (may be NULL): missing genotypes read.
+ * Header, size and ranges are checked before any device work.  The bytes go through the page-locked staging ring in
+ * pieces (pread for the file), each piece decoded while the next is copied; with eg_init_multi every GPU pulls and decodes
+ * only its own SNP range (one contiguous byte range of the file).  `image` is the whole file image, header included. */
+int eg_store_from_bed(const char* path, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked, int64_t* n_missing,
+                      eg_store_t** out);
+int eg_store_from_host_bed(const uint8_t* image, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked,
+                           int64_t* n_missing, eg_store_t** out);
+/* A .bed file -> M.ascii (n lines of L characters) and Mt.ascii (L lines of n), byte-identical to what the text readers
+ * write for the same genotypes; both stores stay in the path cache under those names, so the calculateMMt_rcpp /
+ * calculate_a_and_vara_rcpp calls that follow upload nothing.  How an R user brings a .bed file to AM(). */
+int eg_bed_to_ascii(const char* bed_path, int64_t n, int64_t L, const char* M_ascii, const char* Mt_ascii);
 int eg_store_free(eg_store_t* s);
 int eg_store_info(const eg_store_t* s, int64_t* rows, int64_t* cols, int64_t* pitch, void** device_ptr);
 
@@ -197,6 +221,13 @@ int eg_dev_transpose_i8(const int8_t* d_in, int64_t rows, int64_t cols, int64_t 
 /* K-blocked variants: the store is [ceil(cols/128)][kb_rows][128] bytes; decode fills rows [row0, row0+rows). */
 int eg_dev_decode_kb(const uint8_t* d_src, int64_t src_pitch, int64_t src_bytes_avail, int64_t rows, int64_t cols,
                      int8_t* d_dst, int64_t kb_rows, int64_t row0, int32_t* d_err, void* stream);
+/* .bed SNP rows -> store (format: eg_store_from_bed).  d_snps: nsnp rows of ceil(n/4) bytes at any alignment; they become
+ * markers [m0, m0 + nsnp) of a store of dst_rows_or_L markers, pads written as eg_dev_decode / eg_dev_decode_kb write them.
+ * dst_pitch > 0: row-major Mt store (row pitch, multiple of 128, >= n); dst_pitch == 0: K-blocked M store
+ * [ceil(L/128)][n][128] with L = dst_rows_or_L, where m0 is a multiple of 128 and nsnp is one too unless the piece ends at
+ * L.  *d_missing (may be NULL) += the missing genotypes of the piece. */
+int eg_dev_decode_bed(const uint8_t* d_snps, int64_t n, int64_t nsnp, int8_t* d_dst, int64_t dst_rows_or_L, int64_t dst_pitch,
+                      int64_t m0, uint64_t* d_missing, void* stream);
 int eg_dev_transpose_kb_i8(const int8_t* d_in_kb, int64_t rows, int64_t cols, int8_t* d_out, int64_t out_pitch,
                            void* stream);
 int eg_dev_syrk_i8_kb(const int8_t* d_Mkb, int64_t n, int64_t kcols, int32_t* d_C, int64_t ldc, void* stream);
