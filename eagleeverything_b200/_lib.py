@@ -73,6 +73,9 @@ SIGNATURES = {
     "eg_store_from_bed": (C.c_int, [C.c_char_p, _i64, _i64, _i64, _i64, C.c_int, _lp, C.POINTER(_vp)]),
     "eg_store_from_host_bed": (C.c_int, [_vp, _i64, _i64, _i64, _i64, C.c_int, _lp, C.POINTER(_vp)]),
     "eg_bed_to_ascii": (C.c_int, [C.c_char_p, _i64, _i64, C.c_char_p, C.c_char_p]),
+    "eg_store_stream_file": (C.c_int, [C.c_char_p, _i64, _i64, C.c_int, C.POINTER(_vp)]),
+    "eg_store_stream_bed": (C.c_int, [C.c_char_p, _i64, _i64, _i64, _i64, C.c_int, C.POINTER(_vp)]),
+    "eg_store_stream_host_bed": (C.c_int, [_vp, _i64, _i64, _i64, _i64, C.c_int, C.POINTER(_vp)]),
     "eg_store_transpose": (C.c_int, [_vp, C.POINTER(_vp)]),
     "eg_store_free": (C.c_int, [_vp]),
     "eg_store_info": (C.c_int, [_vp, _lp, _lp, _lp, C.POINTER(_vp)]),

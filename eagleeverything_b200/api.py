@@ -167,6 +167,17 @@ def _bed_bytes(n, L):
     return 3 + int(L) * ((int(n) + 3) // 4)
 
 
+def _host_bytes(image, who):
+    """(object that owns the bytes, size, address) of a .bed image: numpy uint8 array, bytes, or a contiguous CPU tensor."""
+    if hasattr(image, "data_ptr"):
+        if image.device.type != "cpu" or not image.is_contiguous():
+            raise ValueError(f"{who}: a contiguous CPU tensor is needed")
+        return image, image.numel() * image.element_size(), image.data_ptr()
+    keep = np.ascontiguousarray(np.frombuffer(image, dtype=np.uint8) if isinstance(image, (bytes, bytearray))
+                                else image, dtype=np.uint8).reshape(-1)
+    return keep, keep.size, keep.ctypes.data
+
+
 # ------------------------------------------------------------------ resident stores (host buffers in, handles out)
 class GenotypeStore:
     """A decoded int8 genotype matrix resident in HBM (eg_store_t)."""
@@ -227,14 +238,7 @@ class GenotypeStore:
         """As from_bed, from the whole file image in host memory: a numpy uint8 array (or bytes), or a CPU torch tensor --
         page-locked ones (pin_memory()) are copied without staging."""
         lib = _lib.require_gpu()
-        if hasattr(image, "data_ptr"):
-            if image.device.type != "cpu" or not image.is_contiguous():
-                raise ValueError("from_host_bed: a contiguous CPU tensor is needed")
-            size, ptr, keep = image.numel() * image.element_size(), image.data_ptr(), image
-        else:
-            keep = np.ascontiguousarray(np.frombuffer(image, dtype=np.uint8) if isinstance(image, (bytes, bytearray))
-                                        else image, dtype=np.uint8).reshape(-1)
-            size, ptr = keep.size, keep.ctypes.data
+        keep, size, ptr = _host_bytes(image, "from_host_bed")
         if size != _bed_bytes(n, L):
             raise ValueError(f"a .bed image of {L} SNPs x {n} individuals has {_bed_bytes(n, L)} bytes, not {size}")
         h, miss = C.c_void_p(), C.c_int64()
@@ -243,6 +247,41 @@ class GenotypeStore:
         del keep
         s = cls(h.value)
         s.n_missing = miss.value
+        return s
+
+    # -------------------------------------------------------------- streamed stores: data sets larger than device memory
+    @classmethod
+    def stream_file(cls, path, rows, cols, kblocked=True):
+        """A store that leaves the genotypes of a no-space ASCII file on the host: M.ascii (kblocked, rows = n, cols = L) or
+        Mt.ascii (rows = L, cols = n).  mmt / extract_col (M) and a_and_vara (Mt) decode the file piece by piece on every
+        call, with the resident store's results; transpose and the packed export are refused (include/eagle_gpu.h)."""
+        lib = _lib.require_gpu()
+        h = C.c_void_p()
+        _lib.check(lib.eg_store_stream_file(os.fsencode(path), int(rows), int(cols), int(bool(kblocked)), C.byref(h)))
+        return cls(h.value)
+
+    @classmethod
+    def stream_bed(cls, path, n, L, snp0=0, snp1=None, kblocked=True):
+        """As stream_file, from SNPs [snp0, snp1) of a SNP-major .bed file, in either orientation."""
+        lib = _lib.require_gpu()
+        h = C.c_void_p()
+        _lib.check(lib.eg_store_stream_bed(os.fsencode(path), int(n), int(L), int(snp0), int(L if snp1 is None else snp1),
+                                           int(bool(kblocked)), C.byref(h)))
+        return cls(h.value)
+
+    @classmethod
+    def stream_host_bed(cls, image, n, L, snp0=0, snp1=None, kblocked=True):
+        """As stream_bed, from the whole .bed image in host memory (numpy uint8 array, bytes, or a CPU torch tensor; pinned
+        ones are copied without staging).  The store keeps a reference to the image: the library reads it on every call."""
+        lib = _lib.require_gpu()
+        keep, size, ptr = _host_bytes(image, "stream_host_bed")
+        if size != _bed_bytes(n, L):
+            raise ValueError(f"a .bed image of {L} SNPs x {n} individuals has {_bed_bytes(n, L)} bytes, not {size}")
+        h = C.c_void_p()
+        _lib.check(lib.eg_store_stream_host_bed(C.c_void_p(ptr), int(n), int(L), int(snp0), int(L if snp1 is None else snp1),
+                                                int(bool(kblocked)), C.byref(h)))
+        s = cls(h.value)
+        s._source = keep
         return s
 
     def info(self):

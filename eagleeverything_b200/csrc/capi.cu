@@ -8,6 +8,7 @@
 #include <sys/stat.h>
 #include <unistd.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdlib>
@@ -40,6 +41,13 @@ struct eg_store {
     eg_store* part[16] = {};
     int64_t off[17] = {};
     bool mt_orientation = false;   // composite stores: which axis is sharded (row-major parts: rows)
+    // Streamed stores (eg_store_stream_*): d == nullptr; the genotypes stay at their source and every call that reads them
+    // decodes them piece by piece (stream_pieces).  rows / cols / pitch are those of the resident store.
+    int src_kind = 0;                 // 0: resident; SRC_BED / SRC_ASCII_COLS (M.ascii) / SRC_ASCII_ROWS (Mt.ascii)
+    const uint8_t* src_p = nullptr;   // the caller's .bed image (whole file), which outlives the store
+    int src_fd = -1;                  // or the source file, open for the store's life
+    int64_t src_first = 0;            // .bed: SNP of the file that is marker 0 of the store
+    int64_t src_line = 0;             // ASCII: characters per line of the file
 };
 
 namespace eg {
@@ -98,7 +106,11 @@ struct Context {
     size_t free_bytes = 0, recycle_limit = 0;
     cudaEvent_t scan_ev[2] = {nullptr, nullptr};   // around the dominant scan kernel of the last eg_dev_scan on this GPU
     double scan_ops = 0.0;
+    // a streamed scan: one event pair around the scan kernel of every piece (eg_last_scan_kernel reports their sum)
+    bool scan_summing = false;
+    std::vector<cudaEvent_t> scan_sum_ev;
     void reset() {
+        scan_summing = false; scan_sum_ev.clear();
         ready = false; device = -1; sms = 0; stream = copy_stream = nullptr; cublas = nullptr; cache.clear(); clock = 0;
         d_err = nullptr; for (double& t : timing) t = 0; free_blocks.clear(); live_blocks.clear(); free_bytes = 0; recycle_limit = 0; scan_ev[0] = scan_ev[1] = nullptr; scan_ops = 0.0;
     }
@@ -144,7 +156,7 @@ int scan_mode() {
     return g_scan_mode;
 }
 int launch_scan(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const double* d_Wp,
-                const int64_t* d_zero_rows, int n_zero, double* d_a, double* d_vara, cudaStream_t st);
+                const int64_t* d_zero_rows, int n_zero, double* d_a, double* d_vara, cudaStream_t st, bool sliced);
 
 // Stream-ordered allocations from the device's default memory pool (release threshold raised in eg_init), with an
 // exact-size recycling list on top: every forward step asks for the same handful of multi-GB sizes (two 10 GB stores,
@@ -313,7 +325,10 @@ static bool cache_evict_one() {
     cudaStreamSynchronize(g_ctx.stream);
     return true;
 }
+// set by store_alloc when the genotypes of a store do not fit even after eviction (the drop-in exports then stream)
+static thread_local bool t_store_alloc_failed = false;
 static int store_alloc(int64_t rows, int64_t cols, bool kblocked, eg_store** out) {
+    t_store_alloc_failed = false;
     eg_store* s = new eg_store();
     s->rows = rows;
     s->cols = cols;
@@ -331,6 +346,7 @@ static int store_alloc(int64_t rows, int64_t cols, bool kblocked, eg_store** out
         }
         if (e != cudaSuccess) {
             delete s;
+            t_store_alloc_failed = true;
             return set_error(EG_ERR_ALLOC, "out of device memory for a %lld x %lld genotype store", (long long)rows,
                              (long long)cols);
         }
@@ -906,6 +922,7 @@ static void shutdown_slot() {
     eg_cache_clear();
     release_workspaces();
     if (g_ctx.scan_ev[0]) { cudaEventDestroy(g_ctx.scan_ev[0]); cudaEventDestroy(g_ctx.scan_ev[1]); }
+    for (cudaEvent_t e : g_ctx.scan_sum_ev) cudaEventDestroy(e);
     if (g_ctx.cublas) cublasDestroy(g_ctx.cublas);
     if (g_ctx.stream) cudaStreamDestroy(g_ctx.stream);
     if (g_ctx.copy_stream) cudaStreamDestroy(g_ctx.copy_stream);
@@ -943,6 +960,7 @@ static void free_store_tree(eg_store* s) {
     }
     pool_free(s->C32);
     pool_free(s->d);
+    if (s->src_fd >= 0) close(s->src_fd);
     delete s;
 }
 static eg_store* new_composite(int64_t rows, int64_t cols, bool kblocked) {
@@ -999,6 +1017,236 @@ static int store_from_image_any(const uint8_t* image, int64_t cols_total, int64_
     return EG_OK;
 }
 
+// ------------------------------------------------------------------ one piece loop: .bed uploads and streamed stores
+static int64_t ingest_piece_bytes();
+// Where the genotypes of the markers [0, nm) of a piece loop come from.
+enum { SRC_BED = 1, SRC_ASCII_COLS = 2, SRC_ASCII_ROWS = 3 };
+struct PieceSource {
+    HostSrc hs;
+    int kind = SRC_BED;   // SRC_BED: SNP rows of a .bed image; SRC_ASCII_COLS: columns of M.ascii; SRC_ASCII_ROWS: lines of Mt.ascii
+    int64_t n = 0;        // individuals
+    int64_t first = 0;    // marker 0 of the loop in the source: a SNP of the .bed, a column or a line of the text
+    int64_t line = 0;     // ASCII: characters per line
+    int64_t lines = 0;    // ASCII: lines of the file (the last one may lack its '\n')
+};
+// Markers per piece: at most ingest_piece_bytes() source bytes, in whole 128-marker blocks.
+static int64_t piece_markers(const PieceSource& P, int64_t nm) {
+    const int64_t per = P.kind == SRC_BED ? (P.n + 3) / 4 : P.kind == SRC_ASCII_COLS ? P.n : P.line + 1;
+    int64_t piece = ingest_piece_bytes() / per / 128 * 128;
+    if (piece < 128) piece = 128;
+    if (piece > round_up(nm, 128)) piece = round_up(nm, 128);
+    return piece;
+}
+// Markers [0, nm) of P, piece by piece.  Piece k is staged into one of two device buffers on copy_stream (through the
+// page-locked ring unless the source is page-locked memory) while piece k-1 is decoded and consumed on g_ctx.stream.
+// dst != nullptr: every piece is decoded into that store (marker m of the loop is marker m of a store of nm markers);
+// dst == nullptr: into a buffer of one piece, which consume(m, ns, piece) reads (in the store's layout, ns markers) before
+// the next piece is decoded.  ASCII format errors come back with the resident upload's text.  The position is that of the
+// decoder unit that saw the byte, offset by the piece: the resident one for row pieces of Mt.ascii; for column pieces of
+// M.ascii a unit of the piece, which may start at another row or column than the resident upload's unit (both hold the
+// byte).
+static int piece_loop(const PieceSource& P, int64_t nm, bool kblocked, int8_t* dst, uint64_t* d_missing,
+                      const std::function<int(int64_t, int64_t, const int8_t*)>& consume) {
+    const int64_t n = P.n, piece = piece_markers(P, nm), npieces = (nm + piece - 1) / piece;
+    const int64_t bpr = (n + 3) / 4, pitch = kblocked ? 0 : store_pitch(n);
+    const bool ascii = P.kind != SRC_BED;
+    const size_t stg_bytes = P.kind == SRC_BED          ? (size_t)piece * bpr
+                             : P.kind == SRC_ASCII_COLS ? (size_t)n * piece + 64
+                                                        : (size_t)piece * (P.line + 1) + 64;
+    DevBuf stg[2], dec, errs;
+    int rc = EG_OK;
+    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc(stg_bytes, "genotype staging");
+    if (rc == EG_OK && !dst)
+        rc = dec.alloc(kblocked ? (size_t)round_up(piece, 128) * n : (size_t)piece * pitch, "decoded genotype piece");
+    if (rc == EG_OK && ascii) rc = errs.alloc((size_t)npieces * 4 * sizeof(int32_t), "decode status");
+    if (rc != EG_OK) return rc;
+    if (ascii) EG_CUDA(cudaMemsetAsync(errs.p, 0, (size_t)npieces * 4 * sizeof(int32_t), g_ctx.stream));
+    cudaEvent_t copied[2], decoded[2];
+    for (int i = 0; i < 2; i++) {
+        cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
+        cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
+    }
+    cudaEventRecord(decoded[0], g_ctx.stream);
+    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);  // the staging buffers were allocated in g_ctx.stream order
+    for (int64_t k = 0; k < npieces && rc == EG_OK; k++) {
+        const int b = (int)(k & 1);
+        const int64_t m = k * piece, ns = m + piece <= nm ? piece : nm - m, at = P.first + m;
+        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);
+        if (P.kind == SRC_BED) {
+            const size_t bytes = (size_t)ns * (size_t)bpr;
+            rc = h2d_staged_2d(stg[b].p, bytes, P.hs, 3 + (size_t)at * (size_t)bpr, bytes, bytes, 1, g_ctx.copy_stream);
+        } else if (P.kind == SRC_ASCII_COLS) {   // columns [at, at + ns) of every line: a 2-D copy
+            rc = h2d_staged_2d(stg[b].p, (size_t)piece, P.hs, (size_t)at, (size_t)(P.line + 1), (size_t)ns, (size_t)n, g_ctx.copy_stream);
+        } else {                                 // whole lines; never read past the file's last byte
+            size_t bytes = (size_t)ns * (size_t)(P.line + 1);
+            if (at + ns == P.lines) bytes -= 1;
+            rc = h2d_staged_2d(stg[b].p, bytes, P.hs, (size_t)at * (size_t)(P.line + 1), bytes, bytes, 1, g_ctx.copy_stream);
+        }
+        if (rc != EG_OK) break;
+        cudaEventRecord(copied[b], g_ctx.copy_stream);
+        cudaStreamWaitEvent(g_ctx.stream, copied[b], 0);
+        int8_t* out = dst ? dst : dec.as<int8_t>();
+        const int64_t dm = dst ? m : 0;   // first marker of the piece in `out`
+        if (P.kind == SRC_BED)
+            rc = eg_dev_decode_bed(stg[b].as<uint8_t>(), n, ns, out, dst ? nm : ns, pitch, dm, d_missing, g_ctx.stream);
+        else if (P.kind == SRC_ASCII_COLS)
+            rc = eg_dev_decode_kb(stg[b].as<uint8_t>(), piece, (int64_t)stg_bytes, n, ns, out + (dm / 128) * n * 128, n, 0,
+                                  errs.as<int32_t>() + 4 * k, g_ctx.stream);
+        else
+            rc = eg_dev_decode(stg[b].as<uint8_t>(), P.line + 1, (int64_t)stg_bytes, ns, n, out + dm * pitch, pitch,
+                               errs.as<int32_t>() + 4 * k, g_ctx.stream);
+        cudaEventRecord(decoded[b], g_ctx.stream);
+        if (rc == EG_OK && consume) rc = consume(m, ns, out);
+    }
+    std::vector<int32_t> h_err(ascii ? (size_t)npieces * 4 : 0, 0);
+    if (rc == EG_OK && ascii)
+        rc = check_cuda(cudaMemcpyAsync(h_err.data(), errs.p, h_err.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, g_ctx.stream),
+                        "decode status D2H");
+    if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "genotype decode");
+    cudaStreamSynchronize(g_ctx.copy_stream);
+    for (int i = 0; i < 2; i++) {
+        cudaEventDestroy(copied[i]);
+        cudaEventDestroy(decoded[i]);
+    }
+    for (int64_t k = 0; k < npieces && rc == EG_OK && ascii; k++)
+        rc = P.kind == SRC_ASCII_COLS ? decode_status(&h_err[4 * k], 0, P.first + k * piece)
+                                      : decode_status(&h_err[4 * k], P.first + k * piece, 0);
+    return rc;
+}
+
+// The source of a streamed store, and how many pieces a call over all of its markers runs.
+static PieceSource source_of(const eg_store* s) {
+    PieceSource P;
+    P.hs.p = s->src_p;
+    P.hs.fd = s->src_fd;
+    P.kind = s->src_kind;
+    P.n = s->pitch ? s->cols : s->rows;
+    P.first = s->src_first;
+    P.line = s->src_line;
+    P.lines = s->rows;   // M.ascii: n lines; Mt.ascii: L lines
+    return P;
+}
+static int64_t stream_pieces(const eg_store* s) {
+    const int64_t nm = s->pitch ? s->rows : s->cols;
+    const int64_t piece = piece_markers(source_of(s), nm);
+    return (nm + piece - 1) / piece;
+}
+// M.Mt of a streamed M store into C (zeroed here): every decoded piece is contracted into the one int32 accumulator, its
+// zeroed columns corrected with piece-local indices.
+static int mmt_streamed(const eg_store* M, const std::vector<int64_t>& zero_cols, int32_t* d_C) {
+    const int64_t n = M->rows;
+    cudaStream_t st = g_ctx.stream;
+    EG_CUDA(cudaMemsetAsync(d_C, 0, (size_t)n * n * sizeof(int32_t), st));
+    return piece_loop(source_of(M), M->cols, true, nullptr, nullptr, [&](int64_t m, int64_t ns, const int8_t* piece) -> int {
+        EG_TRY(eg_dev_syrk_i8_kb(piece, n, ns, d_C, n, st));
+        std::vector<int64_t> z;
+        for (int64_t c : zero_cols)
+            if (c >= m && c < m + ns) z.push_back(c - m);
+        return z.empty() ? EG_OK : eg_dev_syrk_zero_cols(piece, n, 0, z.data(), (int64_t)z.size(), d_C, n, st);
+    });
+}
+// The scan of a streamed Mt store, with W already folded into d_Wp: every piece runs the contraction on the slices of U that
+// the first piece made, and writes its a / var(a) at its offset of d_a / d_vara (L entries each).  eg_last_scan_kernel then
+// reports the sum over the pieces.
+static int scan_streamed(const eg_store* Mt, const std::vector<int64_t>& zero_rows, const double* d_Wp, double* d_a,
+                         double* d_vara) {
+    const int64_t n = Mt->cols;
+    cudaStream_t st = g_ctx.stream;
+    const PieceSource P = source_of(Mt);
+    const int64_t piece = piece_markers(P, Mt->rows);
+    std::vector<int64_t> z(zero_rows), zl(zero_rows.size());
+    std::sort(z.begin(), z.end());
+    for (size_t i = 0; i < z.size(); i++) zl[i] = z[i] % piece;   // piece-local, grouped by piece
+    DevBuf dz;
+    if (!z.empty()) {
+        EG_TRY(dz.alloc(zl.size() * sizeof(int64_t), "zeroed rows"));
+        EG_CUDA(cudaMemcpyAsync(dz.p, zl.data(), zl.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    }
+    for (cudaEvent_t e : g_ctx.scan_sum_ev) cudaEventDestroy(e);
+    g_ctx.scan_sum_ev.clear();
+    g_ctx.scan_ops = 0.0;
+    g_ctx.scan_summing = true;
+    size_t zi = 0;
+    const int rc = piece_loop(P, Mt->rows, false, nullptr, nullptr, [&](int64_t m, int64_t ns, const int8_t* p) -> int {
+        const size_t z0 = zi;
+        while (zi < z.size() && z[zi] < m + ns) zi++;
+        return launch_scan(p, ns, n, Mt->pitch, d_Wp, zi > z0 ? dz.as<int64_t>() + z0 : nullptr, (int)(zi - z0), d_a + m,
+                           d_vara + m, st, m > 0);
+    });
+    g_ctx.scan_summing = false;
+    return rc;
+}
+// Column `col` of a streamed M store: one SNP row of the .bed, or the n bytes of one column of M.ascii (a 2-D staged copy of
+// width 1), through the same decoders as the resident upload.
+static int extract_streamed(const eg_store* M, int64_t col, int32_t* out) {
+    const int64_t n = M->rows;
+    cudaStream_t st = g_ctx.stream;
+    PieceSource P = source_of(M);
+    P.first += col;
+    DevBuf d;
+    EG_TRY(d.alloc((size_t)n * 4, "column"));
+    EG_TRY(piece_loop(P, 1, true, nullptr, nullptr,
+                      [&](int64_t, int64_t, const int8_t* p) { return eg_dev_extract_col(p, n, 0, 0, d.as<int32_t>(), st); }));
+    EG_CUDA(cudaMemcpyAsync(out, d.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+    return check_cuda(cudaStreamSynchronize(st), "extract D2H");
+}
+// A streamed store: the shape of the resident one, the source instead of the bytes.  Single GPU only.
+static int stream_store_new(int kind, int64_t rows, int64_t cols, bool kblocked, const uint8_t* p, int fd, int64_t first,
+                            int64_t line, const char* who, eg_store** out) {
+    if (g_multi.n > 1) {
+        if (fd >= 0) close(fd);
+        return set_error(EG_ERR_ARG, "%s: streamed stores work on one GPU (eg_init_multi has set up %d)", who, g_multi.n);
+    }
+    const int rc = ensure_init();
+    if (rc != EG_OK) {
+        if (fd >= 0) close(fd);
+        return rc;
+    }
+    eg_store* s = new eg_store();
+    s->rows = rows;
+    s->cols = cols;
+    s->pitch = kblocked ? 0 : store_pitch(cols);
+    s->src_kind = kind;
+    s->src_p = p;
+    s->src_fd = fd;
+    s->src_first = first;
+    s->src_line = line;
+    *out = s;
+    return EG_OK;
+}
+// M.ascii (kblocked: rows = n, cols = L) or Mt.ascii (rows = L, cols = n), checked as eg_store_from_file checks it
+static int stream_file_store(const char* path, int64_t rows, int64_t cols, bool kblocked, eg_store** out) {
+    if (rows <= 0 || cols <= 0) return set_error(EG_ERR_ARG, "dims must be positive");
+    MappedFile f;
+    EG_TRY(f.open_ro(path));
+    EG_TRY(check_image_size(f, path, rows, cols));
+    const int fd = dup(f.fd);
+    if (fd < 0) return set_error(EG_ERR_OPEN, "ERROR: Could not open  %s", path);
+    return stream_store_new(kblocked ? SRC_ASCII_COLS : SRC_ASCII_ROWS, rows, cols, kblocked, nullptr, fd, 0, cols,
+                            "eg_store_stream_file", out);
+}
+// A streamed store the caller owns for one call
+struct OwnedStore {
+    eg_store* s = nullptr;
+    ~OwnedStore() { if (s) free_store_tree(s); }
+};
+// The store of a drop-in export's input file: resident, from the path cache -- or, when its genotypes do not fit on the
+// device even after eviction (store_alloc's EG_ERR_ALLOC) and one GPU is in use, streamed from the file for this call only
+// (owned by `streamed`; nothing goes into the path cache).  Any other failure, also any other allocation, is passed on.
+static int export_store(const char* path, int64_t rows, int64_t cols, bool kblocked, bool allow_multi, OwnedStore& streamed,
+                        eg_store** out) {
+    t_store_alloc_failed = false;
+    const int rc = cached_store(path, rows, cols, kblocked, out, allow_multi);
+    if (rc != EG_ERR_ALLOC || !t_store_alloc_failed || g_multi.n > 1) return rc;
+    EG_TRY(stream_file_store(path, rows, cols, kblocked, &streamed.s));
+    *out = streamed.s;
+    return EG_OK;
+}
+static int refuse_streamed(const eg_store* s, const char* who) {
+    if (!s->src_kind) return EG_OK;
+    return set_error(EG_ERR_ARG, "%s: the store is streamed from its source and holds no genotypes on the device", who);
+}
+
 // ------------------------------------------------------------------ compute helpers on stores
 // A plain store is worked on as slot 0 of 1 on the calling thread, a composite one by every GPU slot on its own thread.
 static const eg_store* slot_part(const eg_store* S, int r) { return S->nparts > 1 ? S->part[r] : S; }
@@ -1020,6 +1268,12 @@ static int partial_product(const eg_store* M, const std::vector<int64_t>& zero_c
     const int64_t n = M->rows;
     cudaStream_t st = g_ctx.stream;
     EG_TRY(C.alloc((size_t)n * n * sizeof(int32_t), "MMt int32 accumulator"));
+    if (M->src_kind) {   // streamed: the zeroed columns are corrected piece by piece
+        Timer t(st);
+        EG_TRY(mmt_streamed(M, zero_cols, C.as<int32_t>()));
+        g_ctx.timing[1] = t.stop();
+        return EG_OK;
+    }
     const char* envk = getenv("EAGLE_KEEP_PRODUCT");   // "0": contract again on every call (bench.py's steady-state leg)
     const bool reuse = !(envk && envk[0] == '0');
     if (M->C32 && reuse) {  // accumulated under the upload (store_from_image_kb): keep it intact for later calls
@@ -1179,8 +1433,11 @@ static int scan_slot(const eg_store* Mt, int r, const std::vector<int64_t>& zero
         const std::vector<int64_t> z = slot_indices(Mt, r, zero_rows);
         {
             Timer t(st);
-            EG_TRY(eg_dev_scan(part->d, L, n, part->pitch, dW.as<double>(), z.empty() ? nullptr : z.data(), (int64_t)z.size(),
-                               oa.as<double>(), ov.as<double>(), st));
+            if (part->src_kind)
+                EG_TRY(scan_streamed(part, z, dW.as<double>(), oa.as<double>(), ov.as<double>()));
+            else
+                EG_TRY(eg_dev_scan(part->d, L, n, part->pitch, dW.as<double>(), z.empty() ? nullptr : z.data(), (int64_t)z.size(),
+                                   oa.as<double>(), ov.as<double>(), st));
             g_ctx.timing[6] = t.stop();
         }
         Timer t(st);   // off[0] is 0 for every store, so a plain store's results start at out_a[0]
@@ -1335,6 +1592,21 @@ extern "C" int eg_get_scan_digits(void) { return scan_i8_digits(); }
 namespace eg {
 // CUDA events around the dominant scan kernel of the last eg_dev_scan call (for roofline reporting)
 void scan_kernel_mark(int which, cudaStream_t st, double ops) {
+    if (g_ctx.scan_summing) {   // a piece of a streamed scan: one more event, the operations add up
+        cudaEvent_t e;
+        if (cudaEventCreate(&e) != cudaSuccess) {
+            cudaGetLastError();
+            return;
+        }
+        cudaEventRecord(e, st);
+        g_ctx.scan_sum_ev.push_back(e);
+        g_ctx.scan_ops += ops;
+        return;
+    }
+    if (which == 0) {
+        for (cudaEvent_t e : g_ctx.scan_sum_ev) cudaEventDestroy(e);
+        g_ctx.scan_sum_ev.clear();
+    }
     if (!g_ctx.scan_ev[0]) {
         cudaEventCreate(&g_ctx.scan_ev[0]);
         cudaEventCreate(&g_ctx.scan_ev[1]);
@@ -1344,7 +1616,20 @@ void scan_kernel_mark(int which, cudaStream_t st, double ops) {
 }
 }  // namespace eg
 extern "C" int eg_last_scan_kernel(double* ms, double* ops) {
-    if (!g_ctx.scan_ev[0] || !ms || !ops) return set_error(EG_ERR_ARG, "eg_last_scan_kernel: no scan has run");
+    if (!ms || !ops) return set_error(EG_ERR_ARG, "eg_last_scan_kernel: null");
+    if (g_ctx.scan_sum_ev.size() >= 2) {   // a streamed scan: the sum over its pieces
+        double sum = 0.0;
+        for (size_t i = 0; i + 1 < g_ctx.scan_sum_ev.size(); i += 2) {
+            EG_CUDA(cudaEventSynchronize(g_ctx.scan_sum_ev[i + 1]));
+            float f = 0;
+            EG_CUDA(cudaEventElapsedTime(&f, g_ctx.scan_sum_ev[i], g_ctx.scan_sum_ev[i + 1]));
+            sum += f;
+        }
+        *ms = sum;
+        *ops = g_ctx.scan_ops;
+        return EG_OK;
+    }
+    if (!g_ctx.scan_ev[0]) return set_error(EG_ERR_ARG, "eg_last_scan_kernel: no scan has run");
     EG_CUDA(cudaEventSynchronize(g_ctx.scan_ev[1]));
     float f = 0;
     EG_CUDA(cudaEventElapsedTime(&f, g_ctx.scan_ev[0], g_ctx.scan_ev[1]));
@@ -1409,6 +1694,7 @@ extern "C" int eg_store_from_host_packed(const uint64_t* words, int64_t rows, in
 extern "C" int eg_store_to_host_packed(const eg_store_t* s, uint64_t* out_words) {
     if (!s || !out_words) return set_error(EG_ERR_ARG, "eg_store_to_host_packed: bad argument");
     if (s->nparts > 1) return set_error(EG_ERR_ARG, "eg_store_to_host_packed: the store is sharded over several GPUs");
+    EG_TRY(refuse_streamed(s, "eg_store_to_host_packed"));
     EG_TRY(ensure_init());
     const int64_t wpr = eg_packed_words_per_row(s->cols);
     DevBuf w;
@@ -1425,6 +1711,7 @@ extern "C" int eg_store_drop_individuals(const eg_store_t* in, const int64_t* id
                                          eg_store_t** out) {
     if (!in || !out || k < 0 || (k > 0 && !idx)) return set_error(EG_ERR_ARG, "eg_store_drop_individuals: bad argument");
     if (in->nparts > 1) return set_error(EG_ERR_ARG, "eg_store_drop_individuals: the store is sharded over several GPUs");
+    EG_TRY(refuse_streamed(in, "eg_store_drop_individuals"));
     Pin pin_in(in);
     EG_TRY(ensure_init());
     const int64_t n_in = individuals_are_rows ? in->rows : in->cols;
@@ -1467,6 +1754,7 @@ extern "C" int eg_store_from_file(const char* path, int64_t rows, int64_t cols, 
 }
 extern "C" int eg_store_transpose(const eg_store_t* in, eg_store_t** out) {
     if (!in || !out) return set_error(EG_ERR_ARG, "null argument");
+    EG_TRY(refuse_streamed(in, "eg_store_transpose"));
     EG_TRY(ensure_init());
     Pin pin(in);
     if (in->nparts > 1) {   // marker shards transpose in place: part r (n x L_r) -> (L_r x n), no exchange
@@ -1507,11 +1795,13 @@ extern "C" int eg_store_info(const eg_store_t* s, int64_t* rows, int64_t* cols, 
     if (rows) *rows = s->rows;
     if (cols) *cols = s->cols;
     if (pitch) *pitch = s->pitch;
-    if (device_ptr) *device_ptr = s->d;   // NULL for a store sharded over several GPUs
+    if (device_ptr) *device_ptr = s->d;   // NULL for a store sharded over several GPUs or streamed from its source
     return EG_OK;
 }
 extern "C" int eg_store_mmt(const eg_store_t* M, const int64_t* zero_cols, int64_t n_zero, double* out_MMt_host) {
     if (!M || !out_MMt_host || n_zero < 0) return set_error(EG_ERR_ARG, "eg_store_mmt: bad argument");
+    if (M->src_kind && M->pitch)
+        return set_error(EG_ERR_ARG, "eg_store_mmt: a streamed store gives M.Mt in the M orientation (kblocked) only");
     EG_TRY(ensure_init());
     std::vector<int64_t> z;
     for (int64_t i = 0; i < n_zero; i++) {
@@ -1537,6 +1827,10 @@ extern "C" int eg_store_extract_col(const eg_store_t* M, int64_t col, int32_t* o
     if (!M || !out || col < 0 || col >= M->cols) return set_error(EG_ERR_ARG, "eg_store_extract_col: bad argument");
     EG_TRY(ensure_init());
     Pin pin(M);
+    if (M->src_kind) {
+        if (M->pitch) return set_error(EG_ERR_ARG, "eg_store_extract_col: a streamed store gives columns in the M orientation (kblocked) only");
+        return extract_streamed(M, col, out);
+    }
     if (M->nparts > 1) {   // the GPU that owns the marker answers
         if (M->mt_orientation) return set_error(EG_ERR_ARG, "eg_store_extract_col: needs an M store");
         return run_all([&](int r) -> int {
@@ -1704,11 +1998,15 @@ extern "C" int eg_calculateMMt_rcpp(const char* f_name_ascii, double max_memory_
     (void)num_cores;
     if (!dims || !out_MMt) return set_error(EG_ERR_ARG, "calculateMMt_rcpp: null argument");
     eg_store* M = nullptr;
-    EG_TRY(cached_store(f_name_ascii, dims[0], dims[1], true, &M));
+    OwnedStore streamed;
+    EG_TRY(export_store(f_name_ascii, dims[0], dims[1], true, true, streamed, &M));
     std::vector<int64_t> z;
     EG_TRY(parse_selected(selected_loci, n_selected_loci, dims[1], z, "calculateMMt_rcpp"));
     if (!quiet) say(message, message_ctx, " M %%*%% t(M) on GPU %d (int8 tensor cores, exact) ", g_ctx.device);
-    return mmt_of_store(M, z, out_MMt, true);
+    if (!quiet && streamed.s)
+        say(message, message_ctx, " M does not fit in device memory: streamed from %s in %lld pieces ", f_name_ascii,
+            (long long)stream_pieces(M));
+    return mmt_of_store(M, z, out_MMt, !streamed.s);
 }
 
 extern "C" int eg_calculate_a_and_vara_rcpp(const char* f_name_ascii, const double* selected_loci,
@@ -1720,10 +2018,14 @@ extern "C" int eg_calculate_a_and_vara_rcpp(const char* f_name_ascii, const doub
     if (!dims || !inv_MMt_sqrt || !dim_reduced_vara || !a || !out_a || !out_vara)
         return set_error(EG_ERR_ARG, "calculate_a_and_vara_rcpp: null argument");
     eg_store* Mt = nullptr;
-    EG_TRY(cached_store(f_name_ascii, dims[0], dims[1], false, &Mt));  // dims of Mt: (L, n)
+    OwnedStore streamed;
+    EG_TRY(export_store(f_name_ascii, dims[0], dims[1], false, true, streamed, &Mt));  // dims of Mt: (L, n)
     std::vector<int64_t> z;
     EG_TRY(parse_selected(selected_loci, n_selected_loci, dims[0], z, "calculate_a_and_vara_rcpp"));
-    if (!quiet)
+    if (!quiet && streamed.s)
+        say(message, message_ctx, "Inside internal function calculate_a_and_vara_rcpp: GPU %d, Mt does not fit in device memory: "
+            "streamed from %s in %lld pieces ", g_ctx.device, f_name_ascii, (long long)stream_pieces(Mt));
+    else if (!quiet)
         say(message, message_ctx, "Inside internal function calculate_a_and_vara_rcpp: GPU %d, no blocking needed ",
             g_ctx.device);
     return scan_of_store(Mt, z, inv_MMt_sqrt, dim_reduced_vara, a, out_a, out_vara);
@@ -1770,7 +2072,8 @@ extern "C" int eg_extract_geno_rcpp(const char* f_name_ascii, double max_memory_
         return set_error(EG_ERR_ARG, "extract_geno_rcpp: locus %lld outside [0, %lld)", (long long)selected_locus,
                          (long long)dims[1]);
     eg_store* M = nullptr;
-    EG_TRY(cached_store(f_name_ascii, dims[0], dims[1], true, &M));  // shares the store with calculateMMt_rcpp
+    OwnedStore streamed;
+    EG_TRY(export_store(f_name_ascii, dims[0], dims[1], true, true, streamed, &M));  // shares the store with calculateMMt_rcpp
     return eg_store_extract_col(M, selected_locus, out);
 }
 
@@ -2175,6 +2478,52 @@ static int write_store_ascii(const eg_store* T, const char* path) {
     }
     return rc;
 }
+// createMt_ASCII_rcpp on a streamed M store: every column piece of M.ascii is decoded, transposed and encoded on the device,
+// and its lines of Mt.ascii are written in order -- the bytes write_store_ascii writes for the resident transpose.  Two
+// page-locked buffers: piece k is written to the file while piece k + 1 is on the device.
+static int write_mt_ascii_streamed(const eg_store* M, const char* path) {
+    const int64_t n = M->rows, line = n + 1, tp = store_pitch(n);
+    const int64_t piece = piece_markers(source_of(M), M->cols);
+    cudaStream_t st = g_ctx.stream;
+    OutFile outf;
+    outf.f = fopen(path, "wb");
+    if (!outf.f) return set_error(EG_ERR_OPEN, "ERROR: Could not open  %s for writing", path);
+    DevBuf T, enc[2];
+    PinnedBuf h[2];
+    cudaEvent_t done[2] = {nullptr, nullptr};
+    size_t pending[2] = {0, 0};
+    int rc = T.alloc((size_t)piece * tp, "transposed genotype piece");
+    for (int i = 0; i < 2 && rc == EG_OK; i++) {
+        rc = enc[i].alloc((size_t)piece * line + 16, "ASCII rows");
+        if (rc == EG_OK) rc = h[i].ensure((size_t)piece * line + 16, "ASCII rows");
+        if (rc == EG_OK) rc = check_cuda(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming), "cudaEventCreate");
+    }
+    auto flush = [&](int b) -> int {   // the lines of the piece in buffer b, once its copy has landed
+        if (!pending[b]) return EG_OK;
+        EG_CUDA(cudaEventSynchronize(done[b]));
+        const size_t wb = pending[b];
+        pending[b] = 0;
+        return fwrite(h[b].p, 1, wb, outf.f) == wb ? EG_OK : set_error(EG_ERR_OPEN, "short write to %s", path);
+    };
+    int64_t k = 0;
+    if (rc == EG_OK)
+        rc = piece_loop(source_of(M), M->cols, true, nullptr, nullptr, [&](int64_t, int64_t ns, const int8_t* p) -> int {
+            const int b = (int)(k++ & 1);
+            EG_TRY(eg_dev_transpose_kb_i8(p, n, ns, T.as<int8_t>(), tp, st));
+            EG_TRY(eg_dev_encode_ascii(T.as<int8_t>(), tp, n, 0, ns, enc[b].as<uint8_t>(), st));
+            EG_CUDA(cudaMemcpyAsync(h[b].p, enc[b].p, (size_t)ns * line, cudaMemcpyDeviceToHost, st));
+            EG_CUDA(cudaEventRecord(done[b], st));
+            pending[b] = (size_t)ns * line;
+            return flush(b ^ 1);   // the previous piece, while this one is in flight
+        });
+    if (rc == EG_OK) rc = flush((int)((k - 1) & 1));
+    cudaStreamSynchronize(st);
+    for (int i = 0; i < 2; i++)
+        if (done[i]) cudaEventDestroy(done[i]);
+    if (fclose(outf.f) != 0 && rc == EG_OK) rc = set_error(EG_ERR_OPEN, "short write to %s", path);
+    outf.f = nullptr;
+    return rc;
+}
 }  // namespace eg
 
 extern "C" int eg_createM_ASCII_rcpp(const char* f_name, const char* f_name_ascii, const char* type, const char* AA, const char* AB,
@@ -2195,7 +2544,6 @@ extern "C" int eg_createM_ASCII_rcpp(const char* f_name, const char* f_name_asci
 // upload anything.
 extern "C" int eg_createMt_ASCII_rcpp(const char* f_name, const char* f_name_ascii, const char* type, double max_memory_in_Gbytes,
                                       const int64_t* dims, int quiet, eg_message_fn message, void* message_ctx) {
-    (void)quiet;
     if (!f_name || !f_name_ascii || !type || !dims) return set_error(EG_ERR_ARG, "createMt_ASCII_rcpp: null argument");
     const int64_t n = dims[0], L = dims[1];
     EG_TRY(ensure_init());
@@ -2204,16 +2552,23 @@ extern "C" int eg_createMt_ASCII_rcpp(const char* f_name, const char* f_name_asc
         if (stat(f_name, &stt) != 0) return set_error(EG_ERR_OPEN, "\n\nERROR: Could not open  %s\n\n\n", f_name);
     }
     eg_store* M = nullptr;
-    EG_TRY(cached_store(f_name, n, L, true, &M, false));
-    Pin pin_m(M);   // held while the transpose is allocated (eviction under memory pressure must skip it)
-    eg_store* Mt = nullptr;
-    EG_TRY(eg_store_transpose(M, &Mt));
-    int rc = write_store_ascii(Mt, f_name_ascii);
-    if (rc != EG_OK) {
-        eg_store_free(Mt);
-        return rc;
-    }
-    {   // the Mt store now corresponds to the file just written: keep it for calculate_a_and_vara_rcpp
+    OwnedStore streamed;
+    EG_TRY(export_store(f_name, n, L, true, false, streamed, &M));
+    if (streamed.s) {   // M does not fit: its column pieces are transposed and written as they are decoded; nothing is cached
+        if (!quiet)
+            say(message, message_ctx, " M does not fit in device memory: streamed from %s in %lld pieces ", f_name,
+                (long long)stream_pieces(M));
+        EG_TRY(write_mt_ascii_streamed(M, f_name_ascii));
+    } else {
+        Pin pin_m(M);   // held while the transpose is allocated (eviction under memory pressure must skip it)
+        eg_store* Mt = nullptr;
+        EG_TRY(eg_store_transpose(M, &Mt));
+        int rc = write_store_ascii(Mt, f_name_ascii);
+        if (rc != EG_OK) {
+            eg_store_free(Mt);
+            return rc;
+        }
+        // the Mt store now corresponds to the file just written: keep it for calculate_a_and_vara_rcpp
         std::string key;
         if (cache_key(f_name_ascii, L, n, false, key) == EG_OK) cache_insert(key, Mt);
         else eg_store_free(Mt);
@@ -2380,54 +2735,29 @@ static int bed_open(const char* path, int64_t n, int64_t L, MappedFile& f) {
                          "= %zu (wrong n / L, or a truncated file?)", path, f.size, (long long)L, (long long)n, want);
     return EG_OK;
 }
-// SNPs [snp0, snp1) of a .bed image -> one plain store.  Pieces of whole 128-SNP blocks (EAGLE_INGEST_PIECE_BYTES bytes at
-// most) go through two device buffers: the staging of piece k+1 overlaps the decode of piece k.
+// SNPs [snp0, snp1) of a .bed image -> one plain store: the piece loop decodes every piece straight into the store.
 static int store_from_bed(const HostSrc& src, int64_t n, int64_t snp0, int64_t snp1, bool kblocked, uint64_t* n_missing,
                           eg_store** out) {
     EG_TRY(ensure_init());
-    const int64_t bpr = (n + 3) / 4, nsnp = snp1 - snp0;
-    int64_t piece = ingest_piece_bytes() / bpr / 128 * 128;
-    if (piece < 128) piece = 128;
-    if (piece > round_up(nsnp, 128)) piece = round_up(nsnp, 128);
+    const int64_t nsnp = snp1 - snp0;
     eg_store* s = nullptr;
     EG_TRY(kblocked ? store_alloc(n, nsnp, true, &s) : store_alloc(nsnp, n, false, &s));
-    DevBuf stg[2], dmiss;
-    int rc = EG_OK;
-    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc((size_t)piece * bpr, ".bed staging");
-    if (rc == EG_OK) rc = dmiss.alloc(sizeof(uint64_t), "missing genotype count");
+    DevBuf dmiss;
+    int rc = dmiss.alloc(sizeof(uint64_t), "missing genotype count");
     if (rc != EG_OK) return finish_store(rc, s, out);
-    cudaEvent_t copied[2], decoded[2];
-    for (int i = 0; i < 2; i++) {
-        cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
-    }
     cudaMemsetAsync(dmiss.p, 0, sizeof(uint64_t), g_ctx.stream);
-    cudaEventRecord(decoded[0], g_ctx.stream);
-    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);  // the staging buffers were allocated in g_ctx.stream order
+    PieceSource P;
+    P.hs = src;
+    P.kind = SRC_BED;
+    P.n = n;
+    P.first = snp0;
     Timer total(g_ctx.stream);
-    int k = 0;
-    for (int64_t m = 0; m < nsnp && rc == EG_OK; m += piece, k++) {
-        const int b = k & 1;
-        const int64_t ns = m + piece <= nsnp ? piece : nsnp - m;
-        const size_t bytes = (size_t)ns * (size_t)bpr;
-        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);
-        rc = h2d_staged_2d(stg[b].p, bytes, src, 3 + (size_t)(snp0 + m) * (size_t)bpr, bytes, bytes, 1, g_ctx.copy_stream);
-        if (rc != EG_OK) break;
-        cudaEventRecord(copied[b], g_ctx.copy_stream);
-        cudaStreamWaitEvent(g_ctx.stream, copied[b], 0);
-        rc = eg_dev_decode_bed(stg[b].as<uint8_t>(), n, ns, s->d, nsnp, s->pitch, m, dmiss.as<uint64_t>(), g_ctx.stream);
-        cudaEventRecord(decoded[b], g_ctx.stream);
-    }
+    rc = piece_loop(P, nsnp, kblocked, s->d, dmiss.as<uint64_t>(), nullptr);
     uint64_t h_miss = 0;
     if (rc == EG_OK)
         rc = check_cuda(cudaMemcpyAsync(&h_miss, dmiss.p, sizeof(h_miss), cudaMemcpyDeviceToHost, g_ctx.stream), "missing count D2H");
     if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), ".bed decode");
-    cudaStreamSynchronize(g_ctx.copy_stream);
     g_ctx.timing[0] = total.stop();  // H2D + decode (overlapped)
-    for (int i = 0; i < 2; i++) {
-        cudaEventDestroy(copied[i]);
-        cudaEventDestroy(decoded[i]);
-    }
     *n_missing = h_miss;
     return finish_store(rc, s, out);
 }
@@ -2520,4 +2850,31 @@ extern "C" int eg_bed_to_ascii(const char* bed_path, int64_t n, int64_t L, const
     if (cache_key(Mt_ascii, L, n, false, key) == EG_OK) cache_insert(key, Mt);
     else eg_store_free(Mt);
     return EG_OK;
+}
+
+// ================================================================== streamed stores (include/eagle_gpu.h)
+extern "C" int eg_store_stream_file(const char* path, int64_t rows, int64_t cols, int kblocked, eg_store_t** out) {
+    if (!path || !out) return set_error(EG_ERR_ARG, "eg_store_stream_file: null argument");
+    return stream_file_store(path, rows, cols, kblocked != 0, out);
+}
+extern "C" int eg_store_stream_bed(const char* path, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked,
+                                   eg_store_t** out) {
+    if (!path || !out) return set_error(EG_ERR_ARG, "eg_store_stream_bed: null argument");
+    EG_TRY(bed_check_range(n, L, snp0, snp1, "eg_store_stream_bed"));
+    MappedFile f;
+    EG_TRY(bed_open(path, n, L, f));
+    const int fd = dup(f.fd);
+    if (fd < 0) return set_error(EG_ERR_OPEN, "ERROR: Could not open  %s", path);
+    const int64_t w = snp1 - snp0;
+    return stream_store_new(SRC_BED, kblocked ? n : w, kblocked ? w : n, kblocked != 0, nullptr, fd, snp0, 0,
+                            "eg_store_stream_bed", out);
+}
+extern "C" int eg_store_stream_host_bed(const uint8_t* image, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked,
+                                        eg_store_t** out) {
+    if (!image || !out) return set_error(EG_ERR_ARG, "eg_store_stream_host_bed: null argument");
+    EG_TRY(bed_check_range(n, L, snp0, snp1, "eg_store_stream_host_bed"));
+    EG_TRY(bed_check_header(image, "the image"));
+    const int64_t w = snp1 - snp0;
+    return stream_store_new(SRC_BED, kblocked ? n : w, kblocked ? w : n, kblocked != 0, image, -1, snp0, 0,
+                            "eg_store_stream_host_bed", out);
 }

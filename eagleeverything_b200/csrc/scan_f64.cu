@@ -233,7 +233,7 @@ extern "C" int64_t eg_scan_wp_elems(int64_t n) {
 
 namespace eg {
 int launch_scan_i8(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const double* d_Wp, int64_t Kpad,
-                   const int64_t* d_zero_rows, int n_zero, double* d_vara, cudaStream_t st);
+                   const int64_t* d_zero_rows, int n_zero, double* d_vara, cudaStream_t st, bool sliced);
 void scan_kernel_mark(int which, cudaStream_t st, double ops);
 int scan_mode();  // 0 = FP64 DMMA (scan_f64_kernel), 1 = exact int8 slices (scan_i8_kernel)
 
@@ -242,8 +242,9 @@ __global__ void zero_entries_kernel(double* v, const int64_t* idx, int n) {
     if (i < n) v[idx[i]] = 0.0;
 }
 
+// sliced: a later piece of a streamed scan with the same d_Wp (the int8 path keeps the slices of U from the first piece)
 int launch_scan(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const double* d_Wp,
-                const int64_t* d_zero_rows, int n_zero, double* d_a, double* d_vara, cudaStream_t st) {
+                const int64_t* d_zero_rows, int n_zero, double* d_a, double* d_vara, cudaStream_t st, bool sliced) {
     ScanParams p;
     p.Mt = d_Mt; p.L = L; p.n = n; p.pitch = pitch; p.Wp = d_Wp;
     p.Kpad = round_up(n, 32);
@@ -263,7 +264,7 @@ int launch_scan(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const d
         zero_entries_kernel<<<(n_zero + 127) / 128, 128, 0, st>>>(d_a, d_zero_rows, n_zero);
         EG_TRY(check_launch("zero_entries_kernel"));
     }
-    if (scan_mode() == 1) return launch_scan_i8(d_Mt, L, n, pitch, d_Wp, p.Kpad, d_zero_rows, n_zero, d_vara, st);
+    if (scan_mode() == 1) return launch_scan_i8(d_Mt, L, n, pitch, d_Wp, p.Kpad, d_zero_rows, n_zero, d_vara, st, sliced);
     EG_CUDA(cudaFuncSetAttribute(scan_f64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SC_SMEM_BYTES));
     const int64_t cap = (int64_t)num_sms() * SC_CTAS_PER_SM;
     const int64_t grid = p.num_blocks < cap ? p.num_blocks : cap;
@@ -288,7 +289,7 @@ extern "C" int eg_dev_scan(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pit
                             "zero rows H2D");
         if (rc) { cudaFree(d_zero); return rc; }
     }
-    int rc = launch_scan(d_Mt, L, n, pitch, d_Wp, d_zero, (int)n_zero, d_a, d_vara, st);
+    int rc = launch_scan(d_Mt, L, n, pitch, d_Wp, d_zero, (int)n_zero, d_a, d_vara, st, false);
     if (d_zero) {
         cudaStreamSynchronize(st);
         cudaFree(d_zero);

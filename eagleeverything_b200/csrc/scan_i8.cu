@@ -714,6 +714,8 @@ struct ScanI8Workspace {
     double* partial = nullptr;  size_t part_cap = 0;
     int2* units = nullptr;      size_t unit_cap = 0;  int units_MB = -1, units_G = -1, units_shape = -1;
     uint32_t* phase = nullptr;  size_t phase_cap = 0;
+    int64_t sliced_n = -1;      // n and digits of the U whose slices Q / expo / scale hold (launch_scan_i8_t's `sliced`)
+    int sliced_digits = 0;
 };
 static thread_local ScanI8Workspace g_si;
 
@@ -749,15 +751,18 @@ int scan_i8_digits() {
 }
 void scan_i8_set_digits(int d) { g_si_digits = d == 6 ? 6 : 7; }
 
-// vara for all rows of an Mt store from the folded matrix U (columns 0..n-1 of Wp)
+// vara for all rows of an Mt store from the folded matrix U (columns 0..n-1 of Wp).  sliced: U is the matrix the previous
+// call on this thread sliced (the pieces of a streamed scan after the first): the digits, exponents and column scales in
+// the workspace are used as they are, and only the contraction and the reduction run.
 template <int S>
 static int launch_scan_i8_t(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const double* d_Wp, int64_t Kpad,
                             const int64_t* d_zero_rows, int n_zero, double* d_vara, cudaStream_t st, double* d_Bout = nullptr,
-                            int64_t ldb = 0) {
+                            int64_t ldb = 0, bool sliced = false) {
     const int full = d_Bout ? 1 : 0;
     int dev = 0;
     EG_CUDA(cudaGetDevice(&dev));
     if (g_si.device != dev) {
+        if (sliced) return set_error(EG_ERR_ARG, "scan_i8: no sliced U on this device");
         if (g_si.device >= 0) scan_i8_release();
         g_si.device = dev;
     }
@@ -787,12 +792,19 @@ static int launch_scan_i8_t(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pi
         g_si.units_G = G;
         g_si.units_shape = shape_key;
     }
+    if (sliced && (g_si.sliced_n != n || g_si.sliced_digits != S || !g_si.Q))
+        return set_error(EG_ERR_ARG, "scan_i8: no sliced U of this shape in the workspace");
     // 1. slice U
-    si_colscale_kernel<<<(unsigned)(G * SI_GCOLS), 256, 0, st>>>(d_Wp, n, Kpad, g_si.expo, g_si.scale, (int64_t)G * SI_GCOLS, SiT<S>::BITS, full);
-    EG_TRY(check_launch("si_colscale_kernel"));
-    si_slice_kernel<S><<<dim3((unsigned)((Kp / 4 + 255) / 256), (unsigned)(G * SI_GCOLS)), 256, 0, st>>>(d_Wp, n, Kpad, g_si.expo,
-                                                                                                   g_si.Q, Kp, full);
-    EG_TRY(check_launch("si_slice_kernel"));
+    if (!sliced) {
+        si_colscale_kernel<<<(unsigned)(G * SI_GCOLS), 256, 0, st>>>(d_Wp, n, Kpad, g_si.expo, g_si.scale, (int64_t)G * SI_GCOLS,
+                                                                     SiT<S>::BITS, full);
+        EG_TRY(check_launch("si_colscale_kernel"));
+        si_slice_kernel<S><<<dim3((unsigned)((Kp / 4 + 255) / 256), (unsigned)(G * SI_GCOLS)), 256, 0, st>>>(d_Wp, n, Kpad, g_si.expo,
+                                                                                                       g_si.Q, Kp, full);
+        EG_TRY(check_launch("si_slice_kernel"));
+        g_si.sliced_n = full ? -1 : n;   // a projection slices another matrix: the scan's U is gone
+        g_si.sliced_digits = S;
+    }
     // 2. the int8 contraction with fused recombination + row-dot
     CUtensorMap tA, tB;
     EG_TRY(si_make_map(&tA, d_Mt, Kp, L, pitch, SI_BM));
@@ -850,9 +862,9 @@ static int launch_scan_i8_t(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pi
 }
 
 int launch_scan_i8(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pitch, const double* d_Wp, int64_t Kpad,
-                   const int64_t* d_zero_rows, int n_zero, double* d_vara, cudaStream_t st) {
-    return scan_i8_digits() == 7 ? launch_scan_i8_t<7>(d_Mt, L, n, pitch, d_Wp, Kpad, d_zero_rows, n_zero, d_vara, st)
-                                 : launch_scan_i8_t<6>(d_Mt, L, n, pitch, d_Wp, Kpad, d_zero_rows, n_zero, d_vara, st);
+                   const int64_t* d_zero_rows, int n_zero, double* d_vara, cudaStream_t st, bool sliced) {
+    return scan_i8_digits() == 7 ? launch_scan_i8_t<7>(d_Mt, L, n, pitch, d_Wp, Kpad, d_zero_rows, n_zero, d_vara, st, nullptr, 0, sliced)
+                                 : launch_scan_i8_t<6>(d_Mt, L, n, pitch, d_Wp, Kpad, d_zero_rows, n_zero, d_vara, st, nullptr, 0, sliced);
 }
 
 // B = Mt * U for a full n x n FP64 matrix U (column-major, ld): every entry exact up to one rounding (7 digits per

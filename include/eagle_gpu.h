@@ -14,7 +14,13 @@
  *   - `selected_loci` follows the reference: 0-based indices as doubles, element 0 == NA_real_
  *     (any NaN) means "none" (calculateMMt_rcpp.cpp:88, calculate_a_and_vara_rcpp.cpp:79);
  *   - `max_memory_in_Gbytes` and `num_cores` are accepted and ignored: GPU residency of the int8
- *     genotypes (1 byte/genotype instead of 8) replaces the host row-blocking they drive;
+ *     genotypes (1 byte/genotype instead of 8) replaces the host row-blocking they drive.  When the
+ *     genotypes of the input file do not fit in device memory even after the path cache has been
+ *     evicted, calculateMMt_rcpp, calculate_a_and_vara_rcpp, extract_geno_rcpp and createMt_ASCII_rcpp
+ *     stream the file through the device piece by piece instead (eg_store_stream_file; one GPU only;
+ *     nothing is cached; a non-quiet call says so) -- the reference's blocked branches, with the same
+ *     results as the resident run.  A multi-GPU set, ReshapeM_rcpp, calculate_reduced_a_rcpp and
+ *     the packed container still fail with EG_ERR_ALLOC then;
  *   - there is NO CPU fallback: without a usable CUDA device every compute entry point fails
  *     with EG_ERR_CUDA.
  */
@@ -194,6 +200,26 @@ int eg_store_from_host_bed(const uint8_t* image, int64_t n, int64_t L, int64_t s
  * write for the same genotypes; both stores stay in the path cache under those names, so the calculateMMt_rcpp /
  * calculate_a_and_vara_rcpp calls that follow upload nothing.  How an R user brings a .bed file to AM(). */
 int eg_bed_to_ascii(const char* bed_path, int64_t n, int64_t L, const char* M_ascii, const char* Mt_ascii);
+/* Streamed stores: genotype sets larger than device memory.  The handle holds the source and no genotype bytes on the
+ * device; every call that reads it stages the source in pieces of whole 128-marker blocks (EAGLE_INGEST_PIECE_BYTES source
+ * bytes at most, 256 MB by default) through the page-locked ring and decodes each piece while the next is copied, with the
+ * same decoders as the resident uploads.  Results are bit-identical to the resident store's.
+ *   source       eg_store_stream_file: M.ascii (kblocked != 0, rows = n, cols = L) or Mt.ascii (kblocked == 0, rows = L,
+ *                cols = n), checked as eg_store_from_file checks it; _bed / _host_bed: SNPs [snp0, snp1) of a .bed file or
+ *                image, checked as eg_store_from_bed / eg_store_from_host_bed check them, in either orientation.  A file
+ *                stays open for the handle's life; a host image must outlive the handle.
+ *   accepted     eg_store_info (device_ptr == NULL; rows, cols and pitch of the resident store), eg_store_mmt and
+ *                eg_store_extract_col on M (kblocked), eg_store_a_and_vara on Mt (the slices of U are made once per call,
+ *                and eg_last_scan_kernel reports the sum over the pieces).  An ASCII format error in any piece is
+ *                EG_ERR_FORMAT with the resident upload's text.  Its "near row, column" names the decoder unit that
+ *                saw the byte: the same position as the resident upload for Mt.ascii; for M.ascii, whose column pieces
+ *                are decoded in other units than the resident upload's whole rows, a unit that holds the byte too.
+ *   refused      eg_store_transpose, eg_store_drop_individuals, eg_store_to_host_packed: EG_ERR_ARG.
+ *   one GPU      under eg_init_multi with more than one GPU the constructors return EG_ERR_ARG. */
+int eg_store_stream_file(const char* path, int64_t rows, int64_t cols, int kblocked, eg_store_t** out);
+int eg_store_stream_bed(const char* path, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked, eg_store_t** out);
+int eg_store_stream_host_bed(const uint8_t* image, int64_t n, int64_t L, int64_t snp0, int64_t snp1, int kblocked,
+                             eg_store_t** out);
 int eg_store_free(eg_store_t* s);
 int eg_store_info(const eg_store_t* s, int64_t* rows, int64_t* cols, int64_t* pitch, void** device_ptr);
 
