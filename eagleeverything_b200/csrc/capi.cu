@@ -31,8 +31,8 @@ struct eg_store {
     int64_t pitch = 0;  // row-major stores (Mt orientation): bytes per row.  0: K-blocked store (M orientation),
                         // [ceil(cols/128)][rows][128] bytes -- the layout the SYRK streams (syrk_i8.cu)
     size_t bytes() const { return pitch ? (size_t)rows * (size_t)pitch : (size_t)((cols + 127) / 128) * (size_t)rows * 128; }
-    // M stores uploaded from a host image: rows x rows int32, M * M^T over all columns of the store, accumulated chunk
-    // by chunk UNDER the host-to-device copy (store_from_image); eg_store_mmt then only finalizes.  nullptr otherwise.
+    // M stores uploaded from a page-locked host image: rows x rows int32, M * M^T over all columns of the store, accumulated
+    // piece by piece UNDER the host-to-device copy (store_from_image); eg_store_mmt then only finalizes.  nullptr otherwise.
     int32_t* C32 = nullptr;
     int pins = 0;   // > 0 while an entry point works on the store: cache eviction under memory pressure skips it
     // Marker-sharded stores (eg_init_multi with more than one GPU): nparts > 1, part[r] lives on GPU slot r and holds the
@@ -339,7 +339,7 @@ static int store_alloc(int64_t rows, int64_t cols, bool kblocked, eg_store** out
     if (e != cudaSuccess) {
         cudaGetLastError();
         // evict cached stores (least recently used first, never one that a caller still holds) and retry once per
-        // eviction; worker threads of a multi-GPU set leave eviction to the orchestrating thread (store_from_image_any)
+        // eviction; worker threads of a multi-GPU set leave eviction to the orchestrating thread (build_composite)
         while (e != cudaSuccess && !t_is_worker && cache_evict_one()) {
             e = fail ? cudaErrorMemoryAllocation : pool_alloc((void**)&s->d, s->bytes() + 256);
             if (e != cudaSuccess) cudaGetLastError();
@@ -374,149 +374,152 @@ static int decode_status(const int32_t* h_err, int64_t row0, int64_t col0) {
                      (long long)(row0 + brow), (long long)(col0 + h_err[2]));
 }
 
-// K-blocked (M orientation) stores: the image is uploaded in COLUMN chunks (2-D copies, ~256 MB each, two staging
-// buffers); every chunk is decoded into its 128-marker blocks and its contribution to M * M^T is accumulated right
-// away (int32, exact, order-free), so that decode and the whole SYRK hide under the PCIe transfer -- at config 3 the
-// upload takes 181 ms and the SYRK 34.  The product stays with the store (eg_store::C32).
-static int store_from_image_kb(const uint8_t* image, int64_t src_pitch_host, int64_t row0, int64_t rows, int64_t col0,
-                               int64_t w, eg_store* s, eg_store** out) {
-    int64_t cw = ((int64_t)(256LL << 20) / rows) / 128 * 128;
-    if (cw < 128) cw = 128;
-    if (cw > round_up(w, 128)) cw = round_up(w, 128);
-    const int64_t nchunks = (w + cw - 1) / cw;
-    DevBuf stg[2], errs;
-    cudaEvent_t copied[2], decoded[2];
-    int rc = EG_OK;
-    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc((size_t)rows * cw + 64, "ASCII staging");
-    if (rc == EG_OK) rc = errs.alloc((size_t)nchunks * 4 * sizeof(int32_t), "decode status");
-    bool eager = rc == EG_OK && rows >= 2;
-    if (eager && pool_alloc((void**)&s->C32, (size_t)rows * rows * sizeof(int32_t)) != cudaSuccess) {
-        cudaGetLastError();
-        s->C32 = nullptr;   // no room for the product: upload only
-        eager = false;
-    }
-    if (rc != EG_OK) return finish_store(rc, s, out);
-    for (int i = 0; i < 2; i++) {
-        cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
-    }
-    cudaMemsetAsync(errs.p, 0, (size_t)nchunks * 4 * sizeof(int32_t), g_ctx.stream);
-    if (eager) cudaMemsetAsync(s->C32, 0, (size_t)rows * rows * sizeof(int32_t), g_ctx.stream);
-    cudaEventRecord(decoded[0], g_ctx.stream);
-    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);  // staging buffers were allocated in g_ctx.stream order
-    Timer total(g_ctx.stream);
-    for (int64_t k = 0; k < nchunks && rc == EG_OK; k++) {
-        const int b = (int)(k & 1);
-        const int64_t c = k * cw, wk = (c + cw <= w) ? cw : w - c;
-        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);
-        const uint8_t* src = image + row0 * src_pitch_host + col0 + c;
-        rc = check_cuda(cudaMemcpy2DAsync(stg[b].p, cw, src, src_pitch_host, wk, rows, cudaMemcpyHostToDevice, g_ctx.copy_stream),
-                        "H2D copy of the ASCII genotype image");
-        if (rc != EG_OK) break;
-        cudaEventRecord(copied[b], g_ctx.copy_stream);
-        cudaStreamWaitEvent(g_ctx.stream, copied[b], 0);
-        int8_t* blocks = s->d + (c / 128) * rows * 128;     // first 128-marker block of this chunk
-        rc = eg_dev_decode_kb(stg[b].as<uint8_t>(), cw, (int64_t)rows * cw + 64, rows, wk, blocks, rows, 0,
-                              errs.as<int32_t>() + 4 * k, g_ctx.stream);
-        cudaEventRecord(decoded[b], g_ctx.stream);
-        if (rc == EG_OK && eager) rc = eg_dev_syrk_i8_kb(blocks, rows, wk, s->C32, rows, g_ctx.stream);
-    }
-    std::vector<int32_t> h_err((size_t)nchunks * 4, 0);
-    if (rc == EG_OK)
-        rc = check_cuda(cudaMemcpyAsync(h_err.data(), errs.p, h_err.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, g_ctx.stream),
-                        "decode status D2H");
-    if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "genotype decode");
-    cudaStreamSynchronize(g_ctx.copy_stream);
-    g_ctx.timing[0] = total.stop();  // H2D + decode + M.Mt (overlapped)
-    for (int i = 0; i < 2; i++) {
-        cudaEventDestroy(copied[i]);
-        cudaEventDestroy(decoded[i]);
-    }
-    for (int64_t k = 0; k < nchunks && rc == EG_OK; k++) rc = decode_status(&h_err[4 * k], row0, col0 + k * cw);
-    return finish_store(rc, s, out);
+// ------------------------------------------------------------------ one piece loop: every genotype upload and streamed call
+static int64_t ingest_piece_bytes();
+// Where the units [0, nm) of a piece loop come from.  A unit is a SNP row of a .bed image, a column of M.ascii or a line
+// of an ASCII file; the store layout says where it lands: a marker of either store, or, for a line of M.ascii, an
+// individual (row) of the K-blocked store.
+enum { SRC_BED = 1, SRC_ASCII_COLS = 2, SRC_ASCII_ROWS = 3 };
+struct PieceSource {
+    HostSrc hs;
+    int kind = SRC_BED;   // SRC_BED: SNP rows of a .bed image; SRC_ASCII_COLS: columns of M.ascii; SRC_ASCII_ROWS: lines
+    int64_t n = 0;        // bytes a unit decodes to: individuals, or the markers of a line of M.ascii
+    int64_t first = 0;    // unit 0 of the loop in the source: a SNP of the .bed, a column or a line of the text
+    int64_t line = 0;     // ASCII: characters per line
+    int64_t cross0 = 0;   // ASCII: the units' bytes are [cross0, cross0 + n) across them: the lines of a column piece,
+                          // the characters of each line of a line piece (a column window)
+};
+static bool whole_lines(const PieceSource& P) { return P.kind == SRC_ASCII_ROWS && P.cross0 == 0 && P.n == P.line; }
+// Staged bytes per unit: a .bed row or a whole line as in the source, n bytes of a column, a line window at a 16-byte pitch.
+static int64_t unit_bytes(const PieceSource& P) {
+    return P.kind == SRC_BED ? (P.n + 3) / 4 : P.kind == SRC_ASCII_COLS ? P.n : whole_lines(P) ? P.line + 1 : round_up(P.n, 16);
 }
-
-// Host ASCII image -> store.  Rows [row0,row1), columns [col0,col1) of an image with `cols_total`
-// characters per line.  Row blocks are staged through two device buffers so that the H2D copy of
-// block k+1 overlaps the decode of block k.
-static int store_from_image(const uint8_t* image, int64_t cols_total, int64_t row0, int64_t row1, int64_t col0,
-                            int64_t col1, bool kblocked, eg_store** out, int fd = -1) {
-    EG_TRY(ensure_init());
-    const int64_t rows = row1 - row0, w = col1 - col0, src_pitch_host = cols_total + 1;
-    if (!image || rows <= 0 || w <= 0 || col0 < 0 || col1 > cols_total || row0 < 0)
-        return set_error(EG_ERR_ARG, "genotype store: bad image range");
-    eg_store* s = nullptr;
-    EG_TRY(store_alloc(rows, w, kblocked, &s));
-    if (kblocked) {
-        // column-chunk pipeline with the M.Mt accumulation under the copy: for page-locked images (2-D copies out of
-        // pageable / mmap'ed memory are staged by the driver and slower than the row-block path below)
-        const char* env = getenv("EAGLE_EAGER_MMT");
-        cudaPointerAttributes at;
-        const bool pinned = cudaPointerGetAttributes(&at, image) == cudaSuccess && at.type == cudaMemoryTypeHost;
-        cudaGetLastError();
-        if (pinned && !(env && env[0] == '0')) return store_from_image_kb(image, src_pitch_host, row0, rows, col0, w, s, out);
-    }
-    const bool full_width = (w == cols_total);
-    const int64_t dev_pitch = full_width ? src_pitch_host : round_up(w, 16);
-    int64_t block_rows = (int64_t)(256LL << 20) / dev_pitch;
-    if (block_rows < 1) block_rows = 1;
-    if (block_rows > rows) block_rows = rows;
-    DevBuf stg[2];
-    cudaEvent_t copied[2], decoded[2];
+// Units per piece: at most ingest_piece_bytes() staged bytes, in whole 128-unit blocks.
+static int64_t piece_markers(const PieceSource& P, int64_t nm) {
+    int64_t piece = ingest_piece_bytes() / unit_bytes(P) / 128 * 128;
+    if (piece < 128) piece = 128;
+    if (piece > round_up(nm, 128)) piece = round_up(nm, 128);
+    return piece;
+}
+// Units [0, nm) of P, piece by piece.  Piece k is staged into one of two device buffers on copy_stream (through the
+// page-locked ring unless the source is page-locked memory) while piece k-1 is decoded and consumed on g_ctx.stream.
+// dst != nullptr: every piece is decoded into that store (unit m is marker m of a store of nm markers, or, for lines of
+// M.ascii, row m of a K-blocked store of nm rows), and consume(m, ns, dst) may follow it; dst == nullptr (not for lines of
+// M.ascii): into a buffer of one piece, which consume(m, ns, piece) reads (in the store's layout, ns markers) before the
+// next piece is decoded.  ASCII format errors come back with the decoders' text.  The position is that of the decoder
+// unit that saw the byte, offset by its piece and window; for column pieces of M.ascii that unit may start at another row
+// or column than a line piece's unit (both hold the byte).
+static int piece_loop(const PieceSource& P, int64_t nm, bool kblocked, int8_t* dst, uint64_t* d_missing,
+                      const std::function<int(int64_t, int64_t, const int8_t*)>& consume) {
+    const int64_t n = P.n, piece = piece_markers(P, nm), npieces = (nm + piece - 1) / piece;
+    const int64_t per = unit_bytes(P), pitch = kblocked ? 0 : store_pitch(n);
+    const size_t src_pitch = (size_t)P.line + 1;
+    const bool ascii = P.kind != SRC_BED;
+    const size_t stg_bytes = (size_t)piece * per + (ascii ? 64 : 0);
+    DevBuf stg[2], dec, errs;
     int rc = EG_OK;
-    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc((size_t)block_rows * dev_pitch + 64, "ASCII staging");
-    if (rc != EG_OK) return finish_store(rc, s, out);
+    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc(stg_bytes, "genotype staging");
+    if (rc == EG_OK && !dst)
+        rc = dec.alloc(kblocked ? (size_t)round_up(piece, 128) * n : (size_t)piece * pitch, "decoded genotype piece");
+    if (rc == EG_OK && ascii) rc = errs.alloc((size_t)npieces * 4 * sizeof(int32_t), "decode status");
+    if (rc != EG_OK) return rc;
+    if (ascii) EG_CUDA(cudaMemsetAsync(errs.p, 0, (size_t)npieces * 4 * sizeof(int32_t), g_ctx.stream));
+    cudaEvent_t copied[2], decoded[2];
     for (int i = 0; i < 2; i++) {
         cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
     }
-    // the staging buffers were allocated in g_ctx.stream order: the copy stream must not run ahead of that
     cudaEventRecord(decoded[0], g_ctx.stream);
-    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);
-    cudaMemsetAsync(g_ctx.d_err, 0, 4 * sizeof(int32_t), g_ctx.stream);
-    double t_h2d = 0;
-    Timer total(g_ctx.stream);
-    int k = 0;
-    for (int64_t r = 0; r < rows && rc == EG_OK; r += block_rows, k++) {
-        const int b = k & 1;
-        const int64_t nr = (r + block_rows <= rows) ? block_rows : rows - r;
-        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);  // staging buffer free again
-        // pageable memory and files go through the page-locked ring with parallel copier threads (hostio.cu); the
-        // decode of this block then overlaps the staging of the next one
-        HostSrc hs;
-        hs.p = image;
-        hs.fd = fd;
-        const size_t soff = (size_t)(row0 + r) * (size_t)src_pitch_host + (size_t)col0;
-        if (full_width) {
-            // the very last line of a file may lack its '\n': never read past row1*pitch - 1
-            size_t bytes = (size_t)nr * src_pitch_host;
-            if (r + nr == rows) bytes -= 1;
-            rc = h2d_staged_2d(stg[b].p, bytes, hs, soff, bytes, bytes, 1, g_ctx.copy_stream);
-        } else {
-            rc = h2d_staged_2d(stg[b].p, (size_t)dev_pitch, hs, soff, (size_t)src_pitch_host, (size_t)w, (size_t)nr, g_ctx.copy_stream);
+    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);  // the staging buffers were allocated in g_ctx.stream order
+    for (int64_t k = 0; k < npieces && rc == EG_OK; k++) {
+        const int b = (int)(k & 1);
+        const int64_t m = k * piece, ns = m + piece <= nm ? piece : nm - m, at = P.first + m;
+        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);
+        if (P.kind == SRC_BED) {
+            const size_t bytes = (size_t)ns * (size_t)per;
+            rc = h2d_staged_2d(stg[b].p, bytes, P.hs, 3 + (size_t)at * (size_t)per, bytes, bytes, 1, g_ctx.copy_stream);
+        } else if (P.kind == SRC_ASCII_COLS) {   // columns [at, at + ns) of n lines: a 2-D copy
+            rc = h2d_staged_2d(stg[b].p, (size_t)piece, P.hs, (size_t)P.cross0 * src_pitch + (size_t)at, src_pitch, (size_t)ns,
+                               (size_t)n, g_ctx.copy_stream);
+        } else if (whole_lines(P)) {             // one copy; the loop's last byte ('\n' or past the file's end) is not read
+            const size_t bytes = (size_t)ns * src_pitch - (k == npieces - 1 ? 1 : 0);
+            rc = h2d_staged_2d(stg[b].p, bytes, P.hs, (size_t)at * src_pitch, bytes, bytes, 1, g_ctx.copy_stream);
+        } else {                                 // a column window of every line: a 2-D copy
+            rc = h2d_staged_2d(stg[b].p, (size_t)per, P.hs, (size_t)at * src_pitch + (size_t)P.cross0, src_pitch, (size_t)n,
+                               (size_t)ns, g_ctx.copy_stream);
         }
         if (rc != EG_OK) break;
         cudaEventRecord(copied[b], g_ctx.copy_stream);
         cudaStreamWaitEvent(g_ctx.stream, copied[b], 0);
-        rc = kblocked ? eg_dev_decode_kb(stg[b].as<uint8_t>(), dev_pitch, (int64_t)block_rows * dev_pitch + 64, nr, w, s->d,
-                                         rows, r, g_ctx.d_err, g_ctx.stream)
-                      : eg_dev_decode(stg[b].as<uint8_t>(), dev_pitch, (int64_t)block_rows * dev_pitch + 64, nr, w,
-                                      s->d + r * s->pitch, s->pitch, g_ctx.d_err, g_ctx.stream);
+        int8_t* out = dst ? dst : dec.as<int8_t>();
+        const int64_t dm = dst ? m : 0;   // first marker of the piece in `out`
+        int32_t* err = ascii ? errs.as<int32_t>() + 4 * k : nullptr;
+        if (P.kind == SRC_BED)
+            rc = eg_dev_decode_bed(stg[b].as<uint8_t>(), n, ns, out, dst ? nm : ns, pitch, dm, d_missing, g_ctx.stream);
+        else if (P.kind == SRC_ASCII_COLS)
+            rc = eg_dev_decode_kb(stg[b].as<uint8_t>(), piece, (int64_t)stg_bytes, n, ns, out + (dm / 128) * n * 128, n, 0, err,
+                                  g_ctx.stream);
+        else if (kblocked)
+            rc = eg_dev_decode_kb(stg[b].as<uint8_t>(), per, (int64_t)stg_bytes, ns, n, dst, nm, m, err, g_ctx.stream);
+        else
+            rc = eg_dev_decode(stg[b].as<uint8_t>(), per, (int64_t)stg_bytes, ns, n, out + dm * pitch, pitch, err, g_ctx.stream);
         cudaEventRecord(decoded[b], g_ctx.stream);
+        if (rc == EG_OK && consume) rc = consume(m, ns, out);
     }
-    int32_t h_err[4] = {0, 0, 0, 0};
-    if (rc == EG_OK)
-        rc = check_cuda(cudaMemcpyAsync(h_err, g_ctx.d_err, sizeof(h_err), cudaMemcpyDeviceToHost, g_ctx.stream),
+    std::vector<int32_t> h_err(ascii ? (size_t)npieces * 4 : 0, 0);
+    if (rc == EG_OK && ascii)
+        rc = check_cuda(cudaMemcpyAsync(h_err.data(), errs.p, h_err.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, g_ctx.stream),
                         "decode status D2H");
     if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "genotype decode");
     cudaStreamSynchronize(g_ctx.copy_stream);
-    t_h2d = total.stop();
-    g_ctx.timing[0] = t_h2d;  // H2D + decode (overlapped)
     for (int i = 0; i < 2; i++) {
         cudaEventDestroy(copied[i]);
         cudaEventDestroy(decoded[i]);
     }
-    if (rc == EG_OK) rc = decode_status(h_err, row0, col0);
+    for (int64_t k = 0; k < npieces && rc == EG_OK && ascii; k++)
+        rc = P.kind == SRC_ASCII_COLS ? decode_status(&h_err[4 * k], P.cross0, P.first + k * piece)
+                                      : decode_status(&h_err[4 * k], P.first + k * piece, P.cross0);
+    return rc;
+}
+
+// Host ASCII image -> store: rows [row0,row1), columns [col0,col1) of an image with `cols_total` characters per line,
+// through the piece loop.  A K-blocked store from page-locked memory goes up in column pieces, and every decoded piece's
+// contribution to M * M^T is accumulated right away (int32, exact, order-free), so that decode and the whole SYRK hide
+// under the PCIe transfer -- at config 3 the upload takes 181 ms and the SYRK 34.  The product stays with the store
+// (eg_store::C32).  Everything else goes up in line pieces (column pieces out of pageable memory or a file would be read
+// in short segments, one per line): a line is a marker of a row-major store or an individual of a K-blocked one.
+static int store_from_image(const uint8_t* image, int64_t cols_total, int64_t row0, int64_t row1, int64_t col0,
+                            int64_t col1, bool kblocked, eg_store** out, int fd = -1) {
+    EG_TRY(ensure_init());
+    const int64_t rows = row1 - row0, w = col1 - col0;
+    if (!image || rows <= 0 || w <= 0 || col0 < 0 || col1 > cols_total || row0 < 0)
+        return set_error(EG_ERR_ARG, "genotype store: bad image range");
+    eg_store* s = nullptr;
+    EG_TRY(store_alloc(rows, w, kblocked, &s));
+    const bool by_cols = kblocked && fd < 0 && host_is_pinned(image);
+    PieceSource P;
+    P.hs.p = image;
+    P.hs.fd = fd;
+    P.kind = by_cols ? SRC_ASCII_COLS : SRC_ASCII_ROWS;
+    P.n = by_cols ? rows : w;
+    P.first = by_cols ? col0 : row0;
+    P.line = cols_total;
+    P.cross0 = by_cols ? row0 : col0;
+    std::function<int(int64_t, int64_t, const int8_t*)> syrk;
+    if (by_cols && rows >= 2) {
+        if (pool_alloc((void**)&s->C32, (size_t)rows * rows * sizeof(int32_t)) == cudaSuccess) {
+            cudaMemsetAsync(s->C32, 0, (size_t)rows * rows * sizeof(int32_t), g_ctx.stream);
+            syrk = [s](int64_t m, int64_t ns, const int8_t* d) {
+                return eg_dev_syrk_i8_kb(d + (m / 128) * s->rows * 128, s->rows, ns, s->C32, s->rows, g_ctx.stream);
+            };
+        } else {
+            cudaGetLastError();
+            s->C32 = nullptr;   // no room for the product: upload only
+        }
+    }
+    Timer total(g_ctx.stream);
+    const int rc = piece_loop(P, by_cols ? w : rows, kblocked, s->d, nullptr, syrk);
+    g_ctx.timing[0] = total.stop();  // H2D + decode (+ M.Mt when accumulated), overlapped
     return finish_store(rc, s, out);
 }
 
@@ -979,14 +982,22 @@ static eg_store* new_composite(int64_t rows, int64_t cols, bool kblocked) {
     }
     return S;
 }
-// run_all with eviction on the orchestrating thread: when a GPU runs out of memory, drop one unheld cached store and retry
-static int run_all_evicting(const std::function<int(int)>& fn, const std::function<void()>& undo) {
+// The parts of composite S (offsets set): part(r) fills S->part[r] on the thread of GPU slot r.  When a GPU runs out of
+// memory, every part is freed, one unheld cached store is dropped on the orchestrating thread and all parts are built again.
+// On failure S is deleted and the first failing slot's message is passed on.
+static int build_composite(eg_store* S, const std::function<int(int)>& part, eg_store** out) {
     for (;;) {
-        const int rc = run_all(fn);
-        if (rc != EG_ERR_ALLOC) return rc;
+        const int rc = run_all(part);
+        if (rc == EG_OK) {
+            *out = S;
+            return EG_OK;
+        }
         const std::string msg = g_err;
-        if (undo) undo();
-        if (!cache_evict_one()) return set_error(EG_ERR_ALLOC, "%s", msg.c_str());
+        run_all([S](int r) { free_part(S, r); return EG_OK; });
+        if (rc != EG_ERR_ALLOC || !cache_evict_one()) {
+            delete S;
+            return set_error(rc, "%s", msg.c_str());
+        }
     }
 }
 // Rows [row0,row1) x columns [col0,col1) of a host image -> a store; with a multi-GPU set (and allow_multi) a composite
@@ -998,120 +1009,15 @@ static int store_from_image_any(const uint8_t* image, int64_t cols_total, int64_
     if (!image || row1 <= row0 || col1 <= col0 || col0 < 0 || col1 > cols_total || row0 < 0)
         return set_error(EG_ERR_ARG, "genotype store: bad image range");
     eg_store* S = new_composite(row1 - row0, col1 - col0, kblocked);
-    auto undo = [S]() { run_all([S](int r) { free_part(S, r); return EG_OK; }); };
-    const int rc = run_all_evicting([&](int r) -> int {
+    EG_TRY(build_composite(S, [&](int r) -> int {
         const int64_t a = S->off[r], b = S->off[r + 1];
         if (a == b) return EG_OK;
         return kblocked ? store_from_image(image, cols_total, row0, row1, col0 + a, col0 + b, true, &S->part[r], fd)
                         : store_from_image(image, cols_total, row0 + a, row0 + b, col0, col1, false, &S->part[r], fd);
-    }, undo);
-    if (rc != EG_OK) {
-        const std::string msg = g_err;
-        undo();
-        delete S;
-        return set_error(rc, "%s", msg.c_str());
-    }
+    }, out));
     g_ctx.timing[0] = 0;
     for (int r = 0; r < g_multi.n; r++) g_ctx.timing[0] = std::max(g_ctx.timing[0], g_ctxs[r].timing[0]);
-    *out = S;
     return EG_OK;
-}
-
-// ------------------------------------------------------------------ one piece loop: .bed uploads and streamed stores
-static int64_t ingest_piece_bytes();
-// Where the genotypes of the markers [0, nm) of a piece loop come from.
-enum { SRC_BED = 1, SRC_ASCII_COLS = 2, SRC_ASCII_ROWS = 3 };
-struct PieceSource {
-    HostSrc hs;
-    int kind = SRC_BED;   // SRC_BED: SNP rows of a .bed image; SRC_ASCII_COLS: columns of M.ascii; SRC_ASCII_ROWS: lines of Mt.ascii
-    int64_t n = 0;        // individuals
-    int64_t first = 0;    // marker 0 of the loop in the source: a SNP of the .bed, a column or a line of the text
-    int64_t line = 0;     // ASCII: characters per line
-    int64_t lines = 0;    // ASCII: lines of the file (the last one may lack its '\n')
-};
-// Markers per piece: at most ingest_piece_bytes() source bytes, in whole 128-marker blocks.
-static int64_t piece_markers(const PieceSource& P, int64_t nm) {
-    const int64_t per = P.kind == SRC_BED ? (P.n + 3) / 4 : P.kind == SRC_ASCII_COLS ? P.n : P.line + 1;
-    int64_t piece = ingest_piece_bytes() / per / 128 * 128;
-    if (piece < 128) piece = 128;
-    if (piece > round_up(nm, 128)) piece = round_up(nm, 128);
-    return piece;
-}
-// Markers [0, nm) of P, piece by piece.  Piece k is staged into one of two device buffers on copy_stream (through the
-// page-locked ring unless the source is page-locked memory) while piece k-1 is decoded and consumed on g_ctx.stream.
-// dst != nullptr: every piece is decoded into that store (marker m of the loop is marker m of a store of nm markers);
-// dst == nullptr: into a buffer of one piece, which consume(m, ns, piece) reads (in the store's layout, ns markers) before
-// the next piece is decoded.  ASCII format errors come back with the resident upload's text.  The position is that of the
-// decoder unit that saw the byte, offset by the piece: the resident one for row pieces of Mt.ascii; for column pieces of
-// M.ascii a unit of the piece, which may start at another row or column than the resident upload's unit (both hold the
-// byte).
-static int piece_loop(const PieceSource& P, int64_t nm, bool kblocked, int8_t* dst, uint64_t* d_missing,
-                      const std::function<int(int64_t, int64_t, const int8_t*)>& consume) {
-    const int64_t n = P.n, piece = piece_markers(P, nm), npieces = (nm + piece - 1) / piece;
-    const int64_t bpr = (n + 3) / 4, pitch = kblocked ? 0 : store_pitch(n);
-    const bool ascii = P.kind != SRC_BED;
-    const size_t stg_bytes = P.kind == SRC_BED          ? (size_t)piece * bpr
-                             : P.kind == SRC_ASCII_COLS ? (size_t)n * piece + 64
-                                                        : (size_t)piece * (P.line + 1) + 64;
-    DevBuf stg[2], dec, errs;
-    int rc = EG_OK;
-    for (int i = 0; i < 2 && rc == EG_OK; i++) rc = stg[i].alloc(stg_bytes, "genotype staging");
-    if (rc == EG_OK && !dst)
-        rc = dec.alloc(kblocked ? (size_t)round_up(piece, 128) * n : (size_t)piece * pitch, "decoded genotype piece");
-    if (rc == EG_OK && ascii) rc = errs.alloc((size_t)npieces * 4 * sizeof(int32_t), "decode status");
-    if (rc != EG_OK) return rc;
-    if (ascii) EG_CUDA(cudaMemsetAsync(errs.p, 0, (size_t)npieces * 4 * sizeof(int32_t), g_ctx.stream));
-    cudaEvent_t copied[2], decoded[2];
-    for (int i = 0; i < 2; i++) {
-        cudaEventCreateWithFlags(&copied[i], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&decoded[i], cudaEventDisableTiming);
-    }
-    cudaEventRecord(decoded[0], g_ctx.stream);
-    cudaStreamWaitEvent(g_ctx.copy_stream, decoded[0], 0);  // the staging buffers were allocated in g_ctx.stream order
-    for (int64_t k = 0; k < npieces && rc == EG_OK; k++) {
-        const int b = (int)(k & 1);
-        const int64_t m = k * piece, ns = m + piece <= nm ? piece : nm - m, at = P.first + m;
-        if (k >= 2) cudaStreamWaitEvent(g_ctx.copy_stream, decoded[b], 0);
-        if (P.kind == SRC_BED) {
-            const size_t bytes = (size_t)ns * (size_t)bpr;
-            rc = h2d_staged_2d(stg[b].p, bytes, P.hs, 3 + (size_t)at * (size_t)bpr, bytes, bytes, 1, g_ctx.copy_stream);
-        } else if (P.kind == SRC_ASCII_COLS) {   // columns [at, at + ns) of every line: a 2-D copy
-            rc = h2d_staged_2d(stg[b].p, (size_t)piece, P.hs, (size_t)at, (size_t)(P.line + 1), (size_t)ns, (size_t)n, g_ctx.copy_stream);
-        } else {                                 // whole lines; never read past the file's last byte
-            size_t bytes = (size_t)ns * (size_t)(P.line + 1);
-            if (at + ns == P.lines) bytes -= 1;
-            rc = h2d_staged_2d(stg[b].p, bytes, P.hs, (size_t)at * (size_t)(P.line + 1), bytes, bytes, 1, g_ctx.copy_stream);
-        }
-        if (rc != EG_OK) break;
-        cudaEventRecord(copied[b], g_ctx.copy_stream);
-        cudaStreamWaitEvent(g_ctx.stream, copied[b], 0);
-        int8_t* out = dst ? dst : dec.as<int8_t>();
-        const int64_t dm = dst ? m : 0;   // first marker of the piece in `out`
-        if (P.kind == SRC_BED)
-            rc = eg_dev_decode_bed(stg[b].as<uint8_t>(), n, ns, out, dst ? nm : ns, pitch, dm, d_missing, g_ctx.stream);
-        else if (P.kind == SRC_ASCII_COLS)
-            rc = eg_dev_decode_kb(stg[b].as<uint8_t>(), piece, (int64_t)stg_bytes, n, ns, out + (dm / 128) * n * 128, n, 0,
-                                  errs.as<int32_t>() + 4 * k, g_ctx.stream);
-        else
-            rc = eg_dev_decode(stg[b].as<uint8_t>(), P.line + 1, (int64_t)stg_bytes, ns, n, out + dm * pitch, pitch,
-                               errs.as<int32_t>() + 4 * k, g_ctx.stream);
-        cudaEventRecord(decoded[b], g_ctx.stream);
-        if (rc == EG_OK && consume) rc = consume(m, ns, out);
-    }
-    std::vector<int32_t> h_err(ascii ? (size_t)npieces * 4 : 0, 0);
-    if (rc == EG_OK && ascii)
-        rc = check_cuda(cudaMemcpyAsync(h_err.data(), errs.p, h_err.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, g_ctx.stream),
-                        "decode status D2H");
-    if (rc == EG_OK) rc = check_cuda(cudaStreamSynchronize(g_ctx.stream), "genotype decode");
-    cudaStreamSynchronize(g_ctx.copy_stream);
-    for (int i = 0; i < 2; i++) {
-        cudaEventDestroy(copied[i]);
-        cudaEventDestroy(decoded[i]);
-    }
-    for (int64_t k = 0; k < npieces && rc == EG_OK && ascii; k++)
-        rc = P.kind == SRC_ASCII_COLS ? decode_status(&h_err[4 * k], 0, P.first + k * piece)
-                                      : decode_status(&h_err[4 * k], P.first + k * piece, 0);
-    return rc;
 }
 
 // The source of a streamed store, and how many pieces a call over all of its markers runs.
@@ -1123,7 +1029,6 @@ static PieceSource source_of(const eg_store* s) {
     P.n = s->pitch ? s->cols : s->rows;
     P.first = s->src_first;
     P.line = s->src_line;
-    P.lines = s->rows;   // M.ascii: n lines; Mt.ascii: L lines
     return P;
 }
 static int64_t stream_pieces(const eg_store* s) {
@@ -1276,7 +1181,7 @@ static int partial_product(const eg_store* M, const std::vector<int64_t>& zero_c
     }
     const char* envk = getenv("EAGLE_KEEP_PRODUCT");   // "0": contract again on every call (bench.py's steady-state leg)
     const bool reuse = !(envk && envk[0] == '0');
-    if (M->C32 && reuse) {  // accumulated under the upload (store_from_image_kb): keep it intact for later calls
+    if (M->C32 && reuse) {  // accumulated under the upload (store_from_image): keep it intact for later calls
         EG_CUDA(cudaMemcpyAsync(C.p, M->C32, (size_t)n * n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
         g_ctx.timing[1] = 0.0;
     } else {
@@ -1761,22 +1666,13 @@ extern "C" int eg_store_transpose(const eg_store_t* in, eg_store_t** out) {
         if (in->mt_orientation) return set_error(EG_ERR_ARG, "eg_store_transpose: sharded Mt stores are not transposed back");
         eg_store* S = new_composite(in->cols, in->rows, false);
         for (int r = 0; r <= in->nparts; r++) S->off[r] = in->off[r];
-        auto undo = [S]() { run_all([S](int r) { free_part(S, r); return EG_OK; }); };
-        const int rc = run_all_evicting([&](int r) -> int {
+        return build_composite(S, [&](int r) -> int {
             const eg_store* p = in->part[r];
             if (!p) return EG_OK;
             EG_TRY(store_alloc(p->cols, p->rows, false, &S->part[r]));
             EG_TRY(eg_dev_transpose_kb_i8(p->d, p->rows, p->cols, S->part[r]->d, S->part[r]->pitch, g_ctx.stream));
             return check_cuda(cudaStreamSynchronize(g_ctx.stream), "transpose");
-        }, undo);
-        if (rc != EG_OK) {
-            const std::string msg = g_err;
-            undo();
-            delete S;
-            return set_error(rc, "%s", msg.c_str());
-        }
-        *out = S;
-        return EG_OK;
+        }, out);
     }
     eg_store* s = nullptr;
     EG_TRY(store_alloc(in->cols, in->rows, false, &s));  // the transpose is always a row-major (Mt-type) store
@@ -2426,103 +2322,87 @@ static int create_ascii_nospace_plink(const char* fname, const char* asciifname,
     *ok = 1;
     return EG_OK;
 }
-// A row-major store as a no-space ASCII file: encode in row blocks of ~256 MB, two page-locked buffers, the D2H of block k
-// running while block k-1 is written.
-static int write_store_ascii(const eg_store* T, const char* path) {
-    if (!T->pitch) return set_error(EG_ERR_ARG, "write_store_ascii: needs a row-major store");
-    const int64_t rows = T->rows, cols = T->cols, line = cols + 1;
+// No-space ASCII lines made on the device, written to a file in order: two device and two page-locked buffers, so that
+// block k is written while block k + 1 is encoded and copied back.
+struct AsciiWriter {
+    const char* path = nullptr;
     OutFile outf;
-    outf.f = fopen(path, "wb");
-    int rc = outf.f ? EG_OK : set_error(EG_ERR_OPEN, "ERROR: Could not open  %s for writing", path);
-    int64_t block_rows = (256LL << 20) / line;
-    if (block_rows < 1) block_rows = 1;
-    if (block_rows > rows) block_rows = rows;
-    DevBuf denc[2];
-    PinnedBuf henc[2];
-    cudaEvent_t done[2] = {nullptr, nullptr};
-    for (int i = 0; i < 2 && rc == EG_OK; i++) {
-        rc = denc[i].alloc((size_t)block_rows * line + 16, "ASCII rows");
-        if (rc == EG_OK) rc = henc[i].ensure((size_t)block_rows * line + 16, "ASCII rows");
-        if (rc == EG_OK) rc = check_cuda(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming), "cudaEventCreate");
-    }
-    int64_t pending_rows[2] = {0, 0};
-    int k = 0;
-    for (int64_t r = 0; rc == EG_OK && r < rows; r += block_rows, k++) {
-        const int b = k & 1;
-        const int64_t nr = r + block_rows <= rows ? block_rows : rows - r;
-        rc = eg_dev_encode_ascii(T->d, T->pitch, cols, r, nr, denc[b].as<uint8_t>(), g_ctx.stream);
-        if (rc == EG_OK)
-            rc = check_cuda(cudaMemcpyAsync(henc[b].p, denc[b].p, (size_t)nr * line, cudaMemcpyDeviceToHost, g_ctx.stream), "D2H of ASCII rows");
-        if (rc == EG_OK) rc = check_cuda(cudaEventRecord(done[b], g_ctx.stream), "cudaEventRecord");
-        pending_rows[b] = nr;
-        if (rc == EG_OK && k >= 1) {  // write the previous block while this one is in flight
-            const int pb = b ^ 1;
-            rc = check_cuda(cudaEventSynchronize(done[pb]), "ASCII rows");
-            const size_t wb = (size_t)pending_rows[pb] * line;
-            if (rc == EG_OK && fwrite(henc[pb].p, 1, wb, outf.f) != wb) rc = set_error(EG_ERR_OPEN, "short write to %s", path);
-            pending_rows[pb] = 0;
-        }
-    }
-    if (rc == EG_OK && k >= 1) {
-        const int pb = (k - 1) & 1;
-        rc = check_cuda(cudaEventSynchronize(done[pb]), "ASCII rows");
-        const size_t wb = (size_t)pending_rows[pb] * line;
-        if (rc == EG_OK && fwrite(henc[pb].p, 1, wb, outf.f) != wb) rc = set_error(EG_ERR_OPEN, "short write to %s", path);
-    }
-    cudaStreamSynchronize(g_ctx.stream);
-    for (int i = 0; i < 2; i++)
-        if (done[i]) cudaEventDestroy(done[i]);
-    if (outf.f) {
-        if (fclose(outf.f) != 0 && rc == EG_OK) rc = set_error(EG_ERR_OPEN, "short write to %s", path);
-        outf.f = nullptr;
-    }
-    return rc;
-}
-// createMt_ASCII_rcpp on a streamed M store: every column piece of M.ascii is decoded, transposed and encoded on the device,
-// and its lines of Mt.ascii are written in order -- the bytes write_store_ascii writes for the resident transpose.  Two
-// page-locked buffers: piece k is written to the file while piece k + 1 is on the device.
-static int write_mt_ascii_streamed(const eg_store* M, const char* path) {
-    const int64_t n = M->rows, line = n + 1, tp = store_pitch(n);
-    const int64_t piece = piece_markers(source_of(M), M->cols);
-    cudaStream_t st = g_ctx.stream;
-    OutFile outf;
-    outf.f = fopen(path, "wb");
-    if (!outf.f) return set_error(EG_ERR_OPEN, "ERROR: Could not open  %s for writing", path);
-    DevBuf T, enc[2];
+    DevBuf enc[2];
     PinnedBuf h[2];
     cudaEvent_t done[2] = {nullptr, nullptr};
     size_t pending[2] = {0, 0};
-    int rc = T.alloc((size_t)piece * tp, "transposed genotype piece");
-    for (int i = 0; i < 2 && rc == EG_OK; i++) {
-        rc = enc[i].alloc((size_t)piece * line + 16, "ASCII rows");
-        if (rc == EG_OK) rc = h[i].ensure((size_t)piece * line + 16, "ASCII rows");
-        if (rc == EG_OK) rc = check_cuda(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming), "cudaEventCreate");
+    int64_t k = 0;   // blocks pushed
+    ~AsciiWriter() {
+        for (int i = 0; i < 2; i++)
+            if (done[i]) cudaEventDestroy(done[i]);
     }
-    auto flush = [&](int b) -> int {   // the lines of the piece in buffer b, once its copy has landed
+    int open(const char* p, size_t block_bytes) {
+        path = p;
+        outf.f = fopen(path, "wb");
+        if (!outf.f) return set_error(EG_ERR_OPEN, "ERROR: Could not open  %s for writing", path);
+        for (int i = 0; i < 2; i++) {
+            EG_TRY(enc[i].alloc(block_bytes, "ASCII rows"));
+            EG_TRY(h[i].ensure(block_bytes, "ASCII rows"));
+            EG_CUDA(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming));
+        }
+        return EG_OK;
+    }
+    uint8_t* next() { return enc[k & 1].as<uint8_t>(); }   // where the next block is encoded (on g_ctx.stream)
+    int push(size_t bytes) {   // the next block is queued: its D2H, then the write of the block before it
+        const int b = (int)(k++ & 1);
+        EG_CUDA(cudaMemcpyAsync(h[b].p, enc[b].p, bytes, cudaMemcpyDeviceToHost, g_ctx.stream));
+        EG_CUDA(cudaEventRecord(done[b], g_ctx.stream));
+        pending[b] = bytes;
+        return flush(b ^ 1);
+    }
+    int flush(int b) {   // the block in buffer b, once its copy has landed
         if (!pending[b]) return EG_OK;
         EG_CUDA(cudaEventSynchronize(done[b]));
         const size_t wb = pending[b];
         pending[b] = 0;
         return fwrite(h[b].p, 1, wb, outf.f) == wb ? EG_OK : set_error(EG_ERR_OPEN, "short write to %s", path);
-    };
-    int64_t k = 0;
+    }
+    int close(int rc) {   // rc: the caller's status; the last block is written only after success
+        if (rc == EG_OK) rc = flush((int)((k - 1) & 1));
+        cudaStreamSynchronize(g_ctx.stream);
+        if (outf.f && fclose(outf.f) != 0 && rc == EG_OK) rc = set_error(EG_ERR_OPEN, "short write to %s", path);
+        outf.f = nullptr;
+        return rc;
+    }
+};
+// A row-major store as a no-space ASCII file, encoded in row blocks of ~256 MB.
+static int write_store_ascii(const eg_store* T, const char* path) {
+    if (!T->pitch) return set_error(EG_ERR_ARG, "write_store_ascii: needs a row-major store");
+    const int64_t rows = T->rows, cols = T->cols, line = cols + 1;
+    int64_t block_rows = (256LL << 20) / line;
+    if (block_rows < 1) block_rows = 1;
+    if (block_rows > rows) block_rows = rows;
+    AsciiWriter w;
+    int rc = w.open(path, (size_t)block_rows * line + 16);
+    for (int64_t r = 0; rc == EG_OK && r < rows; r += block_rows) {
+        const int64_t nr = r + block_rows <= rows ? block_rows : rows - r;
+        rc = eg_dev_encode_ascii(T->d, T->pitch, cols, r, nr, w.next(), g_ctx.stream);
+        if (rc == EG_OK) rc = w.push((size_t)nr * line);
+    }
+    return w.close(rc);
+}
+// createMt_ASCII_rcpp on a streamed M store: every column piece of M.ascii is decoded, transposed and encoded on the device,
+// and its lines of Mt.ascii are written in order -- the bytes write_store_ascii writes for the resident transpose.
+static int write_mt_ascii_streamed(const eg_store* M, const char* path) {
+    const int64_t n = M->rows, line = n + 1, tp = store_pitch(n);
+    const int64_t piece = piece_markers(source_of(M), M->cols);
+    cudaStream_t st = g_ctx.stream;
+    AsciiWriter w;
+    DevBuf T;
+    int rc = w.open(path, (size_t)piece * line + 16);
+    if (rc == EG_OK) rc = T.alloc((size_t)piece * tp, "transposed genotype piece");
     if (rc == EG_OK)
         rc = piece_loop(source_of(M), M->cols, true, nullptr, nullptr, [&](int64_t, int64_t ns, const int8_t* p) -> int {
-            const int b = (int)(k++ & 1);
             EG_TRY(eg_dev_transpose_kb_i8(p, n, ns, T.as<int8_t>(), tp, st));
-            EG_TRY(eg_dev_encode_ascii(T.as<int8_t>(), tp, n, 0, ns, enc[b].as<uint8_t>(), st));
-            EG_CUDA(cudaMemcpyAsync(h[b].p, enc[b].p, (size_t)ns * line, cudaMemcpyDeviceToHost, st));
-            EG_CUDA(cudaEventRecord(done[b], st));
-            pending[b] = (size_t)ns * line;
-            return flush(b ^ 1);   // the previous piece, while this one is in flight
+            EG_TRY(eg_dev_encode_ascii(T.as<int8_t>(), tp, n, 0, ns, w.next(), st));
+            return w.push((size_t)ns * line);
         });
-    if (rc == EG_OK) rc = flush((int)((k - 1) & 1));
-    cudaStreamSynchronize(st);
-    for (int i = 0; i < 2; i++)
-        if (done[i]) cudaEventDestroy(done[i]);
-    if (fclose(outf.f) != 0 && rc == EG_OK) rc = set_error(EG_ERR_OPEN, "short write to %s", path);
-    outf.f = nullptr;
-    return rc;
+    return w.close(rc);
 }
 }  // namespace eg
 
@@ -2769,25 +2649,17 @@ static int store_from_bed_any(const HostSrc& src, int64_t n, int64_t snp0, int64
     EG_TRY(ensure_init());
     eg_store* S = kblocked ? new_composite(n, snp1 - snp0, true) : new_composite(snp1 - snp0, n, false);
     std::vector<uint64_t> miss((size_t)g_multi.n, 0);
-    auto undo = [S]() { run_all([S](int r) { free_part(S, r); return EG_OK; }); };
-    const int rc = run_all_evicting([&](int r) -> int {
+    EG_TRY(build_composite(S, [&](int r) -> int {
         const int64_t a = S->off[r], b = S->off[r + 1];
         if (a == b) return EG_OK;
         return store_from_bed(src, n, snp0 + a, snp0 + b, kblocked, &miss[(size_t)r], &S->part[r]);
-    }, undo);
-    if (rc != EG_OK) {
-        const std::string msg = g_err;
-        undo();
-        delete S;
-        return set_error(rc, "%s", msg.c_str());
-    }
+    }, out));
     *n_missing = 0;
     g_ctx.timing[0] = 0;
     for (int r = 0; r < g_multi.n; r++) {
         *n_missing += miss[(size_t)r];
         g_ctx.timing[0] = std::max(g_ctx.timing[0], g_ctxs[r].timing[0]);
     }
-    *out = S;
     return EG_OK;
 }
 }  // namespace eg

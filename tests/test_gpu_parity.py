@@ -78,14 +78,18 @@ def write_pair(tmp_path, G, tag):
 
 
 # ------------------------------------------------------------------------------- decode
-def test_readblock_bit_exact(synth_small):
+def test_readblock_bit_exact(synth_small, monkeypatch):
     s = synth_small
-    for (f, start, ncols, nrows) in [(s["M"], 0, s["L"], s["n"]), (s["M"], 7, s["L"], 50), (s["M"], 200, 1, 3),
-                                     (s["Mt"], 100, 60, 9), (s["Mt"], 0, s["n"], s["L"]), (s["Mt"], 2999, s["n"], 2)]:
-        got = api.ReadBlock(f, start, ncols, nrows)
-        ref = eo.ReadBlock(f, start, ncols, nrows)
-        assert got.flags.f_contiguous and got.shape == ref.shape
-        assert np.array_equal(got, ref)
+    for piece_bytes in (None, "64"):   # one piece; pieces of 128 lines, whole or a column window of each
+        if piece_bytes:
+            monkeypatch.setenv("EAGLE_INGEST_PIECE_BYTES", piece_bytes)
+        for (f, start, ncols, nrows) in [(s["M"], 0, s["L"], s["n"]), (s["M"], 7, s["L"], 50), (s["M"], 200, 1, 3),
+                                         (s["Mt"], 100, 60, 9), (s["Mt"], 0, s["n"], s["L"]), (s["Mt"], 2999, s["n"], 2),
+                                         (s["Mt"], 5, 150, 2990)]:
+            got = api.ReadBlock(f, start, ncols, nrows)
+            ref = eo.ReadBlock(f, start, ncols, nrows)
+            assert got.flags.f_contiguous and got.shape == ref.shape
+            assert np.array_equal(got, ref), (piece_bytes, start, ncols, nrows)
 
 
 def test_open_and_format_errors(tmp_path, synth_small):

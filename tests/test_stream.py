@@ -233,7 +233,10 @@ def test_streamed_ascii_equals_resident(gpu, tmp_path, monkeypatch):
 def test_bad_byte_in_a_later_piece_gives_the_resident_error(gpu, tmp_path, monkeypatch):
     """Same code and text as the resident upload.  The position is the decoder unit's that saw the byte: the same as the
     resident one for Mt.ascii; for M.ascii, whose column pieces go through other decoder units than the resident upload's
-    whole rows, a unit inside the piece that holds the byte (at most 16 rows of at most one piece's columns)."""
+    whole rows, a unit inside the piece that holds the byte (at most 16 rows of at most one piece's columns).  The
+    resident uploads from pageable memory and files run through the same piece loop in line pieces, so the piece size is
+    set before them too: M.ascii in pieces of 128 lines puts the byte in the second piece, Mt.ascii in pieces of 640
+    lines in the fourth, and both must still report the byte's absolute row."""
     import re
     from oracle import np_oracle as npo
     n, L = 203, 3001
@@ -246,12 +249,14 @@ def test_bad_byte_in_a_later_piece_gives_the_resident_error(gpu, tmp_path, monke
         b[r * (cols + 1) + c] = ord("7")
         open(path, "wb").write(bytes(b))
         kb = path == m
+        monkeypatch.setenv("EAGLE_INGEST_PIECE_BYTES", str(128 * (L + 1)) if kb else str(700 * (n + 1)))
         with pytest.raises(_lib.EagleGpuError) as want:   # the resident uploads: K-blocked M, row-major Mt
             if kb:
                 gpu.GenotypeStore.from_file(path, rows, cols)
             else:
                 gpu.GenotypeStore.from_host_rows(np.frombuffer(bytes(b), np.uint8), rows, cols, 0, rows)
-        monkeypatch.setenv("EAGLE_INGEST_PIECE_BYTES", str(1024 * n) if kb else str(700 * (n + 1)))
+        if kb:
+            monkeypatch.setenv("EAGLE_INGEST_PIECE_BYTES", str(1024 * n))
         s = gpu.GenotypeStore.stream_file(path, rows, cols, kblocked=kb)
         with pytest.raises(_lib.EagleGpuError) as got:
             if kb:
@@ -270,6 +275,56 @@ def test_bad_byte_in_a_later_piece_gives_the_resident_error(gpu, tmp_path, monke
         else:
             assert str(got.value) == str(want.value)
         monkeypatch.delenv("EAGLE_INGEST_PIECE_BYTES")
+
+
+# (route, piece bytes) at n = 403, L = 3001: column pieces of 1024 markers (3), line pieces of 128 individuals (4) or of
+# 640 markers (5); the default piece size takes each upload in one piece
+RESIDENT_PIECES = {"pinned": 1024 * 403, "pageable": 128 * 3002, "pageable_window": 128 * 3002, "file": 128 * 3002,
+                   "file_window": 128 * 3002, "rows_window": 700 * 404}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("route", sorted(RESIDENT_PIECES))
+def test_resident_ascii_uploads_in_pieces_equal_one_piece(gpu, route, tmp_path, monkeypatch):
+    """The resident ASCII uploads run through the piece loop: in several ragged pieces they give the store bytes, K and
+    a / var(a) of one piece.  A page-locked image keeps accumulating M.Mt under the copy (no contraction in mmt)."""
+    import torch
+    from oracle import np_oracle as npo
+    n, L, c0, c1 = 403, 3001, 130, 2777
+    G = synth.genotypes(n, L, seed=18)
+    img = np.concatenate([synth.ascii_image(G).reshape(-1), np.zeros(64, np.uint8)])
+    imgT = synth.ascii_image(np.ascontiguousarray(G.T)).reshape(-1)
+    pinned = torch.from_numpy(img.copy()).pin_memory()
+    m = str(tmp_path / "M.ascii")
+    npo.write_ascii(m, G)
+    S, V, a = synth.scan_inputs(n)
+    kb = route != "rows_window"
+
+    def upload():
+        GS = gpu.GenotypeStore
+        return {"pinned": lambda: GS.from_host_ptr(pinned.data_ptr(), n, L),
+                "pageable": lambda: GS.from_host_ascii(img, n, L),
+                "pageable_window": lambda: GS.from_host_ascii(img, n, L, c0, c1),
+                "file": lambda: GS.from_file(m, n, L),
+                "file_window": lambda: GS.from_file(m, n, L, c0, c1),
+                "rows_window": lambda: GS.from_host_rows(imgT, L, n, c0, c1)}[route]()
+
+    def results():
+        s = upload()
+        i = s.info()
+        words = np.empty((i["rows"], (i["cols"] + 31) // 32), np.uint64)
+        _lib.check(_lib.load().eg_store_to_host_packed(s._h, words.ctypes.data_as(C.c_void_p)))
+        M, Mt = (s, s.transpose()) if kb else (s.transpose(), s)
+        K = M.mmt()
+        syrk_ms = gpu.last_timing()["syrk_ms"]
+        return words, K, syrk_ms, *Mt.a_and_vara(S, V, a)
+
+    one = results()
+    monkeypatch.setenv("EAGLE_INGEST_PIECE_BYTES", str(RESIDENT_PIECES[route]))
+    several = results()
+    for x, y in zip(one[:2] + one[3:], several[:2] + several[3:]):
+        assert np.array_equal(x, y)
+    assert (one[2] == several[2] == 0.0) == (route == "pinned"), (one[2], several[2])
 
 
 @pytest.mark.gpu
