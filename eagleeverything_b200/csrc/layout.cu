@@ -297,7 +297,8 @@ __global__ void __launch_bounds__(256) transpose_kb128_kernel(const int8_t* __re
 // the 10^10 FMAs of config 3 where reading Mt takes 1.7 ms.  Same digit scheme as scan_i8.cu instead: x is written
 // as 2^(e-55) * sum_s q_s 256^(6-s) with 7 balanced int8 digits (|residual| <= 2^(e-56), e from max |x|), the seven
 // integer dot products  A_s(j) = sum_i m_ji q_s(i)  are exact (DP4A, int32) in any order, and they are recombined
-// with ONE rounding.  Identical rows give bit-identical results wherever they sit.
+// with ONE rounding.  Identical rows give bit-identical results wherever they sit.  An x whose largest magnitude is below
+// 2^-1020 (e < -1019) gets the scale ldexp(1, e - 55) = 0, so y = 0: the vectors of the search (E_c, v) are far above it.
 constexpr int GD_KW = 4096;           // words (4 genotypes each) of x digits staged per pass: 7 x 16 KB of shared memory
 constexpr int GD_ROWS_PER_WARP = 8;
 constexpr int GD_SMEM_BYTES = 7 * GD_KW * 4;

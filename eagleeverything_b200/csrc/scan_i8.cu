@@ -581,7 +581,9 @@ scan_i8_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
 
 // ------------------------------------------------------------------ slicing of U
 // per column: e_k with max_i |U_ik| * 2^(-e_k) in [0.5, 127/128) (so that the top digit, carry included,
-// stays <= 127); scale_k = 2^(e_k - 55)
+// stays <= 127); scale_k = 2^(e_k - 55).  A column whose largest magnitude is below 2^-1020 (e_k < -1019) gets
+// scale_k = ldexp(1, e_k - 55) = 0 and its products are flushed to 0: eigenvector columns (unit norm, or scaled by
+// sqrt(count) >= 1) and the scan's folded W never come near it (tests/test_gpu_bcache_exact.py pins the behaviour)
 __global__ void __launch_bounds__(256) si_colscale_kernel(const double* __restrict__ Wp, int64_t n, int64_t ld,
                                                           int32_t* __restrict__ expo, double* __restrict__ scale,
                                                           int64_t ncols_pad, int bits, int full) {
@@ -616,40 +618,42 @@ __global__ void __launch_bounds__(256) si_colscale_kernel(const double* __restri
         scale[k] = s;
     }
 }
-// Q rows for column k = 32 g + kk: g*224 + (kk>>2)*28 + s*4 + (kk&3); thread -> 4 consecutive i
+// Q rows for column k = 32 g + kk: g*224 + (kk>>2)*28 + s*4 + (kk&3); thread -> 4 consecutive i.  Columns are strided
+// over gridDim.y, which cannot exceed 65,535: n beyond that (the projection of a larger U) takes a second pass.
 template <int S>
 __global__ void __launch_bounds__(256) si_slice_kernel(const double* __restrict__ Wp, int64_t n, int64_t ld,
                                                        const int32_t* __restrict__ expo, int8_t* __restrict__ Q,
-                                                       int64_t Kp, int full) {
-    const int64_t k = blockIdx.y;
+                                                       int64_t Kp, int full, int64_t ncols_pad) {
     const int64_t i0 = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 4;
     if (i0 >= Kp) return;
-    const int64_t g = k / SI_GCOLS;
-    const int kk = (int)(k - g * SI_GCOLS);
-    int8_t* base = Q + (g * SiT<S>::BN + (kk >> 2) * SiT<S>::CHUNK + (kk & 3)) * Kp + i0;
-    uint32_t out[S];
+    for (int64_t k = blockIdx.y; k < ncols_pad; k += gridDim.y) {
+        const int64_t g = k / SI_GCOLS;
+        const int kk = (int)(k - g * SI_GCOLS);
+        int8_t* base = Q + (g * SiT<S>::BN + (kk >> 2) * SiT<S>::CHUNK + (kk & 3)) * Kp + i0;
+        uint32_t out[S];
 #pragma unroll
-    for (int s = 0; s < S; s++) out[s] = 0;
-    if (k < n) {
-        const int e = expo[k];
+        for (int s = 0; s < S; s++) out[s] = 0;
+        if (k < n) {
+            const int e = expo[k];
 #pragma unroll
-        for (int d = 0; d < 4; d++) {
-            const int64_t i = i0 + d;
-            if ((full || i <= k) && i < n) {
-                const double xs = ldexp(Wp[i + k * ld], SiT<S>::BITS - e);  // |xs| <= 127 * 2^(8 S - 8) (exact scaling)
-                long long X = fabs(xs) < 3.6e16 ? __double2ll_rn(xs) : 0;  // rint: |residual| <= 1/2 unit = 2^(e - 8 S)  // NaN / Inf: the column's scale is NaN
+            for (int d = 0; d < 4; d++) {
+                const int64_t i = i0 + d;
+                if ((full || i <= k) && i < n) {
+                    const double xs = ldexp(Wp[i + k * ld], SiT<S>::BITS - e);  // |xs| <= 127 * 2^(8 S - 8) (exact scaling)
+                    long long X = fabs(xs) < 3.6e16 ? __double2ll_rn(xs) : 0;  // rint: |residual| <= 1/2 unit = 2^(e - 8 S)  // NaN / Inf: the column's scale is NaN
 #pragma unroll
-                for (int s = S - 1; s > 0; s--) {          // balanced digits, least significant first
-                    const int q = (int)(int8_t)(X & 0xFF);
-                    out[s] |= ((uint32_t)q & 0xFFu) << (8 * d);
-                    X = (X - q) >> 8;                              // exact: X - q is a multiple of 256
+                    for (int s = S - 1; s > 0; s--) {          // balanced digits, least significant first
+                        const int q = (int)(int8_t)(X & 0xFF);
+                        out[s] |= ((uint32_t)q & 0xFFu) << (8 * d);
+                        X = (X - q) >> 8;                              // exact: X - q is a multiple of 256
+                    }
+                    out[0] |= ((uint32_t)(int)X & 0xFFu) << (8 * d);  // top digit in [-127, 127]
                 }
-                out[0] |= ((uint32_t)(int)X & 0xFFu) << (8 * d);  // top digit in [-127, 127]
             }
         }
-    }
 #pragma unroll
-    for (int s = 0; s < S; s++) *reinterpret_cast<uint32_t*>(base + (int64_t)s * 4 * Kp) = out[s];
+        for (int s = 0; s < S; s++) *reinterpret_cast<uint32_t*>(base + (int64_t)s * 4 * Kp) = out[s];
+    }
 }
 
 // (mb, g) -> position in the super-tile order
@@ -799,8 +803,9 @@ static int launch_scan_i8_t(const int8_t* d_Mt, int64_t L, int64_t n, int64_t pi
         si_colscale_kernel<<<(unsigned)(G * SI_GCOLS), 256, 0, st>>>(d_Wp, n, Kpad, g_si.expo, g_si.scale, (int64_t)G * SI_GCOLS,
                                                                      SiT<S>::BITS, full);
         EG_TRY(check_launch("si_colscale_kernel"));
-        si_slice_kernel<S><<<dim3((unsigned)((Kp / 4 + 255) / 256), (unsigned)(G * SI_GCOLS)), 256, 0, st>>>(d_Wp, n, Kpad, g_si.expo,
-                                                                                                       g_si.Q, Kp, full);
+        const int64_t ncols_pad = (int64_t)G * SI_GCOLS;
+        si_slice_kernel<S><<<dim3((unsigned)((Kp / 4 + 255) / 256), (unsigned)(ncols_pad < 65535 ? ncols_pad : 65535)), 256, 0, st>>>(
+            d_Wp, n, Kpad, g_si.expo, g_si.Q, Kp, full, ncols_pad);
         EG_TRY(check_launch("si_slice_kernel"));
         g_si.sliced_n = full ? -1 : n;   // a projection slices another matrix: the scan's U is gone
         g_si.sliced_digits = S;
